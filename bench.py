@@ -2,13 +2,16 @@
 """bench.py -- batched Cobweb predict throughput on B200 (see DESIGN.md "Measurement").
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl engine|reference] [--workload cfg1|cfg2|cfg3|cfg4]
-                  [--mode fused|fp32] [--shard query|store]
+                  [--mode fused|fp32] [--shard query|store] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic queries: dense cobweb_predict_fast
 semantics (every query against every node, path product, top-k) on a tree built by the engine's own
 ifit from synthetic embeddings of the BASELINE.json shape.  One JSON line on stdout (rank 0).  Under
 torchrun the node store is built on rank 0 and broadcast over NCCL, each rank answers its own batch
 (weak scaling) and the results are all-gathered on the device inside the timed step.
+
+--dump-outputs DIR writes the ids and scores of the last timed step as DIR/<name>.npy.  The inputs are seeded, so
+two builds of the project run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -22,6 +25,8 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the tree it runs from as it found it (it may be read-only)
+DUMP_MAX_BYTES = 64 * 10**6
 
 WORKLOADS = {
     # name: (docs, dim, queries per GPU, k, corpus kind, BASELINE.json config it is)
@@ -35,6 +40,24 @@ GOLDEN = {"cfg1": "cfg1_unit_1000x384", "cfg2": "cfg2_unit_1500x1024"}
 
 def log(*a):
     print(*a, file=sys.stderr, flush=True)
+
+
+def dump_outputs(out_dir, ids, scores):
+    """The last timed step's answer as out_dir/ids.npy (float64: exact for any sentence id) and out_dir/scores.npy
+    (float32).  A batch beyond DUMP_MAX_BYTES in all is cut to a fixed seeded sample of its query rows, whose row
+    numbers go to out_dir/rows.npy."""
+    arrays = {"ids": np.asarray(ids, np.float64), "scores": np.asarray(scores, np.float32)}
+    n = len(arrays["ids"])
+    row_bytes = sum(a[:1].nbytes for a in arrays.values())
+    budget = DUMP_MAX_BYTES - 3 * 1024  # the .npy headers
+    if n * row_bytes > budget:
+        rows = np.sort(np.random.default_rng(0).choice(n, budget // (row_bytes + 8), replace=False))
+        arrays = {name: a[rows] for name, a in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log(f"[bench] outputs of the last timed step -> {out_dir}: " + ", ".join(f"{k} {a.shape}" for k, a in arrays.items()))
 
 
 class ClockSampler:
@@ -156,7 +179,7 @@ def run_reference(args, wl):
         cpu_predict_rate(ot, q, k, min_seconds=0.0, max_rounds=1)
     t0 = time.time()
     for _ in range(args.steps):
-        cpu_predict_rate(ot, q, k, min_seconds=0.0, max_rounds=1)
+        ids, scores = oracle_topk(ot, q, k)
     dt = time.time() - t0
     v = sample * args.steps / dt
     line = {
@@ -172,6 +195,8 @@ def run_reference(args, wl):
                                    f"{cores} threads set explicitly"},
         "e2e": {"value": v, "unit": "queries/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ids, scores)
     print(json.dumps(line), flush=True)
 
 
@@ -340,13 +365,20 @@ def _run_engine(args, wl):
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return float(ms.item())
 
+    last_step = [None]
+
+    def step_device_kept():
+        last_step[0] = step_device()
+
     for _ in range(max(args.warmup, 3)):
         step_device()
         step_host()
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    ms_dev = timed(step_device, args.steps)
+    ms_dev = timed(step_device_kept, args.steps)
+    # copied now: the all-gather reuses its buffers in the next call
+    last_out = [t.cpu().numpy() for t in last_step[0]] if args.dump_outputs and rank == 0 else None
     ms_host = timed(step_host, args.steps)
     # the stages of one fused chunk (CUDA events inside cw_fused_profile) / the FP32 score kernel alone
     nq_k = min(qn, ix.fused_workspace(qn, k)["cap_q"]) if fused else min(qn, ix.chunk_queries())
@@ -619,6 +651,8 @@ def _run_engine(args, wl):
                  "rows_per_insert": counters["rows"] / docs,
                  "hbm_frac": (counters["rows"] + counters["levels"] + docs) * (8.0 * dim + 4) / build_s / 1e9 / peaks["hbm_gbs"]},
     }
+    if last_out is not None:
+        dump_outputs(args.dump_outputs, *last_out)
     if world > 1:
         dist.destroy_process_group()
     return line
@@ -643,7 +677,12 @@ def main():
                     help="N>1: 'query' replicates the store and shards the batch (weak scaling, default); "
                          "'store' shards sentences+nodes, every rank answers the whole batch, per-rank top-k "
                          "lists are merged after an NCCL all-gather (strong scaling)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the ids and scores the last one computed as DIR/<name>.npy "
+                         f"(at most {DUMP_MAX_BYTES // 10**6} MB: a larger batch is cut to a fixed seeded sample of its rows)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     wl = list(WORKLOADS[args.workload])
     if args.docs:
         wl[0] = args.docs

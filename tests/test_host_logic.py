@@ -274,6 +274,29 @@ def test_evaluator_matches_the_reference_loop():
     assert got["method"] == "x" and got["time_taken"] == 1.5 and got["avg_latency_ms"] == 5.0
 
 
+def test_bench_dump_outputs_whole_or_seeded_sample(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: a batch under the cap is written whole (ids exact as float64); a larger one as the same
+    seeded sample of rows on every call, under the cap, with its row numbers."""
+    import bench
+    rng = np.random.default_rng(2)
+    ids = rng.integers(0, 1 << 30, (500, 10)).astype(np.int32)
+    scores = rng.standard_normal((500, 10)).astype(np.float32)
+    bench.dump_outputs(str(tmp_path / "whole"), ids, scores)
+    assert sorted(os.listdir(tmp_path / "whole")) == ["ids.npy", "scores.npy"]
+    got = np.load(tmp_path / "whole" / "ids.npy")
+    assert got.dtype == np.float64 and np.array_equal(got.astype(np.int32), ids)
+    assert np.array_equal(np.load(tmp_path / "whole" / "scores.npy"), scores)
+    monkeypatch.setattr(bench, "DUMP_MAX_BYTES", 3 * 1024 + 100 * 128)
+    for name in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / name), ids, scores)
+    files = {f: np.load(tmp_path / "a" / f) for f in ("ids.npy", "scores.npy", "rows.npy")}
+    rows = files["rows.npy"].astype(np.int64)
+    assert len(rows) == 100 and (np.diff(rows) > 0).all()
+    assert np.array_equal(files["ids.npy"], ids[rows]) and np.array_equal(files["scores.npy"], scores[rows])
+    assert all(np.array_equal(a, np.load(tmp_path / "b" / f)) for f, a in files.items())
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= bench.DUMP_MAX_BYTES
+
+
 def test_fused_layout_reproduces_the_path_sums():
     """(C[parent] + w_leaf s_leaf) / len over the fused layout == sum_j (w_j / len) s_j over the root->leaf paths
     (CobwebWrapper.py:160-169), every sentence appears exactly once, sampled tiles lead."""
