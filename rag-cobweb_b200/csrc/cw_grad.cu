@@ -19,7 +19,7 @@ int cw_check_cuda(cudaError_t e, const char *what);
 
 namespace cw {
 
-// grid (position chunks, query groups of 32 per warp, 4 warps per CTA)
+// grid (position chunks, query groups of 32 per warp, 1/2/4 warps per CTA)
 __global__ void __launch_bounds__(128)
 paths_transpose_kernel(const float *__restrict__ G, long long nq, int n_pos, int max_len,
                        const int *__restrict__ path_pm, const int4 *__restrict__ pos_rec,
@@ -143,16 +143,32 @@ extern "C" int cw_rank_scores_bwd(const cw_index *ix, const float *Q, int64_t nq
     }
     if (nq == 0) return 0;
     cudaStream_t st = (cudaStream_t)stream;
-    int rc = cw_check_cuda(cudaMemsetAsync(gs_scratch, 0, (size_t)ix->nn * ldq * sizeof(float), st), "cw_rank_scores_bwd: memset");
+    // warps per CTA of the path transpose: each warp keeps a [max_len][32] run stack and a [max_len] node list in shared
+    // memory, so deep trees get 2 or 1 warps per CTA (the forward path kernel accepts max_len up to 1024)
+    int dev = 0, optin = 0;
+    int rc = cw_check_cuda(cudaGetDevice(&dev), "cw_rank_scores_bwd: device");
     if (rc) return rc;
-    const int wpb = 4;
+    rc = cw_check_cuda(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev), "cw_rank_scores_bwd: smem limit");
+    if (rc) return rc;
+    auto smem_of = [&](int w) {
+        return (size_t)ix->max_len * sizeof(double) + (size_t)w * ix->max_len * (32 * sizeof(float) + sizeof(int));
+    };
+    int wpb = 4;
+    while (wpb > 1 && smem_of(wpb) > (size_t)optin) wpb /= 2;
+    if (smem_of(wpb) > (size_t)optin) {
+        cw_set_error("cw_rank_scores_bwd: max_len=%d needs %zu bytes of shared memory with one warp per CTA, more than the %d one CTA has",
+                     ix->max_len, smem_of(1), optin);
+        return CW_E_ARG;
+    }
+    rc = cw_check_cuda(cudaMemsetAsync(gs_scratch, 0, (size_t)ix->nn * ldq * sizeof(float), st), "cw_rank_scores_bwd: memset");
+    if (rc) return rc;
     const long long groups = (nq + 31) / 32, gblocks = (groups + wpb - 1) / wpb;
     long long want = (148 * 32 + groups - 1) / groups;
     if (want > (ix->n_pos + 255) / 256) want = (ix->n_pos + 255) / 256;
     if (want < 1) want = 1;
     const int chunk_len = (int)((ix->n_pos + want - 1) / want);
     const int n_chunks = (ix->n_pos + chunk_len - 1) / chunk_len;
-    const size_t smem = (size_t)ix->max_len * sizeof(double) + (size_t)wpb * ix->max_len * (32 * sizeof(float) + sizeof(int));
+    const size_t smem = smem_of(wpb);
     if (smem > 48 * 1024) {
         rc = cw_check_cuda(cudaFuncSetAttribute(cw::paths_transpose_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),
                            "cw_rank_scores_bwd: smem attribute");

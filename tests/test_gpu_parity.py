@@ -591,7 +591,7 @@ def test_fused_predict_flagged_queries_and_fallbacks():
             w.set_level_weights(weights)
         w.build_prediction_index()
         ix = w._index
-        for k in (1, 10, 30, 40):
+        for k in (1, 10, 30, 40, 128):  # 128: the fallback's top-k fills all four register slots of the merge
             ix.set_mode("fp32")
             ids32, v32, _ = ix.predict(qd, k, small=False)
             ix.set_mode("fused")
@@ -631,8 +631,10 @@ def test_fused_predict_flagged_queries_and_fallbacks():
 
 def test_small_batch_exact_path():
     """cw_small_predict (thread-per-node FP32 chains, HBM-bound for one query) = the big FP32 kernels bit for bit, for
-    1..32 queries, odd D, through the device call, the host call and cobweb_predict_fast."""
-    for n, d, kind, k in ((900, 100, "unit", 10), (2000, 256, "whitened", 5), (300, 7, "whitened", 1), (600, 1030, "unit", 40)):
+    1..32 queries, odd D, through the device call, the host call and cobweb_predict_fast.  k = 64 puts rank k-1 in lane 31
+    of the second register slot, 65 and 128 use the third and fourth slots of the merge and of the insertion loop."""
+    for n, d, kind, k in ((900, 100, "unit", 10), (2000, 256, "whitened", 5), (300, 7, "whitened", 1), (600, 1030, "unit", 40),
+                          (2000, 64, "unit", 64), (2500, 33, "whitened", 65), (3000, 128, "unit", 128)):
         x = synth.corpus(n, d, kind, seed=31)
         w = CobwebWrapper(corpus=[None] * n, corpus_embeddings=x)
         q, _ = synth.queries(x, 40, kind, seed=32)
