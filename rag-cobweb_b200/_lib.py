@@ -23,7 +23,7 @@ FUSED_MAX_K, FUSED_FB_ROUNDS, SMALL_Q, SID_UNRESOLVED, FUSED_STATS, FUSED_STAGES
 EXPORTS = ["cw_version", "cw_last_error", "cw_store_init", "cw_store_derive", "cw_ifit", "cw_set_ifit_cluster", "cw_selftest_arith", "cw_categorize_ctas", "cw_categorize",
            "cw_index_build", "cw_xt_floats", "cw_score_ldq", "cw_dense_node_scores", "cw_topk_chunks", "cw_dense_paths_topk",
            "cw_predict_dense_host", "cw_index_rows_build",
-           "cw_h_b_bytes", "cw_h_a_bytes", "cw_h_stages", "cw_h_set_build", "cw_h_rows_isotropic", "cw_fused_predict",
+           "cw_h_b_bytes", "cw_h_a_bytes", "cw_h_stages", "cw_h_set_build", "cw_h_rows_isotropic", "cw_fused_flag_words", "cw_fused_predict",
            "cw_fused_predict_host", "cw_fused_profile", "cw_small_scratch_words", "cw_small_predict", "cw_small_predict_host",
            "cw_rank_scores_bwd", "cw_whiten", "cw_ffma_peak", "cw_ffma2_peak"]
 
@@ -66,7 +66,7 @@ class CwFusedIndex(C.Structure):
 class CwFusedWork(C.Structure):
     _fields_ = [("cap_q", C.c_int64), ("ldq", C.c_int64), ("Q_dev", C.c_void_p), ("A_int", C.c_void_p), ("A_leaf", C.c_void_p),
                 ("qv", C.c_void_p), ("S", C.c_void_p), ("slots", C.c_void_p), ("tau", C.c_void_p), ("cap", C.c_int32),
-                ("reserved", C.c_int32), ("cnt", C.c_void_p), ("cand_val", C.c_void_p), ("cand_row", C.c_void_p),
+                ("fin_ml", C.c_int32), ("cnt", C.c_void_p), ("cand_val", C.c_void_p), ("cand_row", C.c_void_p),
                 ("flag", C.c_void_p), ("out_sid_dev", C.c_void_p), ("out_val_dev", C.c_void_p), ("sm_Q", C.c_void_p),
                 ("sm_scores", C.c_void_p), ("sm_scratch", C.c_void_p), ("sm_sid", C.c_void_p), ("sm_val", C.c_void_p),
                 ("sm_n", C.c_void_p), ("stats", C.c_void_p), ("audit_every", C.c_int32), ("audit_phase", C.c_int32)]
@@ -119,6 +119,8 @@ def load():
     L.cw_h_stages.argtypes = [i32c, i32c, i32c]
     L.cw_h_set_build.argtypes = [C.POINTER(CwStore), vp, vp, vp, C.POINTER(CwHSet), vp, vp, vp, vp, vp]
     L.cw_h_rows_isotropic.argtypes = [C.POINTER(CwStore), vp, vp, i32c, vp, vp]
+    L.cw_fused_flag_words.restype = i64
+    L.cw_fused_flag_words.argtypes = [i64, i32c]
     L.cw_fused_predict.argtypes = [C.POINTER(CwFusedIndex), C.POINTER(CwFusedWork), vp, i64, i32, vp, vp, vp]
     L.cw_fused_predict_host.argtypes = [C.POINTER(CwFusedIndex), C.POINTER(CwFusedWork), vp, i64, i32, vp, vp, vp, vp]
     L.cw_fused_profile.argtypes = [C.POINTER(CwFusedIndex), C.POINTER(CwFusedWork), vp, i64, i32, vp, vp, vp, vp]

@@ -14,7 +14,7 @@
 //              exact in the fp32 accumulator), so by Cauchy-Schwarz the whole contraction is off by at most
 //              c1 ||a_q||_2 ||b_n||_2: a bound that costs one FMA per (query, leaf) in the epilogue.  A leaf
 //              whose upper bound stays below the query's threshold is dropped; what survives (~100 of 100k leaves)
-//              is re-scored exactly by the finish kernel.  Leaves almost always have ONE variance for all
+//              is re-scored exactly by the finish stage.  Leaves almost always have ONE variance for all
 //              attributes (a leaf holds one vector or exact duplicates: M2 = 0, var = prior), then
 //              sum_d x^2/var = |x|^2/var is a rank-one term of the epilogue and the contraction runs over D features
 //              (layout F1) instead of 2D (layout F2).
@@ -757,7 +757,7 @@ __device__ __forceinline__ float eps_of(float xx, float inv_prior, float hmax, f
     const float tq = 2.0f * (xx * inv_prior + hmax);
     return wfac * (eps_scale * tq + 1.1920929e-07f * (4.0f + 3.0f * sqrtf((float)max_len)) * 0.5f * (lmax + hmax + tq));
 }
-// tau[q] = (m-th largest of the 32 slot maxima) - margin; a heuristic for speed only: the finish kernel verifies
+// tau[q] = (m-th largest of the 32 slot maxima) - margin; a heuristic for speed only: the finish stage verifies
 // on the device that nothing below the threshold could have mattered.
 __global__ void __launch_bounds__(128)
 h_tau_kernel(const int *__restrict__ slots, const float4 *__restrict__ qv, long long nq, int m, float e1max, float inv_prior,
@@ -787,10 +787,21 @@ __global__ void h_fill_kernel(float *p, long long n, float v) {
     if (i < n) p[i] = v;
 }
 
-// ------------------------------------------------------------------ finish: select, refine, line test, exact re-score
-constexpr int FN_THREADS = 128, FN_WARPS = FN_THREADS / 32;
-constexpr int FN_R = 16;  // rows a warp of the finish kernel scores exactly at a time (sizes its transposition buffer)
+// ------------------------------------------------------------------ finish: select, exact pair scores, line test, top-k
+// Five launches instead of one CTA per query, so that dozens of warps per SM keep row loads in flight and no warp waits
+// at a block barrier for another warp's FMA chain:
+//   fn_select_kernel  one warp per query: interval pruning of the candidates, the refine list, eps, U
+//   fn_exact_kernel   one warp per query: exact node scores of a list of index rows (the refine list, then the ancestors)
+//   fn_line_kernel    one warp per query: a3, the line test, the survivors and their distinct ancestors
+//   fn_exact_kernel   (ancestors)
+//   fn_topk_kernel    one warp per query: exact path sums of the survivors, top-k sentences
+// The per-query lists live in global scratch behind the flag words (cw_fused_flag_words).
+constexpr int FQ_WARPS = 8;  // queries per CTA of the per-query kernels
 constexpr int KC1 = CW_FUSED_KC1, MS = CW_FUSED_MSURV, MAXS = CW_FUSED_MAX_SENT;
+// meta words per query; the survivors (indices into the refine list) follow at FM_SURV
+enum { FM_NSEL, FM_NANC, FM_M, FM_EPS, FM_U, FM_FAIL, FM_SURV = 8, FM_STRIDE = FM_SURV + MS };
+
+__host__ __device__ inline long long fin_words(long long cap_q, int ml) { return cap_q * (FM_STRIDE + 3 * KC1 + 3LL * MS * ml); }
 
 struct FinArgs {
     cw_index ix;
@@ -807,320 +818,396 @@ struct FinArgs {
     const int *leaf_row_b, *leaf_pos, *sent_off, *sent_ids;
     const float *C;
     long long ldq;
-    float e1max, inv_prior, hmax, lmax, wfac, eps_scale;
+    float inv_prior, hmax, lmax, wfac, eps_scale;
     int *out_sid;
     float *out_val;
     int *flag;   // [0] count, [4..] queries
     int *stats;
+    // scratch (fin_carve)
+    int em;          // MS * max_len: ancestor entries per query
+    int *meta;       // [nq, FM_STRIDE]
+    int *ref_row;    // [nq, KC1] leaf rows of the refined candidates
+    int *ref_b;      // [nq, KC1] their index rows
+    float *ref_s;    // [nq, KC1] their exact node scores
+    int *anc_b;      // [nq, em] distinct ancestor index rows of the survivors
+    float *anc_s;    // [nq, em] their exact node scores
+    int *anc_slot;   // [nq, em] (survivor, level) -> entry of anc_b
 };
 
-__host__ __device__ inline size_t fin_smem_bytes(int D, int ML, int cap) {
-    const size_t E = (size_t)MS * ML;
-    return (size_t)ML * 8 + (size_t)FN_WARPS * FN_R * 33 * 8 + (size_t)((D + 3) & ~3) * 4 + (size_t)cap * 14 + (size_t)KC1 * 36 +
-           E * 12 + E * 4 + (size_t)MS * 12 + (size_t)MAXS * 8 + 64 + 16 + 16 + 8 + (size_t)FN_WARPS * FN_R * 8 + 8;
+static void fin_carve(FinArgs &a, int *p, long long cap_q, int ml) {
+    a.em = MS * ml;
+    a.meta = p; p += cap_q * FM_STRIDE;
+    a.ref_row = p; p += cap_q * KC1;
+    a.ref_b = p; p += cap_q * KC1;
+    a.ref_s = reinterpret_cast<float *>(p); p += cap_q * KC1;
+    a.anc_b = p; p += cap_q * a.em;
+    a.anc_s = reinterpret_cast<float *>(p); p += cap_q * a.em;
+    a.anc_slot = p;
 }
 
-__global__ void __launch_bounds__(FN_THREADS)
-h_finish_kernel(const FinArgs a) {
-    extern __shared__ __align__(16) unsigned char fn_smem[];
-    const int D = a.ix.D, ML = a.ix.max_len, cap = a.cap, EMAX = MS * ML;
-    double *lw = reinterpret_cast<double *>(fn_smem);                     // [ML] (rounded to 16 bytes)
-    float2 *stage = reinterpret_cast<float2 *>(lw + ((ML + 1) & ~1));     // [FN_WARPS][FN_R][33]
-    float *xq = reinterpret_cast<float *>(stage + FN_WARPS * FN_R * 33);  // [D]
-    float *cv = xq + ((D + 3) & ~3);                                      // [cap] candidate a1
-    int *cr = reinterpret_cast<int *>(cv + cap);                          // [cap] candidate leaf row
-    float *ce = reinterpret_cast<float *>(cr + cap);                      // [cap] candidate error bound E
-    // selected candidates, best a1 first
-    int *srow = reinterpret_cast<int *>(ce + cap);                        // [KC1] leaf row
-    int *sb = srow + KC1;                                                 // [KC1] index row of the leaf
-    float *ss = reinterpret_cast<float *>(sb + KC1);                      // [KC1] exact leaf term
-    float *sa3 = ss + KC1;                                                // [KC1]
-    int *sns = reinterpret_cast<int *>(sa3 + KC1);                        // [KC1] sentences of the leaf
-    int *ssel = sns + KC1;                                                // [KC1] survivor slot or -1
-    int *sbefore = ssel + KC1;                                            // [KC1]
-    float *swl = reinterpret_cast<float *>(sbefore + KC1);                // [KC1] w_leaf
-    int *slen = reinterpret_cast<int *>(swl + KC1);                       // [KC1] path length
-    // survivors
-    int *nid = slen + KC1;                                                // [E] index row of (survivor, level)
-    int *ulist = nid + EMAX;                                              // [E] unique rows
-    float *uscore = reinterpret_cast<float *>(ulist + EMAX);              // [E]
-    unsigned short *firstc = reinterpret_cast<unsigned short *>(uscore + EMAX);  // [E]
-    unsigned short *slot = firstc + EMAX;                                 // [E]
-    int *mc = reinterpret_cast<int *>(slot + EMAX);                       // [MS] selected index of survivor
-    float *mex = reinterpret_cast<float *>(mc + MS);                      // [MS] exact leaf score
-    int *mso = reinterpret_cast<int *>(mex + MS);                         // [MS] offset of its sentences in the list
-    int *lsid = mso + MS;                                                 // [MAXS]
-    float *lval = reinterpret_cast<float *>(lsid + MAXS);                 // [MAXS]
-    int *misc = reinterpret_cast<int *>(lval + MAXS);                     // [16] counters and broadcast values
-    unsigned short *byrank = reinterpret_cast<unsigned short *>(misc + 16);  // [cap] candidate with a1 rank r
-    const float2 **rowp_s = reinterpret_cast<const float2 **>(byrank + ((cap + 3) & ~3));  // [FN_WARPS][FN_R] row pointers
+__device__ __forceinline__ int warp_sum(int v) {
+    for (int off = 16; off > 0; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
+    return v;
+}
+// candidate order: a1 descending, leaf row ascending (one 64-bit key, larger = better; -0 and +0 are one a1)
+__device__ __forceinline__ unsigned long long cand_key(float v, int row) {
+    return (unsigned long long)((unsigned)float_key(v == 0.0f ? 0.0f : v) ^ 0x80000000u) << 32 | (unsigned)~row;
+}
 
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+// Which candidates need the exact leaf term.  Every candidate has the interval [a1 - E, a1 + E] (E = e1[row] *
+// ||a_q||, the filter's derived bound) around its leaf score with exact leaf term; L_k = the smallest lower end among
+// the k best candidates by a1 is a lower bound of the k-th best such score (k different leaves reach it), so a
+// candidate whose upper end stays 3 eps below L_k cannot reach the line drawn later and is dropped unrefined.  The
+// rest -- the best KC1 of them by a1 -- is refined.  U = the largest upper end among everything left unrefined
+// (dropped or cut here, or rejected by the filter: below tau).  Also adds the filter's candidate count to the stats.
+__global__ void __launch_bounds__(FQ_WARPS * 32)
+fn_select_kernel(const FinArgs a) {
+    extern __shared__ __align__(16) unsigned char fs_smem[];
+    __shared__ unsigned long long cand_sum;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, cap = a.cap;
+    float *cv = reinterpret_cast<float *>(fs_smem) + (size_t)warp * cap * 3;  // [cap] a1
+    int *cr = reinterpret_cast<int *>(cv + cap);                              // [cap] leaf row
+    float *ce = cv + 2 * cap;                                                 // [cap] E
     const float NEG_INF = -__int_as_float(0x7f800000);
-    for (int i = tid; i < ML; i += FN_THREADS) lw[i] = a.ix.level_w[i];
-
-    // exact node scores of the rows list[0..U) with the FP32 path's arithmetic.  The rows are cut into rounds of at
-    // most FN_R; a warp takes a round: lane = row for the arithmetic (every lane runs its row's FMA chain in order),
-    // lane = attribute for the loads (per 32 attributes one coalesced 256-byte load per row, one or two segments ahead
-    // of the arithmetic), transposed through shared memory.  Rounds are packed densely -- the chain phase costs the same
-    // whether a warp holds 1 row or 16, so 13 rows are ONE warp's round, not four.
-    auto exact_round = [&](auto rtag, const int *list, int lo, int cnt, float *outs) {
-        constexpr int R = decltype(rtag)::value;
-        constexpr int DEPTH = R <= 8 ? 2 : 1;  // segments in flight ahead of the arithmetic (registers: 2 R per segment)
-        float2 *stw = stage + warp * FN_R * 33;
-        const float2 **rowp = rowp_s + warp * FN_R;
-        const int b = lane < cnt ? list[lo + lane] : -1;
-        if (lane < R) rowp[lane] = a.RM + (size_t)(b < 0 ? 0 : b) * D;
+    if (threadIdx.x == 0) cand_sum = 0;
+    __syncthreads();
+    const long long q = (long long)blockIdx.x * FQ_WARPS + warp;
+    if (q < a.nq) {
+        const int n_all = a.cnt[q], n = min(n_all, cap);
+        const float4 qq = a.qv[q];
+        const float eps = eps_of(qq.y, a.inv_prior, a.hmax, a.lmax, a.wfac, a.eps_scale, a.ix.max_len);
+        for (int i = lane; i < n; i += 32) {
+            const int row = a.cand_row[q * cap + i];
+            cv[i] = a.cand_val[q * cap + i];
+            cr[i] = row;
+            ce[i] = __fmul_rn(a.leaf_rc[row * 2 + 1].x, qq.z);
+        }
         __syncwarp();
-        float acc = 0.0f;
-        float2 o[DEPTH][R];
-        auto fetch = [&](int d0, float2 (&dst)[R]) {
-            const bool dok = d0 + lane < D;
-#pragma unroll
-            for (int r = 0; r < R; r++) {
-                dst[r] = make_float2(0.0f, 0.0f);
-                if (r < cnt && dok) dst[r] = rowp[r][d0 + lane];  // r < cnt is warp-uniform
+        // L_k: the k-th best key by k rounds of a warp-wide maximum below the previous one; the k best are the keys >= it
+        float Lk = NEG_INF;
+        if (n >= a.k) {
+            unsigned long long last = ~0ull;
+            for (int it = 0; it < a.k; it++) {
+                unsigned long long best = 0;
+                for (int i = lane; i < n; i += 32) {
+                    const unsigned long long key = cand_key(cv[i], cr[i]);
+                    if (key < last && key > best) best = key;
+                }
+                for (int off = 16; off > 0; off >>= 1) {
+                    const unsigned long long o = __shfl_xor_sync(0xffffffffu, best, off);
+                    best = o > best ? o : best;
+                }
+                last = best;
             }
+            int lo = 0x7fffffff;
+            for (int i = lane; i < n; i += 32)
+                if (cand_key(cv[i], cr[i]) >= last) lo = min(lo, float_key(__fsub_rn(__fsub_rn(cv[i], ce[i]), eps)));
+            for (int off = 16; off > 0; off >>= 1) lo = min(lo, __shfl_xor_sync(0xffffffffu, lo, off));
+            Lk = key_float(lo);
+        }
+        int count = 0;
+        for (int i = lane; i < n; i += 32) count += __fmaf_rn(3.0f, eps, __fadd_rn(cv[i], ce[i])) >= Lk;
+        count = warp_sum(count);
+        // refine list: every kept candidate, or the best KC1 of them by a1 when more are kept
+        int* const rrow = a.ref_row + q * KC1;
+        int* const rb = a.ref_b + q * KC1;
+        float umax = NEG_INF;
+        int pos0 = 0;
+        for (int base = 0; base < n; base += 32) {
+            const int i = base + lane;
+            const bool keep = i < n && __fmaf_rn(3.0f, eps, __fadd_rn(cv[i], ce[i])) >= Lk;
+            int pos;
+            if (count <= KC1) {
+                pos = pos0 + __popc(__ballot_sync(0xffffffffu, keep) & ((1u << lane) - 1u));
+                pos0 += __popc(__ballot_sync(0xffffffffu, keep));
+            } else {
+                pos = 0;
+                if (keep) {
+                    const unsigned long long key = cand_key(cv[i], cr[i]);
+                    for (int j = 0; j < n; j++)
+                        pos += cand_key(cv[j], cr[j]) > key && __fmaf_rn(3.0f, eps, __fadd_rn(cv[j], ce[j])) >= Lk;
+                }
+            }
+            if (keep && pos < KC1) {
+                rrow[pos] = cr[i];
+                rb[pos] = a.leaf_row_b[cr[i]];
+            } else if (i < n) {
+                umax = fmaxf(umax, __fadd_rn(cv[i], ce[i]));  // left unrefined
+            }
+        }
+        umax = warp_max(umax);
+        if (lane == 0) {
+            int *m = a.meta + q * FM_STRIDE;
+            m[FM_NSEL] = min(count, KC1);
+            m[FM_EPS] = __float_as_int(eps);
+            m[FM_U] = __float_as_int(fmaxf(a.tau[q], umax));
+            m[FM_FAIL] = n_all > cap ? 1 : 0;  // candidate-buffer overflow
+            atomicAdd(&cand_sum, (unsigned long long)(unsigned)n_all);
+        }
+    }
+    __syncthreads();
+    // candidates appended by the filter (64-bit total in words 5, 6), queries in word 7
+    if (threadIdx.x == 0 && cand_sum) atomicAdd(reinterpret_cast<unsigned long long *>(a.stats + 6), cand_sum);
+    if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(a.stats + 5, (int)a.nq);
+}
+
+__device__ __forceinline__ void cp_async8(void *dst, const void *src) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_u32(dst)), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async4(void *dst, const void *src) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(smem_u32(dst)), "l"(src) : "memory");
+}
+
+// Exact node scores with the FP32 path's arithmetic: out[q * stride + i] = -0.5 (sumlog[b] + sum_d (x_qd r_bd + mb_bd)^2)
+// for b = list[q * stride + i], i < meta[q][n_word].  One warp per query; its rows go in rounds of at most EX_R.  For the
+// arithmetic lane = row (every lane runs its row's FMA chain in ascending d from 0, so the result is bit-identical to
+// dense_score_kernel), for the loads lane = attribute: per 32 attributes of a row one coalesced 256-byte cp.async
+// segment into a ring of EX_STAGES segments, EX_STAGES - 1 ahead of the arithmetic.  A row's segment is padded to
+// EX_RS = 34 float2, so the 16-byte reads by row are conflict-free (8 lanes, 8 different 4-bank groups) and a lane takes
+// its whole segment into registers before the chain runs over it.  No registers hold the rows in flight, so a warp needs
+// only its ring and 12 warps fit on an SM.
+constexpr int EX_WARPS = 4, EX_R = 16, EX_STAGES = 4, EX_RS = 34;
+constexpr int EX_WARP_BYTES = EX_STAGES * EX_R * EX_RS * 8 + EX_STAGES * 32 * 4;
+__global__ void __launch_bounds__(EX_WARPS * 32)
+fn_exact_kernel(const cw_index ix, const float2 *__restrict__ RM, const float *__restrict__ Q, long long nq,
+                const int *__restrict__ list, const int *__restrict__ meta, int n_word, int stride, float *out) {
+    extern __shared__ __align__(16) unsigned char ex_smem[];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, D = ix.D;
+    float2 *ring = reinterpret_cast<float2 *>(ex_smem + (size_t)warp * EX_WARP_BYTES);  // [EX_STAGES][EX_R][EX_RS]
+    float *xr = reinterpret_cast<float *>(ring + EX_STAGES * EX_R * EX_RS);             // [EX_STAGES][32]
+    const long long q = (long long)blockIdx.x * EX_WARPS + warp;
+    if (q >= nq) return;
+    const int n = meta[q * FM_STRIDE + n_word];
+    if (n <= 0) return;
+    const float *xq = Q + q * D;
+    const int n_seg = (D + 31) / 32;
+    const int n_rounds = (n + EX_R - 1) / EX_R, rpr = (n + n_rounds - 1) / n_rounds;  // rows per round <= EX_R
+    for (int lo = 0; lo < n; lo += rpr) {
+        const int cnt = min(rpr, n - lo);
+        const int b = lane < cnt ? list[q * stride + lo + lane] : 0;
+        auto issue = [&](int seg) {
+            if (seg < n_seg) {
+                const int s = seg & (EX_STAGES - 1), d = seg * 32 + lane;
+                for (int r = 0; r < cnt; r++) {
+                    const int br = __shfl_sync(0xffffffffu, b, r);
+                    if (d < D) cp_async8(ring + (s * EX_R + r) * EX_RS + lane, RM + (size_t)br * D + d);
+                }
+                if (d < D) cp_async4(xr + s * 32 + lane, xq + d);
+            }
+            asm volatile("cp.async.commit_group;" ::: "memory");  // one group per segment, empty past the end
         };
 #pragma unroll
-        for (int p = 0; p < DEPTH; p++) fetch(32 * p, o[p]);
-        for (int d0 = 0; d0 < D; d0 += 32 * DEPTH) {
+        for (int p = 0; p < EX_STAGES - 1; p++) issue(p);
+        float acc = 0.0f;
+        for (int seg = 0; seg < n_seg; seg++) {
+            issue(seg + EX_STAGES - 1);
+            asm volatile("cp.async.wait_group %0;" ::"n"(EX_STAGES - 1) : "memory");
+            __syncwarp();
+            const int s = seg & (EX_STAGES - 1), dd = seg * 32;
+            const float2 *rv = ring + (s * EX_R + lane) * EX_RS;
+            const float *xs = xr + s * 32;
+            if (lane < cnt) {
+                if (dd + 32 <= D) {
+                    float4 rr[16], xv[8];
 #pragma unroll
-            for (int p = 0; p < DEPTH; p++) {
-                const int dd = d0 + 32 * p;
-                if (dd >= D) break;  // warp-uniform
+                    for (int j = 0; j < 16; j++) rr[j] = reinterpret_cast<const float4 *>(rv)[j];  // {r, mb} of 2 attributes
 #pragma unroll
-                for (int r = 0; r < R; r++) stw[r * 33 + lane] = o[p][r];
-                __syncwarp();
-                if (dd + 32 * DEPTH < D) fetch(dd + 32 * DEPTH, o[p]);
-                if (lane < cnt) {
-                    if (dd + 32 <= D) {
+                    for (int j = 0; j < 8; j++) xv[j] = reinterpret_cast<const float4 *>(xs)[j];
 #pragma unroll
-                        for (int j4 = 0; j4 < 8; j4++) {
-                            const float4 xv = *reinterpret_cast<const float4 *>(xq + dd + 4 * j4);
-                            const float xs[4] = {xv.x, xv.y, xv.z, xv.w};
-#pragma unroll
-                            for (int e = 0; e < 4; e++) {
-                                const float2 v = stw[lane * 33 + 4 * j4 + e];
-                                const float t = __fmaf_rn(xs[e], v.x, v.y);
-                                acc = __fmaf_rn(t, t, acc);
-                            }
-                        }
-                    } else {
-                        for (int j = 0; j < D - dd; j++) {
-                            const float2 v = stw[lane * 33 + j];
-                            const float t = __fmaf_rn(xq[dd + j], v.x, v.y);
-                            acc = __fmaf_rn(t, t, acc);
-                        }
+                    for (int j = 0; j < 16; j++) {
+                        const float x0 = (j & 1) ? xv[j >> 1].z : xv[j >> 1].x, x1 = (j & 1) ? xv[j >> 1].w : xv[j >> 1].y;
+                        const float t0 = __fmaf_rn(x0, rr[j].x, rr[j].y);
+                        acc = __fmaf_rn(t0, t0, acc);
+                        const float t1 = __fmaf_rn(x1, rr[j].z, rr[j].w);
+                        acc = __fmaf_rn(t1, t1, acc);
+                    }
+                } else {
+                    for (int j = 0; j < D - dd; j++) {
+                        const float2 v = rv[j];
+                        const float t = __fmaf_rn(xs[j], v.x, v.y);
+                        acc = __fmaf_rn(t, t, acc);
                     }
                 }
-                __syncwarp();
             }
+            __syncwarp();  // the slot is refilled by the next issue
         }
-        if (b >= 0) outs[lo + lane] = -0.5f * (a.ix.sumlog[b] + acc);
-    };
-    auto exact_rows = [&](const int *list, int U, float *outs) {
-        if (U <= 0) return;
-        const int n_rounds = (U + FN_R - 1) / FN_R, rpr = (U + n_rounds - 1) / n_rounds;  // rows per round <= FN_R
-        for (int rd = warp; rd < n_rounds; rd += FN_WARPS) {
-            const int lo = rd * rpr, cnt = min(rpr, U - lo);
-            if (cnt <= 0) continue;
-            if (rpr <= 8) exact_round(std::integral_constant<int, 8>{}, list, lo, cnt, outs);
-            else exact_round(std::integral_constant<int, FN_R>{}, list, lo, cnt, outs);
-        }
-    };
-    // the rows a phase is about to score exactly are random 8 D-byte rows of a 0.8 GB array: ask for them in L2 as
-    // soon as the list is known, so that the segment loads of exact_rows find them there
-    auto prefetch_rows = [&](const int *list, int U) {
-        const int lines = (D * 8 + 127) / 128;
-        for (int i = tid; i < U * lines; i += FN_THREADS) {
-            const int b = list[i / lines];
-            if (b >= 0) asm volatile("prefetch.global.L2 [%0];" ::"l"(reinterpret_cast<const char *>(a.RM + (size_t)b * D) + (size_t)(i % lines) * 128));
-        }
-    };
+        if (lane < cnt) out[q * stride + lo + lane] = __fmul_rn(-0.5f, __fadd_rn(ix.sumlog[b], acc));
+    }
+}
 
-    int n_refined = 0, n_rescored = 0;  // counters of this CTA's queries, added to the stats once at the end
-    for (long long q = blockIdx.x; q < a.nq; q += gridDim.x) {
-        __syncthreads();
-        for (int d = tid; d < D; d += FN_THREADS) xq[d] = a.Q[q * D + d];
-        const int n_all = a.cnt[q];
-        const int n = min(n_all, cap);
-        for (int i = tid; i < n; i += FN_THREADS) { cv[i] = a.cand_val[q * cap + i]; cr[i] = a.cand_row[q * cap + i]; }
-        if (tid < 10) misc[tid] = tid == 4 ? 0x7fffffff : (tid == 5 ? float_key(NEG_INF) : 0);
-        for (int i = tid; i < KC1; i += FN_THREADS) ssel[i] = -1;
-        __syncthreads();
-        const float4 qq = a.qv[q];
-        const float eps = eps_of(qq.y, a.inv_prior, a.hmax, a.lmax, a.wfac, a.eps_scale, ML);
-        // ---- which candidates need the exact leaf term.  Every candidate has the interval [a1 - E, a1 + E] (E = e1[row] *
-        // ||a_q||, the filter's derived bound) around its leaf score with exact leaf term; L_k = the k-th largest lower end
-        // is a lower bound of the k-th best such score (k different leaves reach it), so a candidate whose upper end stays
-        // 3 eps below L_k cannot reach the line drawn further down and is dropped unrefined.  The rest -- the best KC1
-        // of them by a1 -- is refined.  U = the largest upper end among everything left unrefined (dropped or cut here,
-        // or rejected by the filter: below tau).
-        for (int i = tid; i < n; i += FN_THREADS) ce[i] = a.leaf_rc[cr[i] * 2 + 1].x * qq.z;
-        __syncthreads();
-        for (int i = tid; i < n; i += FN_THREADS) {
-            const float v = cv[i];
-            const int row = cr[i];
-            int rank = 0;
-            for (int j = 0; j < n; j++) rank += cv[j] > v || (cv[j] == v && cr[j] < row);
-            byrank[rank] = (unsigned short)i;
-            // L_k from the k candidates with the best a1 (any k different leaves give a valid lower bound)
-            if (rank < a.k) atomicMin(&misc[4], float_key(v - ce[i] - eps));
+// a3 = (C[parent] + w_leaf s) / len of the refined leaves, the k-th best sentence score A_k over them, the line
+// thr = A_k - 2 eps and its test against U, the survivors (a3 >= thr), and the distinct index rows on their paths
+// (the leaf itself is already scored).  A query that fails is flagged here for the exact small-batch path.
+__global__ void __launch_bounds__(FQ_WARPS * 32)
+fn_line_kernel(const FinArgs a) {
+    __shared__ float sa3_s[FQ_WARPS][KC1];
+    __shared__ int sns_s[FQ_WARPS][KC1];
+    __shared__ int spos_s[FQ_WARPS][MS], slen_s[FQ_WARPS][MS];
+    __shared__ int counts[2];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, ML = a.ix.max_len;
+    float *sa3 = sa3_s[warp];
+    int *sns = sns_s[warp], *spos = spos_s[warp], *slen = slen_s[warp];
+    const float NEG_INF = -__int_as_float(0x7f800000);
+    if (threadIdx.x < 2) counts[threadIdx.x] = 0;
+    __syncthreads();
+    const long long q = (long long)blockIdx.x * FQ_WARPS + warp;
+    if (q < a.nq) {
+        int *meta = a.meta + q * FM_STRIDE;
+        const int nsel = meta[FM_NSEL];
+        const float eps = __int_as_float(meta[FM_EPS]), U = __int_as_float(meta[FM_U]);
+        int fail = meta[FM_FAIL];
+        const int *rrow = a.ref_row + q * KC1;
+        for (int i = lane; i < nsel; i += 32) {
+            const int row = rrow[i];
+            const float4 r0 = a.leaf_rc[row * 2], r1 = a.leaf_rc[row * 2 + 1];
+            const int par = __float_as_int(r1.y);
+            const float c = par >= 0 ? a.C[(long long)par * a.ldq + q] : 0.0f;
+            sa3[i] = __fmul_rn(__fmaf_rn(r1.z, a.ref_s[q * KC1 + i], c), r0.w);
+            sns[i] = a.sent_off[row + 1] - a.sent_off[row];
         }
-        __syncthreads();
-        const float Lk = n >= a.k ? key_float(misc[4]) : NEG_INF;
-        if (warp == 0) {
-            // candidates in rank order: the kept ones are compacted into the refine list, the rest raises U
-            int count = 0;
-            float umax = NEG_INF;
-            for (int base = 0; base < n; base += 32) {
-                const int r = base + lane;
-                const int i = r < n ? byrank[r] : -1;
-                const bool keep = i >= 0 && cv[i] + ce[i] + 3.0f * eps >= Lk;
-                const unsigned mask = __ballot_sync(0xffffffffu, keep);
-                const int pos = count + __popc(mask & ((1u << lane) - 1u));
-                count += __popc(mask);
-                if (keep && pos < KC1) {
-                    const int row = cr[i];
-                    srow[pos] = row;
-                    sb[pos] = a.leaf_row_b[row];
-                    sns[pos] = a.sent_off[row + 1] - a.sent_off[row];
-                    const float4 r1 = a.leaf_rc[row * 2 + 1];
-                    swl[pos] = r1.z;
-                    slen[pos] = __float_as_int(r1.w);
-                } else if (i >= 0) {
-                    umax = fmaxf(umax, cv[i] + ce[i]);  // left unrefined
+        __syncwarp();
+        // A_k: the a3 of the leaf that holds the k-th sentence in (a3 desc, list position asc) order
+        bool found = false;
+        float Ak = 0.0f;
+        for (int i = lane; i < nsel; i += 32) {
+            const float v = sa3[i];
+            int before = 0;
+            for (int c = 0; c < nsel; c++)
+                if (sa3[c] > v || (sa3[c] == v && c < i)) before += sns[c];
+            if (before < a.k && before + sns[i] >= a.k) found = true, Ak = v;
+        }
+        const unsigned fm = __ballot_sync(0xffffffffu, found);
+        const float thr = fm ? __shfl_sync(0xffffffffu, Ak, __ffs(fm) - 1) - 2.0f * eps : NEG_INF;
+        // Everything unrefined scores (exactly) at most U + 2 eps, the k-th best exact score is at least A_k - eps: the
+        // answer is complete if U + 3 eps < A_k.  With fewer than k sentences among the refined leaves every one of
+        // them is needed and nothing may be left out (U = -inf).
+        if (!(thr - eps > U) && !(U == NEG_INF)) fail = fail ? fail : 2;
+        // survivors: refined leaves at or above the line, in list order
+        int m = 0, n_sent = 0;
+        for (int base = 0; base < nsel; base += 32) {
+            const int i = base + lane;
+            const bool surv = i < nsel && sa3[i] >= thr;
+            const unsigned mask = __ballot_sync(0xffffffffu, surv);
+            const int at = m + __popc(mask & ((1u << lane) - 1u));
+            if (surv) {
+                n_sent += sns[i];
+                if (at < MS) {
+                    meta[FM_SURV + at] = i;
+                    const int row = rrow[i];
+                    spos[at] = a.leaf_pos[row];
+                    slen[at] = __float_as_int(a.leaf_rc[row * 2 + 1].w);
                 }
             }
-            for (int off = 16; off > 0; off >>= 1) umax = fmaxf(umax, __shfl_xor_sync(0xffffffffu, umax, off));
-            if (lane == 0) { misc[7] = min(count, KC1); misc[5] = float_key(umax); }
+            m += __popc(mask);
         }
-        __syncthreads();
-        const int nsel = misc[7];
-        prefetch_rows(sb, nsel);
-        int fail = n_all > cap ? 1 : 0;  // candidate-buffer overflow
-        const float U = fmaxf(a.tau[q], key_float(misc[5]));
-        // ---- exact leaf terms of the selected candidates, a3 = (C[parent] + w s) / len
-        exact_rows(sb, nsel, ss);
-        __syncthreads();
-        if (tid < nsel) {
-            const float4 r0 = a.leaf_rc[srow[tid] * 2];
-            const int par = __float_as_int(a.leaf_rc[srow[tid] * 2 + 1].y);
-            const float c = par >= 0 ? a.C[(long long)par * a.ldq + q] : 0.0f;
-            sa3[tid] = fmaf(swl[tid], ss[tid], c) * r0.w;
-        }
-        __syncthreads();
-        // ---- k-th best sentence score A_k over the refined leaves, line thr = A_k - 2 eps
-        float thr = NEG_INF;
-        {
-            if (tid < nsel) {
-                const float v = sa3[tid];
-                int before = 0;
-                for (int c = 0; c < nsel; c++)
-                    if (sa3[c] > v || (sa3[c] == v && c < tid)) before += sns[c];
-                sbefore[tid] = before;
-                if (before < a.k && before + sns[tid] >= a.k) misc[8] = __float_as_int(v), misc[9] = 1;
-            }
-            __syncthreads();
-            if (misc[9]) thr = __int_as_float(misc[8]) - 2.0f * eps;
-            // Everything unrefined scores (exactly) at most U + 2 eps, the k-th best exact score is at least A_k - eps: the
-            // answer is complete if U + 3 eps < A_k.  With fewer than k sentences among the refined leaves every one of
-            // them is needed and nothing may be left out (U = -inf).
-            if (!(thr - eps > U) && !(U == NEG_INF)) fail = fail ? fail : 2;
-        }
-        // ---- survivors: refined leaves at or above the line
-        if (tid < nsel && sa3[tid] >= thr) {
-            const int at = atomicAdd(&misc[1], 1);
-            if (at < MS) { mc[at] = tid; ssel[tid] = at; }
-            atomicAdd(&misc[2], sns[tid]);
-        }
-        __syncthreads();
-        const int m = misc[1];
-        if (m > MS || misc[2] > MAXS) fail = fail ? fail : 3;
-        n_refined += nsel;
-        n_rescored += m;
+        n_sent = warp_sum(n_sent);
+        if (m > MS || n_sent > MAXS) fail = fail ? fail : 3;
+        if (lane == 0) { atomicAdd(&counts[0], nsel); atomicAdd(&counts[1], m); }
+        int nanc = 0;
         if (fail) {  // flagged: the exact small-batch path answers this query
-            if (tid == 0) {
+            if (lane == 0) {
                 const int at = atomicAdd(a.flag, 1);
                 a.flag[4 + at] = (int)q;
                 a.out_sid[q * a.k] = CW_SID_UNRESOLVED;
                 atomicAdd(a.stats + 0, 1);
                 atomicAdd(a.stats + 1 + fail, 1);
             }
-            continue;
-        }
-        // ---- (survivor, level) -> index row of the ancestors (the leaf itself is already scored); unique rows get a slot
-        const int E = m * ML;
-        for (int e = tid; e < E; e += FN_THREADS) {
-            const int c = e / ML, j = e - c * ML, sel = mc[c];
-            nid[e] = j < slen[sel] - 1 ? a.ix.path_idx[(size_t)a.leaf_pos[srow[sel]] * ML + j] : -1;
-        }
-        __syncthreads();
-        for (int e = tid; e < E; e += FN_THREADS) {
-            const int b = nid[e];
-            if (b < 0) continue;
-            const int c = e / ML, j = e - c * ML;
-            int f = 0;
-            while (nid[f * ML + j] != b) f++;  // first survivor through this node (f <= c)
-            firstc[e] = (unsigned short)f;
-            if (f == c) {
-                const int sl = atomicAdd(&misc[0], 1);
-                ulist[sl] = b;
-                slot[e] = (unsigned short)sl;
+            m = -1;
+        } else {
+            // (survivor, level) -> index row of the ancestor; the first survivor through a node gives it an entry
+            __syncwarp();
+            int *ab = a.anc_b + q * a.em, *slot = a.anc_slot + q * a.em;
+            const int *pidx = a.ix.path_idx;
+            auto node = [&](int c, int j) { return j < slen[c] - 1 ? pidx[(size_t)spos[c] * ML + j] : -1; };
+            const int E = m * ML;
+            for (int base = 0; base < E; base += 32) {
+                const int e = base + lane;
+                int b = -1, f = 0, c = 0, j = 0;
+                if (e < E) {
+                    c = e / ML, j = e - c * ML;
+                    b = node(c, j);
+                    if (b >= 0)
+                        while (node(f, j) != b) f++;  // first survivor through this node (f <= c)
+                }
+                const bool first = b >= 0 && f == c;
+                const unsigned mask = __ballot_sync(0xffffffffu, first);
+                if (first) {
+                    const int sl = nanc + __popc(mask & ((1u << lane) - 1u));
+                    ab[sl] = b;
+                    slot[e] = sl;
+                } else if (b >= 0) {
+                    slot[e] = -2 - (f * ML + j);  // resolved below, once every first entry has its slot
+                }
+                nanc += __popc(mask);
+            }
+            __syncwarp();
+            for (int e = lane; e < E; e += 32) {
+                const int v = slot[e];
+                if (v <= -2) slot[e] = slot[-2 - v];
             }
         }
-        __syncthreads();
-        for (int e = tid; e < E; e += FN_THREADS) {
-            if (nid[e] < 0) continue;
-            const int c = e / ML, j = e - c * ML, f = firstc[e];
-            if (f != c) slot[e] = slot[f * ML + j];
-        }
-        prefetch_rows(ulist, misc[0]);
-        exact_rows(ulist, misc[0], uscore);
-        __syncthreads();
-        // ---- exact leaf scores: sequential FMA along the path, root first, the leaf last (cw_dense_paths_topk's order)
-        if (tid < m) {
-            const int sel = mc[tid], len = slen[sel];
-            float acc = 0.0f;
-            for (int j = 0; j < len - 1; j++) acc = __fmaf_rn((float)(lw[j] / (double)len), uscore[slot[tid * ML + j]], acc);
-            mex[tid] = __fmaf_rn((float)(lw[len - 1] / (double)len), ss[sel], acc);
-        }
-        if (tid == 0) {  // sentence list offsets (m <= 32)
-            int off = 0;
-            for (int c = 0; c < m; c++) { mso[c] = off; off += sns[mc[c]]; }
-            misc[3] = off;
-        }
-        __syncthreads();
-        // ---- sentences of the survivors ranked by (score desc, sentence id asc)
-        const int ns_tot = misc[3];
-        for (int c = warp; c < m; c += FN_WARPS) {
-            const int row = srow[mc[c]], s0 = a.sent_off[row], cntc = sns[mc[c]];
-            for (int i = lane; i < cntc; i += 32) { lsid[mso[c] + i] = a.sent_ids[s0 + i]; lval[mso[c] + i] = mex[c]; }
-        }
-        __syncthreads();
-        for (int i = tid; i < ns_tot; i += FN_THREADS) {
-            const float v = lval[i];
-            const int sid = lsid[i];
-            int rank = 0;
-            for (int j = 0; j < ns_tot; j++) rank += lval[j] > v || (lval[j] == v && lsid[j] < sid);
-            if (rank < a.k) { a.out_sid[q * a.k + rank] = sid; a.out_val[q * a.k + rank] = v; }
-        }
-        for (int r = ns_tot + tid; r < a.k; r += FN_THREADS) {  // fewer than k sentences in the index
-            a.out_sid[q * a.k + r] = -1;
-            a.out_val[q * a.k + r] = NEG_INF;
-        }
+        if (lane == 0) { meta[FM_NANC] = nanc; meta[FM_M] = m; }
     }
-    if (tid == 0 && (n_refined | n_rescored)) { atomicAdd(a.stats + 10, n_refined); atomicAdd(a.stats + 11, n_rescored); }
+    __syncthreads();
+    // leaves refined and leaves re-scored, flagged queries included
+    if (threadIdx.x == 0 && (counts[0] | counts[1])) { atomicAdd(a.stats + 10, counts[0]); atomicAdd(a.stats + 11, counts[1]); }
 }
 
-__global__ void h_stats_kernel(const int *__restrict__ cnt, long long nq, int *stats) {
-    // candidates appended by the filter (64-bit total in words 5, 6), queries in word 7
-    unsigned long long s = 0;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nq; i += (long long)gridDim.x * blockDim.x) s += (unsigned)cnt[i];
-    for (int off = 16; off > 0; off >>= 1) s += __shfl_xor_sync(0xffffffffu, s, off);
-    if ((threadIdx.x & 31) == 0 && s) atomicAdd(reinterpret_cast<unsigned long long *>(stats + 6), s);
-    if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(stats + 5, (int)nq);
+// exact leaf scores of the survivors: sequential FMA along the path, root first, the leaf last (cw_dense_paths_topk's
+// order); their sentences ranked by (score desc, sentence id asc)
+__global__ void __launch_bounds__(FQ_WARPS * 32)
+fn_topk_kernel(const FinArgs a) {
+    __shared__ int lsid_s[FQ_WARPS][MAXS];
+    __shared__ float lval_s[FQ_WARPS][MAXS];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, ML = a.ix.max_len;
+    const long long q = (long long)blockIdx.x * FQ_WARPS + warp;
+    if (q >= a.nq) return;
+    const int *meta = a.meta + q * FM_STRIDE;
+    const int m = meta[FM_M];
+    if (m < 0) return;  // flagged
+    int *lsid = lsid_s[warp];
+    float *lval = lval_s[warp];
+    const float NEG_INF = -__int_as_float(0x7f800000);
+    int row = 0, ns = 0;
+    float mex = 0.0f;
+    if (lane < m) {  // m <= MS = 32
+        const int sel = meta[FM_SURV + lane];
+        row = a.ref_row[q * KC1 + sel];
+        const int len = __float_as_int(a.leaf_rc[row * 2 + 1].w);
+        const int *slot = a.anc_slot + q * a.em + lane * ML;
+        const float *as = a.anc_s + q * a.em;
+        float acc = 0.0f;
+#pragma unroll 1
+        for (int j = 0; j < len - 1; j++) acc = __fmaf_rn((float)(a.ix.level_w[j] / (double)len), as[slot[j]], acc);
+        mex = __fmaf_rn((float)(a.ix.level_w[len - 1] / (double)len), a.ref_s[q * KC1 + sel], acc);
+        ns = a.sent_off[row + 1] - a.sent_off[row];
+    }
+    int off = ns;  // inclusive prefix sum of the sentence counts
+    for (int d = 1; d < 32; d <<= 1) {
+        const int o = __shfl_up_sync(0xffffffffu, off, d);
+        if (lane >= d) off += o;
+    }
+    const int ns_tot = __shfl_sync(0xffffffffu, off, 31);
+    off -= ns;
+    for (int c = 0; c < m; c++) {
+        const int s0 = __shfl_sync(0xffffffffu, row, c), cntc = __shfl_sync(0xffffffffu, ns, c),
+                  o = __shfl_sync(0xffffffffu, off, c);
+        const float v = __shfl_sync(0xffffffffu, mex, c);
+        const int first = a.sent_off[s0];
+        for (int i = lane; i < cntc; i += 32) { lsid[o + i] = a.sent_ids[first + i]; lval[o + i] = v; }
+    }
+    __syncwarp();
+    for (int i = lane; i < ns_tot; i += 32) {
+        const float v = lval[i];
+        const int sid = lsid[i];
+        int rank = 0;
+        for (int j = 0; j < ns_tot; j++) rank += lval[j] > v || (lval[j] == v && lsid[j] < sid);
+        if (rank < a.k) { a.out_sid[q * a.k + rank] = sid; a.out_val[q * a.k + rank] = v; }
+    }
+    for (int r = ns_tot + lane; r < a.k; r += 32) {  // fewer than k sentences in the index
+        a.out_sid[q * a.k + r] = -1;
+        a.out_val[q * a.k + r] = NEG_INF;
+    }
 }
 
 __global__ void h_unresolved_kernel(const int *flag, int capacity, int *stats) {
@@ -1152,6 +1239,7 @@ __global__ void h_audit_cmp_kernel(const int *__restrict__ which, int n_a, int k
 
 using namespace cwh;
 
+extern "C" int64_t cw_fused_flag_words(int64_t cap_q, int32_t max_len) { return 4 + cap_q + CW_SMALL_Q + fin_words(cap_q, max_len); }
 extern "C" int cw_h_stages(int32_t D, int32_t layout, int32_t nprod) { return stages_of(D, layout, nprod); }
 extern "C" int64_t cw_h_b_bytes(int32_t n_rows, int32_t D, int32_t layout, int32_t nprod) {
     return (int64_t)((n_rows + TN - 1) / TN) * stages_of(D, layout, nprod) * SIDE;
@@ -1292,8 +1380,6 @@ static int fused_chunk(const cw_fused_index *fi, const cw_fused_work *w, const f
     mark(4);
     if ((rc = h_launch<1, EPI_FILTER>(&fi->leaves, w->A_leaf, nq, 0, fi->leaves.n_ntiles, epi, st))) return rc;
     mark(5);
-    h_stats_kernel<<<32, 256, 0, st>>>(w->cnt, nq, w->stats);
-
     FinArgs a;
     a.ix = fi->ix;
     a.RM = reinterpret_cast<const float2 *>(fi->rows);
@@ -1313,7 +1399,6 @@ static int fused_chunk(const cw_fused_index *fi, const cw_fused_work *w, const f
     a.sent_ids = fi->sent_ids;
     a.C = w->S;
     a.ldq = ldq;
-    a.e1max = fi->e1max;
     a.inv_prior = inv_prior;
     a.hmax = fi->hmax;
     a.lmax = fi->lmax;
@@ -1323,17 +1408,23 @@ static int fused_chunk(const cw_fused_index *fi, const cw_fused_work *w, const f
     a.out_val = out_val;
     a.flag = w->flag;
     a.stats = w->stats;
-    const size_t smem = fin_smem_bytes(D, fi->ix.max_len, w->cap);
-    if (smem > 200 * 1024) {
-        cw_set_error("cw_fused_predict: finish kernel needs %lld bytes of shared memory (D=%d max_len=%d cap=%d)", (long long)smem, D,
-                     fi->ix.max_len, w->cap);
-        return CW_E_ARG;
-    }
-    if ((rc = cw_check_cuda(cudaFuncSetAttribute(h_finish_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),
-                            "cw_fused: smem attribute")))
+    fin_carve(a, w->flag + 4 + w->cap_q + CW_SMALL_Q, w->cap_q, w->fin_ml);
+    // the candidates of a select warp sit in shared memory: at most FQ_WARPS x 2048 x 12 bytes (fused_args_ok bounds cap)
+    const int sel_smem = FQ_WARPS * w->cap * 12, ex_smem = EX_WARPS * EX_WARP_BYTES;
+    if ((rc = cw_check_cuda(cudaFuncSetAttribute(fn_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, sel_smem),
+                            "cw_fused: smem attribute")) ||
+        (rc = cw_check_cuda(cudaFuncSetAttribute(fn_exact_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ex_smem),
+                            "cw_fused: smem attribute")) ||
+        (rc = cw_check_cuda(cudaFuncSetAttribute(fn_exact_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
+                                                 cudaSharedmemCarveoutMaxShared),
+                            "cw_fused: carveout attribute")))
         return rc;
-    const unsigned grid = (unsigned)(nq < 148 * 32 ? nq : 148 * 32);
-    h_finish_kernel<<<grid, FN_THREADS, smem, st>>>(a);
+    const unsigned gq = (unsigned)((nq + FQ_WARPS - 1) / FQ_WARPS), gx = (unsigned)((nq + EX_WARPS - 1) / EX_WARPS);
+    fn_select_kernel<<<gq, FQ_WARPS * 32, sel_smem, st>>>(a);
+    fn_exact_kernel<<<gx, EX_WARPS * 32, ex_smem, st>>>(a.ix, a.RM, Q, nq, a.ref_b, a.meta, FM_NSEL, KC1, a.ref_s);
+    fn_line_kernel<<<gq, FQ_WARPS * 32, 0, st>>>(a);
+    fn_exact_kernel<<<gx, EX_WARPS * 32, ex_smem, st>>>(a.ix, a.RM, Q, nq, a.anc_b, a.meta, FM_NANC, a.em, a.anc_s);
+    fn_topk_kernel<<<gq, FQ_WARPS * 32, 0, st>>>(a);
     if ((rc = cw_check_cuda(cudaGetLastError(), "cw_fused_predict"))) return rc;
     mark(6);
     // flagged queries: exact small-batch path, driven by the device-side count
@@ -1373,7 +1464,8 @@ static bool fused_args_ok(const cw_fused_index *fi, const cw_fused_work *w, int 
     if (fi->n_sample_tiles < 0 || fi->n_sample_tiles > fi->leaves.n_ntiles) return false;
     if (w->cap_q < TQ || (w->cap_q % TQ) || w->ldq != w->cap_q || !w->A_leaf || (fi->n_int && (!w->A_int || !w->S)) || !w->qv ||
         !w->slots || !w->tau || w->cap < 4 || w->cap > 2048 || (w->cap & 3) || !w->cnt || !w->cand_val || !w->cand_row || !w->flag || !w->sm_Q ||
-        !w->sm_scores || !w->sm_scratch || !w->sm_sid || !w->sm_val || !w->sm_n || !w->stats)
+        !w->sm_scores || !w->sm_scratch || !w->sm_sid || !w->sm_val || !w->sm_n || !w->stats ||
+        w->fin_ml < fi->ix.max_len)
         return false;
     return true;
 }
@@ -1443,7 +1535,7 @@ extern "C" int cw_fused_predict_host(const cw_fused_index *fi, const cw_fused_wo
 
 // One chunk with CUDA events at the stage boundaries; synchronises.  stage_ms[CW_FUSED_STAGES]: query operands,
 // internal-row scores (fp16 x3), cumulative sums, sampled tiles + threshold, leaf filter (fp16 x1), finish (select /
-// refine / exact re-score), tail (device-side fallback rounds, audit).
+// refine / line test / exact re-score / top-k), tail (device-side fallback rounds, audit).
 extern "C" int cw_fused_profile(const cw_fused_index *fi, const cw_fused_work *w, const float *Q, int64_t nq, int k,
                                 int32_t *out_sid, float *out_val, float *stage_ms_host, void *stream) {
     if (!fused_args_ok(fi, w, k) || !Q || !out_sid || !out_val || !stage_ms_host || nq < 1 || nq > w->cap_q) {

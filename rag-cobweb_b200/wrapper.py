@@ -172,7 +172,7 @@ class DenseIndex:
         hx["sent_off"], hx["sent_ids"] = F["sent_off"], F["sent_ids"]
         fi.leaf_row_b, fi.leaf_pos = hx["leaf_rows"].data_ptr(), hx["leaf_pos"].data_ptr()
         fi.sent_off, fi.sent_ids = hx["sent_off"].data_ptr(), hx["sent_ids"].data_ptr()
-        # row-major {r, mb} rows: the operands of the exact arithmetic in the finish kernel
+        # row-major {r, mb} rows: the operands of the exact arithmetic in the finish stage
         hx["rows"] = torch.empty((self.nn, d, 2), dtype=torch.float32, device=dev)
         _lib.check(L.cw_index_rows_build(store, self.order.data_ptr(), self.nn, hx["rows"].data_ptr(), st),
                    "cw_index_rows_build")
@@ -249,7 +249,8 @@ class DenseIndex:
 
     def fused_chunk_queries(self):
         n_int_pad = (self.hx["n_int"] + _lib.H_TILE - 1) // _lib.H_TILE * _lib.H_TILE
-        return int(max(256, min(32768, self.SCORE_BUDGET_BYTES // (max(n_int_pad, 1) * 4)) // 256 * 256))
+        per_query = (max(n_int_pad, 1) + _lib.load().cw_fused_flag_words(1, self.max_len)) * 4  # node scores + finish lists
+        return int(max(256, min(32768, self.SCORE_BUDGET_BYTES // per_query) // 256 * 256))
 
     def fused_workspace(self, nq, k):
         """cw_fused_work for chunks of up to nq queries (rounded to whole tiles, at most fused_chunk_queries())."""
@@ -274,14 +275,14 @@ class DenseIndex:
             cnt=torch.zeros(cap_q, dtype=torch.int32, device=dev),
             cand_val=torch.empty((cap_q, cap), dtype=torch.float32, device=dev),
             cand_row=torch.empty((cap_q, cap), dtype=torch.int32, device=dev),
-            flag=torch.zeros(4 + cap_q + _lib.SMALL_Q, dtype=torch.int32, device=dev),
+            flag=torch.zeros(L.cw_fused_flag_words(cap_q, self.max_len), dtype=torch.int32, device=dev),
             sid=torch.empty((cap_q, k), dtype=torch.int32, device=dev),
             val=torch.empty((cap_q, k), dtype=torch.float32, device=dev),
             stats=torch.zeros(_lib.FUSED_STATS, dtype=torch.int32, device=dev),
             stats_host=torch.zeros(_lib.FUSED_STATS, dtype=torch.int32).pin_memory(),
         )
         w = _lib.CwFusedWork()
-        w.cap_q, w.ldq, w.cap = cap_q, cap_q, cap
+        w.cap_q, w.ldq, w.cap, w.fin_ml = cap_q, cap_q, cap, self.max_len
         w.Q_dev, w.A_int, w.A_leaf, w.qv, w.S = (hw[n].data_ptr() for n in ("Q", "A_int", "A_leaf", "qv", "S"))
         w.slots, w.tau, w.cnt, w.cand_val, w.cand_row = (hw[n].data_ptr() for n in ("slots", "tau", "cnt", "cand_val", "cand_row"))
         w.flag, w.out_sid_dev, w.out_val_dev, w.stats = (hw[n].data_ptr() for n in ("flag", "sid", "val", "stats"))
