@@ -117,7 +117,7 @@ def load():
     L.cw_h_a_bytes.argtypes = [i64, i32c, i32c, i32c]
     L.cw_h_stages.restype = i32c
     L.cw_h_stages.argtypes = [i32c, i32c, i32c]
-    L.cw_h_set_build.argtypes = [C.POINTER(CwStore), vp, vp, vp, C.POINTER(CwHSet), vp, vp, vp, vp, vp]
+    L.cw_h_set_build.argtypes = [C.POINTER(CwStore), vp, vp, vp, C.POINTER(CwHSet), vp, vp, vp, vp, vp, vp, vp]
     L.cw_h_rows_isotropic.argtypes = [C.POINTER(CwStore), vp, vp, i32c, vp, vp]
     L.cw_fused_flag_words.restype = i64
     L.cw_fused_flag_words.argtypes = [i64, i32c]

@@ -2,7 +2,9 @@
 // (src/cobweb/CobwebWrapper.py:210-265) on tcgen05 with fp16 operands ("fused" mode, DESIGN.md section 5).
 //
 //   s[q,n]    = -0.5*(sumlog[n] + sum_d (x_qd - mu_nd)^2 / var_nd) = h[n] - 0.5 * sum_f A[q,f] * B[n,f]
-//   leaf score sum_j (w_j/len) s_j = (C[parent] + w_leaf s_leaf) / len,  C[n] = C[parent(n)] + w_depth(n) s_n
+//   leaf score sum_j (w_j/len) s_j = (C[parent] + w_leaf s_leaf) / len,  C[n] = sum_{j in path(n)} w_j s_j
+//   C is linear in the row operands: C[n] = h'_n - 0.5 sum_f A[q,f] B'_n[f] with B'_n = sum_j w_j B_j, h'_n = sum_j w_j h_j,
+//   so the internal rows carry the path-summed operands and their scores are the ancestor sums.
 //
 // Two operand precisions, one kernel:
 //   NPROD = 3  every operand v (scaled by a per-row power of two into the fp16 range) is split v = hi + lo into two
@@ -171,7 +173,7 @@ __device__ __forceinline__ void tile_coords(long long t, int n_qtiles, int n_nti
 }
 
 // What the epilogue does with a finished 128 x 256 accumulator (lane = query, column = row of the operand set):
-//   EPI_NODE    s = h - 0.5 acc, written row-major: out[row * ldq + q]                        (internal rows)
+//   EPI_NODE    s = h - 0.5 acc, written row-major: out[row * ldq + q]     (internal rows: the ancestor sums C)
 //   EPI_TAU     leaf score a1 of the sampled leaf tiles; per query the maximum over the rows r with r % 32 == j goes
 //               to slot j (32 different leaves per query reach their slot values)
 //   EPI_FILTER  a1 and its upper bound a1 + e1[row] * ||a_q||; (a1, row) appended to the query's candidate buffer when
@@ -618,11 +620,15 @@ __device__ __forceinline__ float var_at(const cw_store &s, int node, float cnt, 
 }
 
 // Index rows: one warp per row of the operand set (rows past n_rows are zero padding of the last tile).
+// Internal rows (int_par given) hold their path sums B'_n = sum_{j in path(n)} w_j B_j, h'_n = sum_j w_j h_j, summed in
+// binary64 walking int_par up from the row, so that the score kernel's s = h' - 0.5 acc IS the ancestor sum
+// C[n] = sum_j w_j s_j.  Walking up needs no scratch (a level-by-level build would need a binary64 [n_int, 2D] buffer).
+// int_par[n] < n: the internal rows are ordered by depth.
 constexpr double C1 = 0.0009765625 * 1.002;  // 2^-10 + 2^-22 (two fp16 roundings per product), with slack for the fp32 conversions
 __global__ void __launch_bounds__(256)
 hn_build_kernel(cw_store s, const int *__restrict__ order, const int *__restrict__ rows, const float *__restrict__ sumlog,
-                cw_h_set hs, const float *__restrict__ leaf_w, const float *__restrict__ leaf_il,
-                const int *__restrict__ leaf_par, const int *__restrict__ leaf_len) {
+                cw_h_set hs, const int *__restrict__ int_par, const float *__restrict__ int_w, const float *__restrict__ leaf_w,
+                const float *__restrict__ leaf_il, const int *__restrict__ leaf_par, const int *__restrict__ leaf_len) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int row = blockIdx.x * 8 + warp;
     if (row >= hs.n_ntiles * TN) return;
@@ -631,17 +637,33 @@ hn_build_kernel(cw_store s, const int *__restrict__ order, const int *__restrict
     int node = 0, brow = 0;
     float cnt = 0.0f;
     if (valid) { brow = rows[row]; node = order[brow]; cnt = s.count[node]; }
+    // the rows whose operands make up this row's: the path for an internal row (weights int_w), the row itself (weight 1)
+    // for a leaf row.  A parent that is not an earlier row breaks the depth order the walk relies on: trap (the launch
+    // fails with an error) rather than return truncated sums.
+    auto up = [&](int j) {
+        if (!int_par) return -1;
+        const int p = int_par[j];
+        if (p >= j) __trap();
+        return p;
+    };
+    auto weight = [&](int j) { return int_par ? (double)int_w[j] : 1.0; };
     float mx = 0.0f;
     double b2 = 0.0, hsum = 0.0;
     if (valid) {
         for (int d = lane; d < D; d += 32) {
-            const double iv = 1.0 / (double)var_at(s, node, cnt, d);
-            const double mu = (double)s.mean[(size_t)node * D + d];
-            const double m = -2.0 * mu * iv;
+            // w = 1 (a leaf row, one step) multiplies and adds to 0 exactly: the row's own operands bit for bit
+            double iv = 0.0, m = 0.0;
+            for (int j = row; j >= 0; j = up(j)) {
+                const int nj = order[rows[j]];
+                const double w = weight(j), ivj = 1.0 / (double)var_at(s, nj, s.count[nj], d);
+                const double mu = (double)s.mean[(size_t)nj * D + d];
+                iv += w * ivj;
+                m += w * (-2.0 * mu * ivj);
+                hsum += w * mu * mu * ivj;
+            }
             mx = fmaxf(mx, (float)fabs(m) * (1.0f + 1e-6f));
             b2 += m * m;
-            hsum += mu * mu * iv;
-            if (layout == CW_H_F2) { mx = fmaxf(mx, (float)iv * (1.0f + 1e-6f)); b2 += iv * iv; }
+            if (layout == CW_H_F2) { mx = fmaxf(mx, (float)fabs(iv) * (1.0f + 1e-6f)); b2 += iv * iv; }
         }
     }
     mx = warp_max(mx);
@@ -653,22 +675,33 @@ hn_build_kernel(cw_store s, const int *__restrict__ order, const int *__restrict
     const int n_sl = slabs_of(D, layout), n_sl_pad = nprod == 3 ? n_sl : (n_sl + 1) & ~1;
     unsigned char *Bset = reinterpret_cast<unsigned char *>(hs.B);
     for (int slab = lane >> 2; slab < n_sl_pad; slab += 8) {
+        double t[8] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+        if (valid && slab < n_sl) {
+            for (int j = row; j >= 0; j = up(j)) {
+                const int nj = order[rows[j]];
+                const float cj = s.count[nj];
+                const double w = weight(j);
+#pragma unroll
+                for (int e = 0; e < 8; e++) {
+                    const int d = layout == CW_H_F1 ? slab * 32 + c * 8 + e : slab * 16 + (c & 1) * 8 + e;
+                    if (d < D) {
+                        const double ivj = 1.0 / (double)var_at(s, nj, cj, d);
+                        t[e] += (layout == CW_H_F2 && c < 2) ? w * ivj : w * (-2.0 * (double)s.mean[(size_t)nj * D + d] * ivj);
+                    }
+                }
+            }
+        }
         float v[8];
 #pragma unroll
-        for (int e = 0; e < 8; e++) {
-            const int d = layout == CW_H_F1 ? slab * 32 + c * 8 + e : slab * 16 + (c & 1) * 8 + e;
-            double t = 0.0;
-            if (valid && slab < n_sl && d < D) {
-                const double iv = 1.0 / (double)var_at(s, node, cnt, d);
-                t = (layout == CW_H_F2 && c < 2) ? iv : -2.0 * (double)s.mean[(size_t)node * D + d] * iv;
-            }
-            v[e] = (float)(t * mul);
-        }
+        for (int e = 0; e < 8; e++) v[e] = (float)(t[e] * mul);
         unsigned char *hi = nprod == 3 ? Bset + ((size_t)(tile * n_sl + slab) * 2) * IMG : Bset + (size_t)(tile * n_sl_pad + slab) * IMG;
         store_chunk(hi, nprod == 3 ? hi + IMG : nullptr, swz_off(r, c), v);
     }
     if (lane == 0) {
-        const double h = valid ? -0.5 * ((double)sumlog[brow] + hsum) : 0.0;
+        double lsum = 0.0;  // sum_j w_j sumlog_j
+        if (valid)
+            for (int j = row; j >= 0; j = up(j)) lsum += weight(j) * (double)sumlog[rows[j]];
+        const double h = valid ? -0.5 * (lsum + hsum) : 0.0;
         if (nprod == 3) {
             reinterpret_cast<float2 *>(hs.rc)[row] = make_float2((float)h, valid ? (float)(-0.5 * ldexp(1.0, -sb)) : 0.0f);
         } else {
@@ -704,48 +737,6 @@ h_iso_kernel(cw_store s, const int *__restrict__ order, const int *__restrict__ 
     bool same = true;
     for (int d = lane; d < s.D; d += 32) same = same && var_at(s, node, cnt, d) == v0;
     if (!__all_sync(0xffffffffu, same) && lane == 0) atomicExch(flag, 0);
-}
-
-// ------------------------------------------------------------------ cumulative ancestor sums, one launch
-// C[n][q] = C[parent(n)][q] + w_n * S[n][q] in place on S.  A CTA owns a strip of 32 queries and walks the internal
-// rows level by level (rows of one level are independent; the parents of level l are in level l-1, which this CTA
-// finished before the barrier).
-constexpr int CS_COLS = 32;
-__global__ void __launch_bounds__(256)
-h_cumsum_kernel(float *S, long long ldq, const int *__restrict__ int_parent, const float *__restrict__ int_w,
-                const int *__restrict__ level_off, int n_levels) {
-    const int q4 = blockIdx.x * CS_COLS + (threadIdx.x & 7) * 4;
-    if (q4 >= ldq) return;
-    const int rl = threadIdx.x >> 3;  // 32 rows per pass
-    for (int l = 0; l < n_levels; l++) {
-        const int r0 = level_off[l], r1 = level_off[l + 1];
-        for (int rb = r0 + rl; rb < r1; rb += 128) {
-            float4 sv[4], cv[4];
-            float w[4];
-#pragma unroll
-            for (int u = 0; u < 4; u++) {
-                const int n = rb + 32 * u;
-                cv[u] = make_float4(0.f, 0.f, 0.f, 0.f);
-                if (n < r1) {
-                    const int par = int_parent[n];
-                    w[u] = int_w[n];
-                    sv[u] = *reinterpret_cast<const float4 *>(S + (long long)n * ldq + q4);
-                    if (par >= 0) cv[u] = *reinterpret_cast<const float4 *>(S + (long long)par * ldq + q4);
-                }
-            }
-#pragma unroll
-            for (int u = 0; u < 4; u++) {
-                const int n = rb + 32 * u;
-                if (n < r1) {
-                    float4 o;
-                    o.x = fmaf(w[u], sv[u].x, cv[u].x); o.y = fmaf(w[u], sv[u].y, cv[u].y);
-                    o.z = fmaf(w[u], sv[u].z, cv[u].z); o.w = fmaf(w[u], sv[u].w, cv[u].w);
-                    *reinterpret_cast<float4 *>(S + (long long)n * ldq + q4) = o;
-                }
-            }
-        }
-        __syncthreads();
-    }
 }
 
 // ------------------------------------------------------------------ filter threshold
@@ -1254,16 +1245,17 @@ static bool set_ok(const cw_h_set *hs, int D) {
 }
 
 extern "C" int cw_h_set_build(const cw_store *s, const int32_t *order, const int32_t *rows, const float *sumlog, const cw_h_set *hs,
-                              const float *leaf_w, const float *leaf_inv_len, const int32_t *leaf_parent, const int32_t *leaf_len,
-                              void *stream) {
+                              const int32_t *int_parent, const float *int_w, const float *leaf_w, const float *leaf_inv_len,
+                              const int32_t *leaf_parent, const int32_t *leaf_len, void *stream) {
     if (!s || !order || !rows || !sumlog || !set_ok(hs, s->D) ||
-        (hs->nprod == 1 && (!leaf_w || !leaf_inv_len || !leaf_parent || !leaf_len))) {
+        (hs->nprod == 3 && (!int_parent || !int_w)) ||
+        (hs->nprod == 1 && (int_parent || int_w || !leaf_w || !leaf_inv_len || !leaf_parent || !leaf_len))) {
         cw_set_error("cw_h_set_build: bad argument / inconsistent header");
         return CW_E_ARG;
     }
     const int n_pad = hs->n_ntiles * TN;
-    hn_build_kernel<<<(n_pad + 7) / 8, 256, 0, (cudaStream_t)stream>>>(*s, order, rows, sumlog, *hs, leaf_w, leaf_inv_len, leaf_parent,
-                                                                      leaf_len);
+    hn_build_kernel<<<(n_pad + 7) / 8, 256, 0, (cudaStream_t)stream>>>(*s, order, rows, sumlog, *hs, int_parent, int_w, leaf_w,
+                                                                      leaf_inv_len, leaf_parent, leaf_len);
     return cw_check_cuda(cudaGetLastError(), "cw_h_set_build");
 }
 
@@ -1359,11 +1351,8 @@ static int fused_chunk(const cw_fused_index *fi, const cw_fused_work *w, const f
         epi.rc = fi->internal.rc;
         epi.n_rows = fi->internal.n_rows;
         if ((rc = h_launch<3, EPI_NODE>(&fi->internal, w->A_int, nq, 0, fi->internal.n_ntiles, epi, st))) return rc;
-        mark(2);
-        const int strips = (int)((n_pad + CS_COLS - 1) / CS_COLS);
-        h_cumsum_kernel<<<strips, 256, 0, st>>>(w->S, ldq, fi->int_parent, fi->int_w, fi->level_off, fi->n_levels);
     }
-    if (!fi->n_int) mark(2);
+    mark(2);  // the internal operands are path sums: S holds the ancestor sums C already, this stage is empty
     mark(3);
     epi.rc = fi->leaves.rc;
     epi.n_rows = fi->leaves.n_rows;
@@ -1459,7 +1448,7 @@ static bool fused_args_ok(const cw_fused_index *fi, const cw_fused_work *w, int 
         return false;
     if (!set_ok(&fi->leaves, fi->ix.D) || fi->leaves.nprod != 1 || fi->leaves.n_rows != fi->n_leaf) return false;
     if (fi->n_int && (!set_ok(&fi->internal, fi->ix.D) || fi->internal.nprod != 3 || fi->internal.layout != CW_H_F2 ||
-                      fi->internal.n_rows != fi->n_int || !fi->int_parent || !fi->int_w || !fi->level_off || fi->n_levels < 1))
+                      fi->internal.n_rows != fi->n_int))
         return false;
     if (fi->n_sample_tiles < 0 || fi->n_sample_tiles > fi->leaves.n_ntiles) return false;
     if (w->cap_q < TQ || (w->cap_q % TQ) || w->ldq != w->cap_q || !w->A_leaf || (fi->n_int && (!w->A_int || !w->S)) || !w->qv ||
@@ -1534,7 +1523,8 @@ extern "C" int cw_fused_predict_host(const cw_fused_index *fi, const cw_fused_wo
 }
 
 // One chunk with CUDA events at the stage boundaries; synchronises.  stage_ms[CW_FUSED_STAGES]: query operands,
-// internal-row scores (fp16 x3), cumulative sums, sampled tiles + threshold, leaf filter (fp16 x1), finish (select /
+// internal-row scores (fp16 x3, the ancestor sums), cumulative sums (empty: kept so the stage list stays the same),
+// sampled tiles + threshold, leaf filter (fp16 x1), finish (select /
 // refine / line test / exact re-score / top-k), tail (device-side fallback rounds, audit).
 extern "C" int cw_fused_profile(const cw_fused_index *fi, const cw_fused_work *w, const float *Q, int64_t nq, int k,
                                 int32_t *out_sid, float *out_val, float *stage_ms_host, void *stream) {

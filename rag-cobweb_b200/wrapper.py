@@ -31,8 +31,8 @@ class DenseIndex:
     # How the top-k of a query batch is computed (ids and scores are the same bit for bit in both modes):
     #   "fp32"   every (query, node) score on the FP32 pipe, (x*r + mb)^2 per triple (cw_dense.cu), path product and
     #            top-k over the [nodes, queries] score matrix: the form that DEFINES the result;
-    #   "fused"  tcgen05 fp16 pipeline (cw_half.cu): internal rows with split operands (hi + lo, three products) ->
-    #            cumulative ancestor sums; leaf rows with ONE fp16 product as a filter with a derived error bound;
+    #   "fused"  tcgen05 fp16 pipeline (cw_half.cu): internal rows with path-summed split operands (hi + lo, three
+    #            products), whose scores are the ancestor sums; leaf rows with ONE fp16 product as a filter with a derived error bound;
     #            the survivors are re-scored with the FP32 form's exact arithmetic; queries the device cannot decide
     #            (and an always-on audit sample) go through the exact small-batch path.
     # Batches of up to SMALL_Q queries take the exact small-batch path in every mode (one query: HBM-bound).
@@ -145,14 +145,14 @@ class DenseIndex:
             _lib.check(iso, "cw_h_rows_isotropic")
         hx["leaf_layout"] = _lib.H_F1 if iso == 1 else _lib.H_F2
 
-        def hset(rows_t, n_rows, layout, nprod, leaf):
+        def hset(rows_t, n_rows, layout, nprod, internal, leaf):
             hs = _lib.CwHSet()
             hs.n_rows, hs.n_ntiles = n_rows, (n_rows + _lib.H_TILE - 1) // _lib.H_TILE
             hs.n_stages, hs.nprod, hs.layout = L.cw_h_stages(d, layout, nprod), nprod, layout
             B = torch.empty(L.cw_h_b_bytes(n_rows, d, layout, nprod), dtype=torch.uint8, device=dev)
             rc = torch.empty(hs.n_ntiles * _lib.H_TILE * (2 if nprod == 3 else 8), dtype=torch.float32, device=dev)
             hs.B, hs.rc = B.data_ptr(), rc.data_ptr()
-            ptrs = [t.data_ptr() for t in leaf] if leaf else [None] * 4
+            ptrs = [t.data_ptr() if t is not None else None for t in internal + leaf]
             _lib.check(L.cw_h_set_build(store, self.order.data_ptr(), rows_t.data_ptr(), self.sumlog.data_ptr(), C.byref(hs),
                                         *ptrs, st), "cw_h_set_build")
             return hs, B, rc
@@ -162,12 +162,14 @@ class DenseIndex:
         fi.n_int, fi.n_leaf, fi.n_sample_tiles = n_int, n_leaf, hx["n_s"]
         if n_int:
             hx["int_rows"] = F["int_rows"]
-            fi.internal, hx["B_int"], hx["rc_int"] = hset(hx["int_rows"], n_int, _lib.H_F2, 3, None)
+            # internal rows: operands summed along the path with the level weights (their scores are the ancestor sums)
+            fi.internal, hx["B_int"], hx["rc_int"] = hset(hx["int_rows"], n_int, _lib.H_F2, 3, [F["int_parent"], F["int_w"]],
+                                                          [None] * 4)
             hx["int_parent"], hx["int_w"], hx["level_off"] = F["int_parent"], F["int_w"], F["level_off"]
             fi.int_parent, fi.int_w, fi.level_off = hx["int_parent"].data_ptr(), hx["int_w"].data_ptr(), hx["level_off"].data_ptr()
             fi.n_levels = int(F["level_off"].numel()) - 1
         hx["leaf_aux"] = [F["leaf_w"], F["leaf_inv_len"], F["leaf_parent"], F["leaf_len"]]
-        fi.leaves, hx["B_leaf"], hx["rc_leaf"] = hset(hx["leaf_rows"], n_leaf, hx["leaf_layout"], 1, hx["leaf_aux"])
+        fi.leaves, hx["B_leaf"], hx["rc_leaf"] = hset(hx["leaf_rows"], n_leaf, hx["leaf_layout"], 1, [None] * 2, hx["leaf_aux"])
         hx["leaf_pos"] = torch.searchsorted(self._pos_leaf_row, F["leaf_rows"].to(torch.int64)).to(torch.int32)
         hx["sent_off"], hx["sent_ids"] = F["sent_off"], F["sent_ids"]
         fi.leaf_row_b, fi.leaf_pos = hx["leaf_rows"].data_ptr(), hx["leaf_pos"].data_ptr()

@@ -15,7 +15,7 @@ python bench.py --steps 2 --warmup 1 --no-cpu-baseline > gpurun_out/plain.log 2>
 ncu --metrics gpu__time_duration.sum --clock-control none -c 3000 --csv --log-file gpurun_out/${tag}_launches.csv \
     python bench.py --steps 2 --warmup 1 --no-cpu-baseline > gpurun_out/ncu_launches.log 2>&1
 python tools/fused_once.py > gpurun_out/once.log 2>&1 &&
-ncu --set full --import-source on --clock-control none -k regex:"h_score_kernel|h_finish|h_cumsum|hq_build|small_scores|paths_small" -s 12 -c 10 \
+ncu --set full --import-source on --clock-control none -k regex:"h_score_kernel|fn_|hq_build|small_scores|paths_small" -s 12 -c 10 \
     -o gpurun_out/${tag}_fused python tools/fused_once.py > gpurun_out/ncu_full.log 2>&1
 tail -2 gpurun_out/ncu_full.log
 python tools/ifit_small.py 3000 768 unit > gpurun_out/ifit_small.log 2>&1 &&

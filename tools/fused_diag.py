@@ -1,5 +1,6 @@
 """Stage-by-stage check of the fused tcgen05 predict (cw_half.cu) against the FP32 form on one tree:
-cumulative ancestor sums, filter scores and their error bound, candidate counts, final ids/scores, timing.
+cumulative ancestor sums (against a float64 sum of the FP32 node scores, and as a fraction of eps), filter scores and
+their error bound, candidate counts, final ids/scores, timing.
   python tools/fused_diag.py [docs] [dim] [unit|whitened] [queries] [k]"""
 import ctypes as C
 import os
@@ -53,6 +54,13 @@ if hx["n_int"]:
     err = (Cgot - Cref).abs()
     print(f"cumulative sums: max abs err {float(err.max()):.3e} (max |C| {float(Cref.abs().max()):.3f}); root row err "
           f"{float(err[0].max()):.3e}", flush=True)
+    # against eps of each query (cw_half.cu eps_of); C enters a leaf score divided by the path length, which is left out
+    fi = hx["fi"]
+    tq = 2.0 * ((qd.double() ** 2).sum(1) / fi.prior_var + fi.hmax)
+    op = fi.wfac * fi.eps_scale * tq
+    eps = op + fi.wfac * 2.0 ** -23 * (4.0 + 3.0 * ix.max_len ** 0.5) * 0.5 * (fi.lmax + fi.hmax + tq)
+    print(f"cumulative sums vs eps: max |C - C_ref| / eps {float((err / eps[None, :]).max()):.4f}, / eps operand term "
+          f"(eps_scale T wfac) {float((err / op[None, :]).max()):.4f}", flush=True)
 # ---- filter candidates: a1 vs the exact leaf score, against the bound
 cnt = hw["cnt"][:nq].cpu().numpy()
 print(f"candidates per query: mean {cnt.mean():.1f} median {np.median(cnt):.0f} max {cnt.max()} (cap {ix.FUSED_CAP})", flush=True)
