@@ -19,13 +19,14 @@ TILE_N, TILE_K, MAX_K, MAX_D, MAX_CHILDREN = 128, 16, 128, 4096, 2048
 IFIT_NODE_SLACK, IFIT_POOL_SLACK = 160, 16384
 H_TILE, H_F1, H_F2 = 256, 1, 2
 FUSED_MAX_K, FUSED_FB_ROUNDS, SMALL_Q, SID_UNRESOLVED, FUSED_STATS, FUSED_STAGES = 30, 2, 32, -2, 12, 7
+PAIR_MAX_M, PAIR_MAX_LEN = 1024, 1024
 
 EXPORTS = ["cw_version", "cw_last_error", "cw_store_init", "cw_store_derive", "cw_ifit", "cw_set_ifit_cluster", "cw_selftest_arith", "cw_categorize_ctas", "cw_categorize",
            "cw_index_build", "cw_xt_floats", "cw_score_ldq", "cw_dense_node_scores", "cw_topk_chunks", "cw_dense_paths_topk",
            "cw_predict_dense_host", "cw_index_rows_build",
            "cw_h_b_bytes", "cw_h_a_bytes", "cw_h_stages", "cw_h_set_build", "cw_h_rows_isotropic", "cw_fused_flag_words", "cw_fused_predict",
            "cw_fused_predict_host", "cw_fused_profile", "cw_small_scratch_words", "cw_small_predict", "cw_small_predict_host",
-           "cw_rank_scores_bwd", "cw_whiten", "cw_ffma_peak", "cw_ffma2_peak"]
+           "cw_rank_scores_bwd", "cw_pair_scratch_words", "cw_pair_scores", "cw_pair_scores_bwd", "cw_whiten", "cw_ffma_peak", "cw_ffma2_peak"]
 
 
 class CwStore(C.Structure):
@@ -129,6 +130,10 @@ def load():
     L.cw_small_predict.argtypes = [C.POINTER(CwIndex), vp, i64, vp, vp, i32c, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.cw_small_predict_host.argtypes = [C.POINTER(CwIndex), vp, i64, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.cw_rank_scores_bwd.argtypes = [C.POINTER(CwIndex), vp, i64, vp, vp, i64, vp, vp]
+    L.cw_pair_scratch_words.restype = i64
+    L.cw_pair_scratch_words.argtypes = [i64, i32c, i32c]
+    L.cw_pair_scores.argtypes = [C.POINTER(CwIndex), vp, vp, i32c, vp, i64, vp, i32c, vp, vp, vp]
+    L.cw_pair_scores_bwd.argtypes = [C.POINTER(CwIndex), vp, vp, i32c, vp, i64, vp, i32c, vp, vp, vp, vp]
     L.cw_whiten.argtypes = [vp, i64, C.c_int32, vp, vp, C.c_int32, vp, vp, vp, vp, vp]
     L.cw_ffma_peak.argtypes = [i32, i32, i32, vp, vp]
     L.cw_ffma2_peak.argtypes = [i32, i32, i32, vp, vp]

@@ -22,6 +22,7 @@ UNITS = [
     ("cw_half.cu", []),
     ("cw_whiten.cu", []),
     ("cw_grad.cu", []),
+    ("cw_pairs.cu", []),
 ]
 
 

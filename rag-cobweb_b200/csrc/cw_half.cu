@@ -950,7 +950,9 @@ __device__ __forceinline__ void cp_async4(void *dst, const void *src) {
 }
 
 // Exact node scores with the FP32 path's arithmetic: out[q * stride + i] = -0.5 (sumlog[b] + sum_d (x_qd r_bd + mb_bd)^2)
-// for b = list[q * stride + i], i < meta[q][n_word].  One warp per query; its rows go in rounds of at most EX_R.  For the
+// for b = list[q * stride + i], i < n = meta[q * meta_stride + n_word].  One warp per (query, row block): blockIdx.y
+// takes rows [y * per, (y + 1) * per) with per = max(EX_R, ceil(n / gridDim.y)), so a long list is spread over several
+// warps (gridDim.y = 1: one warp takes the whole list); a warp's rows go in rounds of at most EX_R.  For the
 // arithmetic lane = row (every lane runs its row's FMA chain in ascending d from 0, so the result is bit-identical to
 // dense_score_kernel), for the loads lane = attribute: per 32 attributes of a row one coalesced 256-byte cp.async
 // segment into a ring of EX_STAGES segments, EX_STAGES - 1 ahead of the arithmetic.  A row's segment is padded to
@@ -961,19 +963,22 @@ constexpr int EX_WARPS = 4, EX_R = 16, EX_STAGES = 4, EX_RS = 34;
 constexpr int EX_WARP_BYTES = EX_STAGES * EX_R * EX_RS * 8 + EX_STAGES * 32 * 4;
 __global__ void __launch_bounds__(EX_WARPS * 32)
 fn_exact_kernel(const cw_index ix, const float2 *__restrict__ RM, const float *__restrict__ Q, long long nq,
-                const int *__restrict__ list, const int *__restrict__ meta, int n_word, int stride, float *out) {
+                const int *__restrict__ list, const int *__restrict__ meta, int meta_stride, int n_word, int stride,
+                float *out) {
     extern __shared__ __align__(16) unsigned char ex_smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, D = ix.D;
     float2 *ring = reinterpret_cast<float2 *>(ex_smem + (size_t)warp * EX_WARP_BYTES);  // [EX_STAGES][EX_R][EX_RS]
     float *xr = reinterpret_cast<float *>(ring + EX_STAGES * EX_R * EX_RS);             // [EX_STAGES][32]
     const long long q = (long long)blockIdx.x * EX_WARPS + warp;
     if (q >= nq) return;
-    const int n = meta[q * FM_STRIDE + n_word];
-    if (n <= 0) return;
+    const int n_all = meta[q * meta_stride + n_word];
+    const int per = max(EX_R, (n_all + (int)gridDim.y - 1) / (int)gridDim.y), first = (int)blockIdx.y * per;
+    if (first >= n_all) return;
+    const int n = min(n_all, first + per);  // rows [first, n)
     const float *xq = Q + q * D;
     const int n_seg = (D + 31) / 32;
-    const int n_rounds = (n + EX_R - 1) / EX_R, rpr = (n + n_rounds - 1) / n_rounds;  // rows per round <= EX_R
-    for (int lo = 0; lo < n; lo += rpr) {
+    const int n_rounds = (n - first + EX_R - 1) / EX_R, rpr = (n - first + n_rounds - 1) / n_rounds;  // rows per round <= EX_R
+    for (int lo = first; lo < n; lo += rpr) {
         const int cnt = min(rpr, n - lo);
         const int b = lane < cnt ? list[q * stride + lo + lane] : 0;
         auto issue = [&](int seg) {
@@ -1230,6 +1235,23 @@ __global__ void h_audit_cmp_kernel(const int *__restrict__ which, int n_a, int k
 
 using namespace cwh;
 
+// fn_exact_kernel for other translation units (cw_pairs.cu); the attributes are per device, so they are set per call
+int cw_exact_rows_attr() {
+    int rc = cw_check_cuda(cudaFuncSetAttribute(fn_exact_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                EX_WARPS * EX_WARP_BYTES), "cw_exact_rows: smem attribute");
+    if (!rc)
+        rc = cw_check_cuda(cudaFuncSetAttribute(fn_exact_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
+                                                cudaSharedmemCarveoutMaxShared), "cw_exact_rows: carveout attribute");
+    return rc;
+}
+void cw_exact_rows_launch(const cw_index &ix, const float2 *RM, const float *Q, long long nq, const int *list,
+                          const int *meta, int meta_stride, int n_word, int stride, float *out, int row_blocks,
+                          cudaStream_t st) {
+    const dim3 grid((unsigned)((nq + EX_WARPS - 1) / EX_WARPS), (unsigned)row_blocks);
+    fn_exact_kernel<<<grid, EX_WARPS * 32, EX_WARPS * EX_WARP_BYTES, st>>>(ix, RM, Q, nq, list, meta, meta_stride, n_word,
+                                                                          stride, out);
+}
+
 extern "C" int64_t cw_fused_flag_words(int64_t cap_q, int32_t max_len) { return 4 + cap_q + CW_SMALL_Q + fin_words(cap_q, max_len); }
 extern "C" int cw_h_stages(int32_t D, int32_t layout, int32_t nprod) { return stages_of(D, layout, nprod); }
 extern "C" int64_t cw_h_b_bytes(int32_t n_rows, int32_t D, int32_t layout, int32_t nprod) {
@@ -1399,20 +1421,16 @@ static int fused_chunk(const cw_fused_index *fi, const cw_fused_work *w, const f
     a.stats = w->stats;
     fin_carve(a, w->flag + 4 + w->cap_q + CW_SMALL_Q, w->cap_q, w->fin_ml);
     // the candidates of a select warp sit in shared memory: at most FQ_WARPS x 2048 x 12 bytes (fused_args_ok bounds cap)
-    const int sel_smem = FQ_WARPS * w->cap * 12, ex_smem = EX_WARPS * EX_WARP_BYTES;
+    const int sel_smem = FQ_WARPS * w->cap * 12;
     if ((rc = cw_check_cuda(cudaFuncSetAttribute(fn_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, sel_smem),
                             "cw_fused: smem attribute")) ||
-        (rc = cw_check_cuda(cudaFuncSetAttribute(fn_exact_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ex_smem),
-                            "cw_fused: smem attribute")) ||
-        (rc = cw_check_cuda(cudaFuncSetAttribute(fn_exact_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                                 cudaSharedmemCarveoutMaxShared),
-                            "cw_fused: carveout attribute")))
+        (rc = cw_exact_rows_attr()))
         return rc;
-    const unsigned gq = (unsigned)((nq + FQ_WARPS - 1) / FQ_WARPS), gx = (unsigned)((nq + EX_WARPS - 1) / EX_WARPS);
+    const unsigned gq = (unsigned)((nq + FQ_WARPS - 1) / FQ_WARPS);
     fn_select_kernel<<<gq, FQ_WARPS * 32, sel_smem, st>>>(a);
-    fn_exact_kernel<<<gx, EX_WARPS * 32, ex_smem, st>>>(a.ix, a.RM, Q, nq, a.ref_b, a.meta, FM_NSEL, KC1, a.ref_s);
+    cw_exact_rows_launch(a.ix, a.RM, Q, nq, a.ref_b, a.meta, FM_STRIDE, FM_NSEL, KC1, a.ref_s, 1, st);
     fn_line_kernel<<<gq, FQ_WARPS * 32, 0, st>>>(a);
-    fn_exact_kernel<<<gx, EX_WARPS * 32, ex_smem, st>>>(a.ix, a.RM, Q, nq, a.anc_b, a.meta, FM_NANC, a.em, a.anc_s);
+    cw_exact_rows_launch(a.ix, a.RM, Q, nq, a.anc_b, a.meta, FM_STRIDE, FM_NANC, a.em, a.anc_s, 1, st);
     fn_topk_kernel<<<gq, FQ_WARPS * 32, 0, st>>>(a);
     if ((rc = cw_check_cuda(cudaGetLastError(), "cw_fused_predict"))) return rc;
     mark(6);

@@ -41,6 +41,7 @@ class DenseIndex:
     TENSOR_MIN_NODES = 16384      # smaller indexes are answered on the FP32 pipe (launch-bound there; same result)
     EPS_SCALE = 2.0 ** -18        # |fp16x3 ancestor sums - fp32| relative to the operand magnitudes (cw_half.cu eps_of)
     AUDIT_EVERY = 2048            # one query in AUDIT_EVERY is answered again by the exact path and compared (0 = off)
+    PAIR_BUDGET_BYTES = 4 << 30   # pair-scoring scratch per query chunk (row lists, their scores, the level maps)
 
     def __init__(self, tree, leaf_of_sentence, level_weights=None, sentence_ids=None):
         """leaf_of_sentence[i] = leaf node id of sentence i.  sentence_ids (optional, sorted global
@@ -102,6 +103,8 @@ class DenseIndex:
         self._sm = None
         self._hws = None
         self.hx = None
+        self._rows = None
+        self._pos_of_sid = None
         self.mode = "fp32"
         self.eps_scale = self.EPS_SCALE
         self.audit_every = self.AUDIT_EVERY
@@ -174,10 +177,7 @@ class DenseIndex:
         hx["sent_off"], hx["sent_ids"] = F["sent_off"], F["sent_ids"]
         fi.leaf_row_b, fi.leaf_pos = hx["leaf_rows"].data_ptr(), hx["leaf_pos"].data_ptr()
         fi.sent_off, fi.sent_ids = hx["sent_off"].data_ptr(), hx["sent_ids"].data_ptr()
-        # row-major {r, mb} rows: the operands of the exact arithmetic in the finish stage
-        hx["rows"] = torch.empty((self.nn, d, 2), dtype=torch.float32, device=dev)
-        _lib.check(L.cw_index_rows_build(store, self.order.data_ptr(), self.nn, hx["rows"].data_ptr(), st),
-                   "cw_index_rows_build")
+        hx["rows"] = self.rows()
         fi.rows = hx["rows"].data_ptr()
         # constants of eps: hmax = max_b sum_d mean^2/var (= sum_d mb^2), lmax = max_b |sumlog|,
         # wfac = max over path lengths of sum_j |level_w[j]| / len; e1max = largest rounding-error coefficient of a leaf
@@ -196,10 +196,30 @@ class DenseIndex:
         hx["smem_ok"] = self.max_len <= 512
         self.hx = hx
 
+    def rows(self):
+        """Row-major {r, mb} rows [nn, D, 2] (cw_index_rows_build), built on first use: the operands of the exact
+        arithmetic in the fused finish stage and in pair scoring."""
+        if self._rows is None:
+            rows = torch.empty((self.nn, self.tree.d, 2), dtype=torch.float32, device=self.tree.device)
+            _lib.check(_lib.load().cw_index_rows_build(self.tree.store.struct(), self.order.data_ptr(), self.nn,
+                                                       rows.data_ptr(), _lib.stream_ptr()), "cw_index_rows_build")
+            self._rows = rows
+        return self._rows
+
+    def pos_of_sid(self):
+        """[n_pos] int32: position (row of path_idx) of each sentence id, the inverse of pos_rec[:, 3]; built on first use."""
+        if self._pos_of_sid is None:
+            p = torch.full((self.n_pos,), -1, dtype=torch.int32, device=self.tree.device)
+            p[self.pos_rec[:, 3].long()] = torch.arange(self.n_pos, dtype=torch.int32, device=p.device)
+            self._pos_of_sid = p
+        return self._pos_of_sid
+
     def bytes(self):
         b = (self.R.numel() + self.MB.numel() + self.sumlog.numel()) * 4
+        if self._rows is not None:
+            b += self._rows.numel() * 4
         if self.hx is not None:
-            b += sum(self.hx[n].numel() * self.hx[n].element_size() for n in ("B_int", "rc_int", "B_leaf", "rc_leaf", "rows")
+            b += sum(self.hx[n].numel() * self.hx[n].element_size() for n in ("B_int", "rc_int", "B_leaf", "rc_leaf")
                      if n in self.hx)
         return b
 
@@ -398,6 +418,65 @@ class DenseIndex:
                                                      _lib.stream_ptr()), "cw_small_predict_host")
         return sid.view(-1)[:k].tolist()
 
+    # ------------------------------------------------------------------ pair scores
+    def _pair_calls(self, ids):
+        """Column blocks of at most PAIR_MAX_M candidates and query chunks that fit PAIR_BUDGET_BYTES of scratch:
+        yields (query slice, column slice, scratch)."""
+        L, (nq, m) = _lib.load(), ids.shape
+        mb = min(m, _lib.PAIR_MAX_M)
+        per_query = int(L.cw_pair_scratch_words(1, mb, self.max_len))
+        _lib.check(min(per_query, 0), "cw_pair_scratch_words")
+        step = max(1, min(nq, self.PAIR_BUDGET_BYTES // (4 * per_query)))
+        scratch = torch.empty(max(1, step * per_query), dtype=torch.int32, device=ids.device)
+        for c0 in range(0, m, mb):
+            for q0 in range(0, nq, step):
+                yield slice(q0, min(nq, q0 + step)), slice(c0, min(m, c0 + mb)), scratch
+
+    def _pair_check(self):
+        if self.sentence_ids is not None:
+            raise ValueError("pair scores are indexed by global sentence id; not available on a sentence shard")
+
+    def pair_scores(self, Q, ids):
+        """[nq, m] exact leaf scores of sentences ids[q, c] (-1 = padding -> -inf) for queries Q [nq, D], bit for bit the
+        FP32 form's (cw_pair_scores).  Ids must lie in [-1, n_pos)."""
+        self._pair_check()
+        L = _lib.load()
+        out = torch.empty(ids.shape, dtype=torch.float32, device=Q.device)
+        if not self.n_pos or not ids.numel():
+            return out.fill_(float("-inf"))
+        rows, pos = self.rows(), self.pos_of_sid()
+        for qs, cs, scratch in self._pair_calls(ids):
+            cand = ids[qs, cs].contiguous()
+            o = torch.empty(cand.shape, dtype=torch.float32, device=Q.device)
+            q = Q[qs]
+            _lib.check(L.cw_pair_scores(C.byref(self.ix), rows.data_ptr(), pos.data_ptr(), self.n_pos, q.data_ptr(),
+                                        q.shape[0], cand.data_ptr(), cand.shape[1], o.data_ptr(), scratch.data_ptr(),
+                                        _lib.stream_ptr()), "cw_pair_scores")
+            out[qs, cs] = o
+        return out
+
+    def pair_scores_bwd(self, Q, ids, grad_out):
+        """dL/dQ [nq, D] for dL/d(pair_scores(Q, ids)) = grad_out [nq, m] (cw_pair_scores_bwd); column blocks are added
+        in order, so the result is the same bits on every run."""
+        self._pair_check()
+        L = _lib.load()
+        grad = torch.zeros_like(Q)
+        if not self.n_pos or not ids.numel():
+            return grad
+        rows, pos = self.rows(), self.pos_of_sid()
+        part = torch.empty_like(Q) if ids.shape[1] > _lib.PAIR_MAX_M else None
+        for qs, cs, scratch in self._pair_calls(ids):
+            cand = ids[qs, cs].contiguous()
+            g = grad_out[qs, cs].contiguous().to(torch.float32)
+            q = Q[qs]
+            dst = grad[qs] if part is None else part[qs]
+            _lib.check(L.cw_pair_scores_bwd(C.byref(self.ix), rows.data_ptr(), pos.data_ptr(), self.n_pos, q.data_ptr(),
+                                            q.shape[0], cand.data_ptr(), cand.shape[1], g.data_ptr(), dst.data_ptr(),
+                                            scratch.data_ptr(), _lib.stream_ptr()), "cw_pair_scores_bwd")
+            if part is not None:
+                grad[qs] += part[qs]
+        return grad
+
     STAGES = ("query_operands", "internal_scores_f16x3", "cumulative_sums", "sample_threshold", "leaf_filter_f16", "finish",
               "fallback_audit_tail")
 
@@ -476,6 +555,21 @@ class _RankScores(torch.autograd.Function):
             _lib.check(_lib.load().cw_rank_scores_bwd(C.byref(ix.ix), Q[lo:lo + n].data_ptr(), n, g.data_ptr(), gs.data_ptr(),
                                                       n, out[lo:lo + n].data_ptr(), _lib.stream_ptr()), "cw_rank_scores_bwd")
         return out, None
+
+
+class _PairScores(torch.autograd.Function):
+    """score_sentences with a gradient w.r.t. the queries (cw_pair_scores_bwd)."""
+
+    @staticmethod
+    def forward(ctx, Q, ids, index):
+        ctx.index = index
+        ctx.save_for_backward(Q.detach(), ids)
+        return index.pair_scores(Q.detach(), ids)
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        Q, ids = ctx.saved_tensors
+        return ctx.index.pair_scores_bwd(Q, ids, grad_out.contiguous()), None, None
 
 
 class CobwebWrapper:
@@ -693,6 +787,62 @@ class CobwebWrapper:
             return _RankScores.apply(Qd.contiguous(), self._index)
         _, _, leaf = self._index.predict(self.tree._as_device_mat(Q), 0, want_leaf_scores=True, mode="fp32")
         return leaf
+
+    def score_sentences(self, Q, ids):
+        """Additive: the Cobweb leaf scores of chosen sentences, bit for bit rank_scores_batch(Q)[q, ids[q, c]], without
+        scoring the rest of the tree.  Q [nq, D] or [D]; ids [nq, m] sentence ids per query, or [m] for the same list
+        for every query; -1 is padding and scores -inf.  Returns [nq, m] float32 on the device ([m] for a [D] query).
+        Differentiable w.r.t. Q when Q requires grad; padding gets no gradient, a repeated id gets the sum of its
+        entries' gradients."""
+        self.build_prediction_index()
+        single = torch.is_tensor(Q) and Q.dim() == 1 or not torch.is_tensor(Q) and np.ndim(Q) == 1
+        if torch.is_tensor(Q) and Q.requires_grad:
+            if Q.dim() not in (1, 2) or Q.shape[-1] != self.tree.d:
+                raise ValueError(f"Q must be [nq, {self.tree.d}] or [{self.tree.d}]")
+            Qd = Q.to(device=self.device, dtype=torch.float32).reshape(-1, self.tree.d).contiguous()
+        else:
+            Qd = self.tree._as_device_mat(Q).reshape(-1, self.tree.d).contiguous()
+        ids = torch.as_tensor(ids, device=Qd.device)
+        if ids.dtype.is_floating_point or ids.dtype == torch.bool or ids.dim() not in (1, 2):
+            raise ValueError("ids must be an integer tensor of shape [m] or [nq, m]")
+        if ids.dim() == 1:
+            ids = ids.unsqueeze(0).expand(Qd.shape[0], -1)
+        elif ids.shape[0] != Qd.shape[0]:
+            raise ValueError(f"ids has {ids.shape[0]} rows for {Qd.shape[0]} queries")
+        n = len(self)
+        if ids.numel() and bool(((ids < -1) | (ids >= n)).any()):
+            raise ValueError(f"sentence ids must lie in [-1, {n}) (-1 = padding)")
+        ids = ids.to(torch.int32).contiguous()
+        if Qd.requires_grad:
+            out = _PairScores.apply(Qd, ids, self._index)
+        else:
+            out = self._index.pair_scores(Qd, ids)
+        return out[0] if single else out
+
+    def rerank(self, Q, ids, k):
+        """Additive: the k best of the given candidates by exact Cobweb score, ranked like predict_fast_batch (score
+        desc, sentence id asc).  Q [nq, D] or [D]; ids as in score_sentences.  Returns (ids [nq, k] int32, scores [nq, k])
+        ([k] each for a [D] query), padded with -1 / -inf when fewer than k valid candidates exist.  Entries are ranked
+        as given: an id passed twice can appear twice."""
+        k = int(k)
+        if k < 0:
+            raise ValueError("k must be >= 0")
+        with torch.no_grad():
+            scores = self.score_sentences(Q.detach() if torch.is_tensor(Q) else Q, ids)
+        single = scores.dim() == 1
+        scores = scores.unsqueeze(0) if single else scores
+        ids = torch.as_tensor(ids, device=scores.device).to(torch.int32).reshape(-1, scores.shape[1])
+        ids = ids.expand(scores.shape[0], -1)
+        # (score desc, id asc), padding last: sort by id (padding as the largest), then stably by score
+        tie = torch.where(ids < 0, torch.iinfo(torch.int32).max, ids)
+        _, o1 = torch.sort(tie, dim=1, stable=True)
+        s2, o2 = torch.sort(scores.gather(1, o1), dim=1, descending=True, stable=True)
+        top_ids, top_val = ids.gather(1, o1.gather(1, o2))[:, :k], s2[:, :k]
+        if top_ids.shape[1] < k:
+            pad = k - top_ids.shape[1]
+            top_ids = torch.cat([top_ids, top_ids.new_full((top_ids.shape[0], pad), -1)], 1)
+            top_val = torch.cat([top_val, top_val.new_full((top_val.shape[0], pad), float("-inf"))], 1)
+        return (top_ids[0], top_val[0]) if single else (top_ids, top_val)
 
     def cobweb_predict_indexed(self, input, k=5, return_ids=False, is_embedding=False):
         """CobwebWrapper.cobweb_predict_indexed (CobwebWrapper.py:210-265), noise-free."""
