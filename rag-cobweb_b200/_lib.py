@@ -26,7 +26,8 @@ EXPORTS = ["cw_version", "cw_last_error", "cw_store_init", "cw_store_derive", "c
            "cw_predict_dense_host", "cw_index_rows_build",
            "cw_h_b_bytes", "cw_h_a_bytes", "cw_h_stages", "cw_h_set_build", "cw_h_rows_isotropic", "cw_fused_flag_words", "cw_fused_predict",
            "cw_fused_predict_host", "cw_fused_profile", "cw_small_scratch_words", "cw_small_predict", "cw_small_predict_host",
-           "cw_rank_scores_bwd", "cw_pair_scratch_words", "cw_pair_scores", "cw_pair_scores_bwd", "cw_whiten", "cw_ffma_peak", "cw_ffma2_peak"]
+           "cw_rank_scores_bwd", "cw_pair_scratch_words", "cw_pair_scores", "cw_pair_scores_bwd", "cw_whiten", "cw_ffma_peak", "cw_ffma2_peak",
+           "cw_leaf_tags", "cw_dense_paths_topk_tagged", "cw_small_predict_tagged", "cw_fused_predict_tagged"]
 
 
 class CwStore(C.Structure):
@@ -71,6 +72,10 @@ class CwFusedWork(C.Structure):
                 ("flag", C.c_void_p), ("out_sid_dev", C.c_void_p), ("out_val_dev", C.c_void_p), ("sm_Q", C.c_void_p),
                 ("sm_scores", C.c_void_p), ("sm_scratch", C.c_void_p), ("sm_sid", C.c_void_p), ("sm_val", C.c_void_p),
                 ("sm_n", C.c_void_p), ("stats", C.c_void_p), ("audit_every", C.c_int32), ("audit_phase", C.c_int32)]
+
+
+class CwTagFilter(C.Structure):
+    _fields_ = [("query_tags", C.c_void_p), ("pos_tags", C.c_void_p), ("leaf_tags", C.c_void_p), ("sent_tags", C.c_void_p)]
 
 
 class CobwebB200Error(RuntimeError):
@@ -134,6 +139,12 @@ def load():
     L.cw_pair_scratch_words.argtypes = [i64, i32c, i32c]
     L.cw_pair_scores.argtypes = [C.POINTER(CwIndex), vp, vp, i32c, vp, i64, vp, i32c, vp, vp, vp]
     L.cw_pair_scores_bwd.argtypes = [C.POINTER(CwIndex), vp, vp, i32c, vp, i64, vp, i32c, vp, vp, vp, vp]
+    L.cw_leaf_tags.argtypes = [vp, vp, i32c, vp, vp, vp]
+    tfp = C.POINTER(CwTagFilter)
+    L.cw_dense_paths_topk_tagged.argtypes = [C.POINTER(CwIndex), tfp, vp, i64, i64, i32, vp, vp, vp, vp]
+    L.cw_small_predict_tagged.argtypes = [C.POINTER(CwIndex), tfp, vp, i64, vp, vp, i32c, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp,
+                                          vp]
+    L.cw_fused_predict_tagged.argtypes = [C.POINTER(CwFusedIndex), C.POINTER(CwFusedWork), tfp, vp, i64, i32, vp, vp, vp]
     L.cw_whiten.argtypes = [vp, i64, C.c_int32, vp, vp, C.c_int32, vp, vp, vp, vp, vp]
     L.cw_ffma_peak.argtypes = [i32, i32, i32, vp, vp]
     L.cw_ffma2_peak.argtypes = [i32, i32, i32, vp, vp]

@@ -283,12 +283,15 @@ struct __align__(16) PathRec {
 // position p + PF_DIST are in flight (cp.async into a per-lane ring) while position p is consumed.
 // Deeper non-shared levels (an ancestor above the grandparent changed: ~1 position in 60) are read
 // on demand.
-template <bool LEAF, bool K32>
+// TAGGED: a position is offered to its query's list only if its sentence is eligible (pos_tags & qtags[q]); the path
+// sums of every position are still formed, since the next positions build on them.  The tag rides in the record's pad0.
+template <bool LEAF, bool K32, bool TAGGED>
 __global__ void __launch_bounds__(256, 3)
 paths_topk_kernel(const float *__restrict__ ST, unsigned ldq, long long nq, int n_pos, int max_len,
                   const int *__restrict__ path_pm, const int4 *__restrict__ pos_rec,
                   const double *__restrict__ level_w, int k, float *leaf_scores, float *cand_s, int *cand_i,
-                  int n_chunks, int chunk_len, int *shared_thr, const int *__restrict__ nq_dev) {
+                  int n_chunks, int chunk_len, int *shared_thr, const int *__restrict__ nq_dev,
+                  const unsigned *__restrict__ qtags, const unsigned *__restrict__ pos_tags) {
     extern __shared__ __align__(16) unsigned char pt_smem[];
     if (nq_dev) nq = min(nq, (long long)*nq_dev);  // count decided on the device (flagged queries of the fused mode)
     // level weights in binary64; the path weight of level j on a path of length len is
@@ -320,6 +323,7 @@ paths_topk_kernel(const float *__restrict__ ST, unsigned ldq, long long nq, int 
     float thr_s = NEG_INF;
     int thr_i = 0x7fffffff;
     const bool collect = k > 0 && qvalid;
+    const unsigned qtag = TAGGED && qvalid ? qtags[q] : 0u;
     // Threshold shared by the chunks of a query: the k-th best of ANY chunk's full list is a lower bound of the k-th
     // best over all positions, so a score strictly below it cannot be in the final top-k.  Each lane publishes its own
     // k-th best (atomicMax on an order-preserving integer key) and re-reads the shared bound once per 32 positions;
@@ -339,6 +343,7 @@ paths_topk_kernel(const float *__restrict__ ST, unsigned ldq, long long nq, int 
             const int *path = path_pm + (size_t)(p0 + r) * max_len;
             if (R.m <= R.len - 2) R.par = path[R.len - 2];
             if (R.m <= R.len - 3) R.gpar = path[R.len - 3];
+            if (TAGGED) R.pad0 = (int)pos_tags[p0 + r];
         }
         return R;
     };
@@ -424,7 +429,8 @@ paths_topk_kernel(const float *__restrict__ ST, unsigned ldq, long long nq, int 
         // top-k: lanes whose candidate beats their query's k-th best are served one at a time by
         // the whole warp (lane r handles rank r of that query's list): no divergent shifting loops
         unsigned need = __ballot_sync(0xffffffffu, collect && acc >= gthr &&
-                                                       (acc > thr_s || (acc == thr_s && (unsigned)sid < (unsigned)thr_i)));
+                                                       (acc > thr_s || (acc == thr_s && (unsigned)sid < (unsigned)thr_i)) &&
+                                                       (!TAGGED || ((unsigned)R.pad0 & qtag) != 0u));
         if (K32) {
             // one rank per lane: read, ballot the insertion point, shift by one, done
             while (need) {
@@ -621,8 +627,10 @@ extern "C" int cw_dense_node_scores(const cw_index *ix, const float *Q, int64_t 
 extern "C" int64_t cw_topk_chunks(int64_t n_pos) { return (n_pos + 1023) / 1024 + 1; }
 
 // nq_dev (optional): the number of live queries is read on the device (<= nq, which sizes the launch)
+// tf (optional): offer eligible positions only (no leaf scores then)
 static int paths_topk_launch(const cw_index *ix, const float *node_scores, int64_t ldq, int64_t nq, int k, float *leaf_scores,
-                             int32_t *out_sid, float *out_score, int32_t *scratch, const int *nq_dev, cudaStream_t st) {
+                             int32_t *out_sid, float *out_score, int32_t *scratch, const int *nq_dev, cudaStream_t st,
+                             const cw_tag_filter *tf = nullptr) {
     if (!ix || !node_scores || nq < 0 || k < 0 || k > CW_MAX_K || ix->n_pos < 1 || !ix->path_idx || !ix->pos_rec ||
         !ix->level_w || ix->max_len < 1 || ix->max_len > PT_MAXLEN || ldq < nq || ldq > 0x7fffffffLL ||
         (k > 0 && (!out_sid || !out_score || !scratch))) {
@@ -672,8 +680,9 @@ static int paths_topk_launch(const cw_index *ix, const float *node_scores, int64
         if (rc) return rc;
     }
     const size_t smem = fixed + (size_t)wpb * per_warp;
-    auto kern = leaf_scores ? (k <= 32 ? paths_topk_kernel<true, true> : paths_topk_kernel<true, false>)
-                            : (k <= 32 ? paths_topk_kernel<false, true> : paths_topk_kernel<false, false>);
+    auto kern = tf ? (k <= 32 ? paths_topk_kernel<false, true, true> : paths_topk_kernel<false, false, true>)
+              : leaf_scores ? (k <= 32 ? paths_topk_kernel<true, true, false> : paths_topk_kernel<true, false, false>)
+                            : (k <= 32 ? paths_topk_kernel<false, true, false> : paths_topk_kernel<false, false, false>);
     if (smem > 48 * 1024) {
         int rc = cw_check_cuda(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),
                                "cw_dense_paths_topk: smem attribute");
@@ -681,7 +690,8 @@ static int paths_topk_launch(const cw_index *ix, const float *node_scores, int64
     }
     kern<<<dim3(n_chunks, (unsigned)gblocks), wpb * 32, smem, st>>>(
         node_scores, (unsigned)ldq, nq, ix->n_pos, ix->max_len, ix->path_idx, reinterpret_cast<const int4 *>(ix->pos_rec),
-        ix->level_w, k, leaf_scores, cand_s, cand_i, n_chunks, chunk_len, shared_thr, nq_dev);
+        ix->level_w, k, leaf_scores, cand_s, cand_i, n_chunks, chunk_len, shared_thr, nq_dev, tf ? tf->query_tags : nullptr,
+        tf ? tf->pos_tags : nullptr);
     if (k > 0)
         merge_topk_kernel<<<(unsigned)((nq + 7) / 8), 256, 0, st>>>(cand_s, cand_i, nq, n_chunks, k, out_sid, out_score, nq_dev);
     return cw_check_cuda(cudaGetLastError(), "cw_dense_paths_topk");
@@ -696,6 +706,16 @@ extern "C" int cw_dense_paths_topk(const cw_index *ix, const float *node_scores,
         return CW_E_ARG;
     }
     return paths_topk_launch(ix, node_scores, ldq, nq, k, leaf_scores, out_sid, out_score, scratch, nullptr, (cudaStream_t)stream);
+}
+
+extern "C" int cw_dense_paths_topk_tagged(const cw_index *ix, const cw_tag_filter *tf, const float *node_scores, int64_t ldq,
+                                          int64_t nq, int k, int32_t *out_sid, float *out_score, int32_t *scratch, void *stream) {
+    CwRange range("cw_dense_paths_topk_tagged");
+    if (!tf || !tf->query_tags || !tf->pos_tags || k < 1 || ldq < cw_score_ldq(nq)) {
+        cw_set_error("cw_dense_paths_topk_tagged: bad argument (query_tags and pos_tags needed, k >= 1, ldq >= cw_score_ldq(nq))");
+        return CW_E_ARG;
+    }
+    return paths_topk_launch(ix, node_scores, ldq, nq, k, nullptr, out_sid, out_score, scratch, nullptr, (cudaStream_t)stream, tf);
 }
 
 // One call = batched cobweb_predict_fast(return_ids=True) on HOST buffers with the FP32 form
@@ -807,10 +827,14 @@ __global__ void small_scatter_kernel(const int *__restrict__ which, int off, con
 // levels of a path are independent loads of the [rows, CW_SMALL_Q] score matrix, which sits in L2), the chain
 // acc = fma((float)(level_w[j]/len), s_j, acc) runs root first like paths_topk_kernel's; a warp keeps the running
 // top-k of its chunk in registers (topk_offer).  grid (ceil(n_chunks / 4), queries), 4 warps = 4 chunks per CTA.
+// TAGGED: only positions whose sentence is eligible (pos_tags & the query's mask) are scored and offered; query i of
+// the launch is query which[which_off + i] of qtags when a which list is given.
+template <bool TAGGED>
 __global__ void __launch_bounds__(128)
 paths_small_kernel(const float *__restrict__ ST, int nq, const int *__restrict__ nq_dev, int n_pos, int max_len,
                    const int *__restrict__ path_pm, const int4 *__restrict__ pos_rec, const double *__restrict__ level_w, int k,
-                   float *cand_s, int *cand_i, int n_chunks, int chunk_len) {
+                   float *cand_s, int *cand_i, int n_chunks, int chunk_len, const unsigned *__restrict__ qtags,
+                   const unsigned *__restrict__ pos_tags, const int *__restrict__ which, int which_off) {
     extern __shared__ __align__(16) unsigned char ps_smem[];
     double *lw = reinterpret_cast<double *>(ps_smem);
     if (nq_dev) nq = min(nq, *nq_dev);
@@ -821,6 +845,7 @@ paths_small_kernel(const float *__restrict__ ST, int nq, const int *__restrict__
     const int lane = threadIdx.x & 31, chunk = blockIdx.x * 4 + (threadIdx.x >> 5);
     if (chunk >= n_chunks) return;
     const int p0 = chunk * chunk_len, p1 = min(n_pos, p0 + chunk_len);
+    const unsigned qtag = TAGGED ? qtags[which ? which[which_off + q] : q] : 0u;
     float ls[PT_SLOTS];
     int li[PT_SLOTS];
     topk_init(ls, li);
@@ -828,7 +853,7 @@ paths_small_kernel(const float *__restrict__ ST, int nq, const int *__restrict__
         const int p = pb + lane;
         float acc = 0.0f;
         int sid = -1;
-        if (p < p1) {
+        if (p < p1 && (!TAGGED || (pos_tags[p] & qtag) != 0u)) {
             const int4 rc = pos_rec[p];
             const int len = rc.x;
             sid = rc.w;
@@ -847,12 +872,14 @@ extern "C" int64_t cw_small_scratch_words(int64_t n_pos, int k) {
     return (int64_t)CW_SMALL_Q * cw_topk_chunks(n_pos < 1 ? 1 : n_pos) * (k > 0 ? k : 1) * 2;
 }
 
+// tf (optional): the tagged form (cw_small_predict_tagged)
 int cw_small_predict_impl(const cw_index *ix, const float *Q, int64_t nq, const int32_t *which, const int32_t *n_dev,
                           int32_t which_off, int scatter, int k, float *sm_Q, float *sm_scores, int32_t *sm_scratch, int32_t *sm_sid,
-                          float *sm_val, int32_t *sm_n, int32_t *out_sid, float *out_val, cudaStream_t st) {
+                          float *sm_val, int32_t *sm_n, int32_t *out_sid, float *out_val, cudaStream_t st,
+                          const cw_tag_filter *tf) {
     CwRange range("cw_small_predict");
     if (!ix || !Q || nq < 0 || nq > CW_SMALL_Q || k < 1 || k > CW_MAX_K || !sm_scores || !sm_scratch || !out_sid || !out_val ||
-        (which && (!sm_Q || !sm_sid || !sm_val || !sm_n)) || (n_dev && !which)) {
+        (which && (!sm_Q || !sm_sid || !sm_val || !sm_n)) || (n_dev && !which) || (tf && (!tf->query_tags || !tf->pos_tags))) {
         cw_set_error("cw_small_predict: bad argument (nq=%lld, at most %d; k=%d)", (long long)nq, CW_SMALL_Q, k);
         return CW_E_ARG;
     }
@@ -890,9 +917,10 @@ int cw_small_predict_impl(const cw_index *ix, const float *Q, int64_t nq, const 
     const int n_chunks = (ix->n_pos + chunk_len - 1) / chunk_len;
     float *cand_s = reinterpret_cast<float *>(sm_scratch);
     int *cand_i = sm_scratch + (size_t)nq * n_chunks * k;
-    paths_small_kernel<<<dim3((n_chunks + 3) / 4, (unsigned)nq), 128, (size_t)ix->max_len * sizeof(double), st>>>(
+    (tf ? paths_small_kernel<true> : paths_small_kernel<false>)<<<dim3((n_chunks + 3) / 4, (unsigned)nq), 128,
+                                                                  (size_t)ix->max_len * sizeof(double), st>>>(
         sm_scores, (int)nq, cnt, ix->n_pos, ix->max_len, ix->path_idx, reinterpret_cast<const int4 *>(ix->pos_rec), ix->level_w, k,
-        cand_s, cand_i, n_chunks, chunk_len);
+        cand_s, cand_i, n_chunks, chunk_len, tf ? tf->query_tags : nullptr, tf ? tf->pos_tags : nullptr, which, which_off);
     merge_topk_kernel<<<(unsigned)((nq + 7) / 8), 256, 0, st>>>(cand_s, cand_i, nq, n_chunks, k, which ? sm_sid : out_sid,
                                                                which ? sm_val : out_val, cnt);
     int rc = cw_check_cuda(cudaGetLastError(), "cw_small_predict: paths");
@@ -905,7 +933,19 @@ extern "C" int cw_small_predict(const cw_index *ix, const float *Q, int64_t nq, 
                                 int32_t which_off, int scatter, int k, float *sm_Q, float *sm_scores, int32_t *sm_scratch, int32_t *sm_sid,
                                 float *sm_val, int32_t *sm_n, int32_t *out_sid, float *out_val, void *stream) {
     return cw_small_predict_impl(ix, Q, nq, which, n_dev, which_off, scatter, k, sm_Q, sm_scores, sm_scratch, sm_sid, sm_val, sm_n, out_sid,
-                                 out_val, (cudaStream_t)stream);
+                                 out_val, (cudaStream_t)stream, nullptr);
+}
+
+extern "C" int cw_small_predict_tagged(const cw_index *ix, const cw_tag_filter *tf, const float *Q, int64_t nq, const int32_t *which,
+                                       const int32_t *n_dev, int32_t which_off, int scatter, int k, float *sm_Q, float *sm_scores,
+                                       int32_t *sm_scratch, int32_t *sm_sid, float *sm_val, int32_t *sm_n, int32_t *out_sid,
+                                       float *out_val, void *stream) {
+    if (!tf) {
+        cw_set_error("cw_small_predict_tagged: no tag filter");
+        return CW_E_ARG;
+    }
+    return cw_small_predict_impl(ix, Q, nq, which, n_dev, which_off, scatter, k, sm_Q, sm_scores, sm_scratch, sm_sid, sm_val, sm_n, out_sid,
+                                 out_val, (cudaStream_t)stream, tf);
 }
 
 extern "C" int cw_small_predict_host(const cw_index *ix, const float *Q_host, int64_t nq, int k, float *sm_Q, float *sm_scores,
@@ -922,7 +962,7 @@ extern "C" int cw_small_predict_host(const cw_index *ix, const float *Q_host, in
                            "cw_small_predict_host: H2D");
     if (rc) return rc;
     if ((rc = cw_small_predict_impl(ix, sm_Q, nq, nullptr, nullptr, 0, 0, k, sm_Q, sm_scores, sm_scratch, sm_sid, sm_val, sm_n, sm_sid,
-                                    sm_val, st)))
+                                    sm_val, st, nullptr)))
         return rc;
     if ((rc = cw_check_cuda(cudaMemcpyAsync(out_sid_host, sm_sid, (size_t)nq * k * sizeof(int32_t), cudaMemcpyDeviceToHost, st),
                             "cw_small_predict_host: D2H ids")))

@@ -178,6 +178,9 @@ __device__ __forceinline__ void tile_coords(long long t, int n_qtiles, int n_nti
 //               to slot j (32 different leaves per query reach their slot values)
 //   EPI_FILTER  a1 and its upper bound a1 + e1[row] * ||a_q||; (a1, row) appended to the query's candidate buffer when
 //               the bound reaches tau[q]
+// TAGGED (TAU and FILTER): a row counts only if it is eligible, leaf_tags[row] & qtags[q] != 0 (the leaf holds at least one
+// sentence the query may see).  The row's tag is staged in shared memory in place of its parent row (record word 5),
+// which only the staging itself reads.
 enum { EPI_NODE = 0, EPI_TAU = 1, EPI_FILTER = 2 };
 struct HEpi {
     float *out;           // NODE: [rows, ldq]
@@ -219,10 +222,11 @@ struct KCfg {
 };
 static_assert(KCfg<true>::SMEM * 2 + 2048 <= 227 * 1024 + 1024, "two half-tile CTAs per SM");
 
-template <int NPROD, int MODE, bool HALF>
+template <int NPROD, int MODE, bool HALF, bool TAGGED>
 __global__ void __launch_bounds__(KCfg<HALF>::THR, KCfg<HALF>::CTAS)
 h_score_kernel(const unsigned char *__restrict__ A, const unsigned char *__restrict__ B, const HEpi epi, int n_qtiles,
-               int nt_begin, int n_ntiles, int n_stages, int pq) {
+               int nt_begin, int n_ntiles, int n_stages, int pq, const unsigned *__restrict__ qtags,
+               const unsigned *__restrict__ leaf_tags) {
     using K = KCfg<HALF>;
     extern __shared__ unsigned char smem_raw[];
     const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;  // swizzle atoms need their natural alignment
@@ -392,7 +396,13 @@ h_score_kernel(const unsigned char *__restrict__ A, const unsigned char *__restr
                         const float4 *src = reinterpret_cast<const float4 *>(epi.rc) + (n0 + e) * 2;
                         const float4 r1 = __ldg(src + 1);
                         recs_s[rbuf * (TN * 2) + e * 2] = __ldg(src);
-                        recs_s[rbuf * (TN * 2) + e * 2 + 1] = r1;
+                        if (TAGGED) {
+                            float4 r1t = r1;
+                            r1t.y = __uint_as_float(n0 + e < epi.n_rows ? leaf_tags[n0 + e] : 0u);
+                            recs_s[rbuf * (TN * 2) + e * 2 + 1] = r1t;
+                        } else {
+                            recs_s[rbuf * (TN * 2) + e * 2 + 1] = r1;
+                        }
                         const int par = __float_as_int(r1.y), prev = __shfl_up_sync(0xffffffffu, par, 1);
                         coff_s[rbuf * TN + e] = (long long)(par < 0 ? 0 : par) * ldq * 4;
                         const bool head = (lane & (BW - 1)) == 0 || par != prev;
@@ -440,6 +450,11 @@ h_score_kernel(const unsigned char *__restrict__ A, const unsigned char *__restr
                     if (live0) tau0 = epi.tau[qbase];
                     if (live1) tau1 = epi.tau[qbase + TM];
                 }
+                unsigned qtag0 = 0u, qtag1 = 0u;
+                if (TAGGED) {
+                    if (live0) qtag0 = qtags[qbase];
+                    if (live1) qtag1 = qtags[qbase + TM];
+                }
                 float smax[BW];  // TAU: this warp only ever sees the rows r with (r / 16) % 4 == sub: slots (sub & 1) * 16 + j
 #pragma unroll
                 for (int j = 0; j < BW; j++) smax[j] = -__int_as_float(0x7f800000);
@@ -463,19 +478,32 @@ h_score_kernel(const unsigned char *__restrict__ A, const unsigned char *__restr
                     const float4 qv = qh ? qv1 : qv0;
                     const float tau = qh ? tau1 : tau0;
                     const bool live = qh ? live1 : live0;
+                    const unsigned qtag = qh ? qtag1 : qtag0;
                     float sc[BW];
                     unsigned hit = 0;
                     float c = 0.0f;
 #pragma unroll
                     for (int j = 0; j < BW; j++) {
                         const float4 r0 = recs[(cb * BW + j) * 2];      // {alpha, beta, gamma, delta}, broadcast read
-                        const float e1 = recs[(cb * BW + j) * 2 + 1].x;
+                        float e1 = 0.0f;
+                        bool elig = true;
+                        if (TAGGED && MODE == EPI_TAU) {
+                            elig = (__float_as_uint(recs[(cb * BW + j) * 2 + 1].y) & qtag) != 0u;
+                        } else if (TAGGED) {
+                            const float2 r1 = *reinterpret_cast<const float2 *>(recs + (cb * BW + j) * 2 + 1);  // {e1, tag}
+                            e1 = r1.x;
+                            elig = (__float_as_uint(r1.y) & qtag) != 0u;
+                        } else {
+                            e1 = recs[(cb * BW + j) * 2 + 1].x;
+                        }
                         c = (hm & (1u << j)) ? cur[j] : c;             // ancestor sum of this row's run
                         const float t0 = fmaf(r0.z, qv.y, r0.y);       // beta + gamma |x|^2
                         const float t1 = fmaf(r0.w, c, t0);            // + C[parent] / len
                         sc[j] = fmaf(r0.x, __uint_as_float(v[j]) * qv.x, t1);
-                        if (MODE == EPI_TAU) smax[j] = fmaxf(smax[j], sc[j]);
-                        else if (fmaf(e1, qv.z, sc[j]) >= tau) hit |= 1u << j;
+                        // an ineligible row leaves its slot alone: a slot no eligible row reaches keeps its fill
+                        // (0x80 bytes, about -3.4e38), so the threshold drops to -inf when fewer than m slots are reached
+                        if (MODE == EPI_TAU) { if (elig) smax[j] = fmaxf(smax[j], sc[j]); }
+                        else if (elig && fmaf(e1, qv.z, sc[j]) >= tau) hit |= 1u << j;
                     }
                     if (MODE == EPI_FILTER) {
                         // rows past the set are tile padding (only in the last tile)
@@ -823,6 +851,8 @@ struct FinArgs {
     int *anc_b;      // [nq, em] distinct ancestor index rows of the survivors
     float *anc_s;    // [nq, em] their exact node scores
     int *anc_slot;   // [nq, em] (survivor, level) -> entry of anc_b
+    // tagged form (cw_fused_predict_tagged): the queries' masks and the sentences' tags
+    const unsigned *qtags, *sent_tags;
 };
 
 static void fin_carve(FinArgs &a, int *p, long long cap_q, int ml) {
@@ -1034,6 +1064,14 @@ fn_exact_kernel(const cw_index ix, const float2 *__restrict__ RM, const float *_
 // a3 = (C[parent] + w_leaf s) / len of the refined leaves, the k-th best sentence score A_k over them, the line
 // thr = A_k - 2 eps and its test against U, the survivors (a3 >= thr), and the distinct index rows on their paths
 // (the leaf itself is already scored).  A query that fails is flagged here for the exact small-batch path.
+// TAGGED: a leaf counts its eligible sentences only.  Every candidate leaf holds at least one, and counting the others
+// would let A_k rise above the k-th best eligible score and drop leaves of the answer.
+__device__ __forceinline__ int eligible_sentences(const FinArgs &a, int row, unsigned qtag) {
+    int n = 0;
+    for (int i = a.sent_off[row]; i < a.sent_off[row + 1]; i++) n += (a.sent_tags[a.sent_ids[i]] & qtag) != 0u;
+    return n;
+}
+template <bool TAGGED>
 __global__ void __launch_bounds__(FQ_WARPS * 32)
 fn_line_kernel(const FinArgs a) {
     __shared__ float sa3_s[FQ_WARPS][KC1];
@@ -1053,13 +1091,14 @@ fn_line_kernel(const FinArgs a) {
         const float eps = __int_as_float(meta[FM_EPS]), U = __int_as_float(meta[FM_U]);
         int fail = meta[FM_FAIL];
         const int *rrow = a.ref_row + q * KC1;
+        const unsigned qtag = TAGGED ? a.qtags[q] : 0u;
         for (int i = lane; i < nsel; i += 32) {
             const int row = rrow[i];
             const float4 r0 = a.leaf_rc[row * 2], r1 = a.leaf_rc[row * 2 + 1];
             const int par = __float_as_int(r1.y);
             const float c = par >= 0 ? a.C[(long long)par * a.ldq + q] : 0.0f;
             sa3[i] = __fmul_rn(__fmaf_rn(r1.z, a.ref_s[q * KC1 + i], c), r0.w);
-            sns[i] = a.sent_off[row + 1] - a.sent_off[row];
+            sns[i] = TAGGED ? eligible_sentences(a, row, qtag) : a.sent_off[row + 1] - a.sent_off[row];
         }
         __syncwarp();
         // A_k: the a3 of the leaf that holds the k-th sentence in (a3 desc, list position asc) order
@@ -1150,7 +1189,8 @@ fn_line_kernel(const FinArgs a) {
 }
 
 // exact leaf scores of the survivors: sequential FMA along the path, root first, the leaf last (cw_dense_paths_topk's
-// order); their sentences ranked by (score desc, sentence id asc)
+// order); their sentences ranked by (score desc, sentence id asc).  TAGGED: their eligible sentences only.
+template <bool TAGGED>
 __global__ void __launch_bounds__(FQ_WARPS * 32)
 fn_topk_kernel(const FinArgs a) {
     __shared__ int lsid_s[FQ_WARPS][MAXS];
@@ -1166,6 +1206,7 @@ fn_topk_kernel(const FinArgs a) {
     const float NEG_INF = -__int_as_float(0x7f800000);
     int row = 0, ns = 0;
     float mex = 0.0f;
+    const unsigned qtag = TAGGED ? a.qtags[q] : 0u;
     if (lane < m) {  // m <= MS = 32
         const int sel = meta[FM_SURV + lane];
         row = a.ref_row[q * KC1 + sel];
@@ -1176,7 +1217,7 @@ fn_topk_kernel(const FinArgs a) {
 #pragma unroll 1
         for (int j = 0; j < len - 1; j++) acc = __fmaf_rn((float)(a.ix.level_w[j] / (double)len), as[slot[j]], acc);
         mex = __fmaf_rn((float)(a.ix.level_w[len - 1] / (double)len), a.ref_s[q * KC1 + sel], acc);
-        ns = a.sent_off[row + 1] - a.sent_off[row];
+        ns = TAGGED ? eligible_sentences(a, row, qtag) : a.sent_off[row + 1] - a.sent_off[row];
     }
     int off = ns;  // inclusive prefix sum of the sentence counts
     for (int d = 1; d < 32; d <<= 1) {
@@ -1190,7 +1231,19 @@ fn_topk_kernel(const FinArgs a) {
                   o = __shfl_sync(0xffffffffu, off, c);
         const float v = __shfl_sync(0xffffffffu, mex, c);
         const int first = a.sent_off[s0];
-        for (int i = lane; i < cntc; i += 32) { lsid[o + i] = a.sent_ids[first + i]; lval[o + i] = v; }
+        if (!TAGGED) {
+            for (int i = lane; i < cntc; i += 32) { lsid[o + i] = a.sent_ids[first + i]; lval[o + i] = v; }
+        } else {
+            const int n_all = a.sent_off[s0 + 1] - first;
+            int at = o;
+            for (int base = 0; base < n_all; base += 32) {
+                const int sid = base + lane < n_all ? a.sent_ids[first + base + lane] : -1;
+                const bool ok = sid >= 0 && (a.sent_tags[sid] & qtag) != 0u;
+                const unsigned mask = __ballot_sync(0xffffffffu, ok);
+                if (ok) { const int i = at + __popc(mask & ((1u << lane) - 1u)); lsid[i] = sid; lval[i] = v; }
+                at += __popc(mask);
+            }
+        }
     }
     __syncwarp();
     for (int i = lane; i < ns_tot; i += 32) {
@@ -1231,9 +1284,30 @@ __global__ void h_audit_cmp_kernel(const int *__restrict__ which, int n_a, int k
     if (!same && out_sid[q * k] != CW_SID_UNRESOLVED) atomicAdd(stats + 9, 1);
 }
 
+// leaf_tags[r] = OR of the tags of leaf row r's sentences (torch has no scatter-OR)
+__global__ void leaf_tags_kernel(const int *__restrict__ sent_off, const int *__restrict__ sent_ids, int n_leaf,
+                                 const unsigned *__restrict__ sent_tags, unsigned *leaf_tags) {
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= n_leaf) return;
+    unsigned t = 0u;
+    for (int i = sent_off[r]; i < sent_off[r + 1]; i++) t |= sent_tags[sent_ids[i]];
+    leaf_tags[r] = t;
+}
+
 }  // namespace cwh
 
 using namespace cwh;
+
+extern "C" int cw_leaf_tags(const int32_t *sent_off, const int32_t *sent_ids, int32_t n_leaf, const uint32_t *sent_tags,
+                            uint32_t *leaf_tags, void *stream) {
+    if (!sent_off || !sent_ids || !sent_tags || !leaf_tags || n_leaf < 0) {
+        cw_set_error("cw_leaf_tags: bad argument");
+        return CW_E_ARG;
+    }
+    if (n_leaf == 0) return 0;
+    leaf_tags_kernel<<<(n_leaf + 255) / 256, 256, 0, (cudaStream_t)stream>>>(sent_off, sent_ids, n_leaf, sent_tags, leaf_tags);
+    return cw_check_cuda(cudaGetLastError(), "cw_leaf_tags");
+}
 
 // fn_exact_kernel for other translation units (cw_pairs.cu); the attributes are per device, so they are set per call
 int cw_exact_rows_attr() {
@@ -1296,11 +1370,12 @@ extern "C" int cw_h_rows_isotropic(const cw_store *s, const int32_t *order, cons
     return out;
 }
 
-template <int NPROD, int MODE, bool HALF>
-static int h_launch_t(const cw_h_set *hs, const void *A, int64_t nq, int nt_begin, int nt_count, const HEpi &epi, cudaStream_t st) {
+template <int NPROD, int MODE, bool HALF, bool TAGGED>
+static int h_launch_t(const cw_h_set *hs, const void *A, int64_t nq, int nt_begin, int nt_count, const HEpi &epi, cudaStream_t st,
+                      const cw_tag_filter *tf) {
     using K = KCfg<HALF>;
     const int n_qtiles = (int)((nq + K::TQK - 1) / K::TQK);
-    auto kern = h_score_kernel<NPROD, MODE, HALF>;
+    auto kern = h_score_kernel<NPROD, MODE, HALF, TAGGED>;
     int rc = cw_check_cuda(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, K::SMEM), "cw_h: smem attribute");
     if (rc) return rc;
     int dev = 0, sms = 148;
@@ -1315,25 +1390,36 @@ static int h_launch_t(const cw_h_set *hs, const void *A, int64_t nq, int nt_begi
     const int n_panels = (n_qtiles + pq_max - 1) / pq_max;
     const int pq = (n_qtiles + n_panels - 1) / n_panels;
     kern<<<grid, K::THR, K::SMEM, st>>>(reinterpret_cast<const unsigned char *>(A), reinterpret_cast<const unsigned char *>(hs->B),
-                                        epi, n_qtiles, nt_begin, nt_count, hs->n_stages, pq);
+                                        epi, n_qtiles, nt_begin, nt_count, hs->n_stages, pq, tf ? tf->query_tags : nullptr,
+                                        tf ? tf->leaf_tags : nullptr);
     return cw_check_cuda(cudaGetLastError(), "cw_h: score kernel");
 }
-// the one-product kernels take half tiles (two CTAs per SM) unless COBWEB_B200_FULL_TILE=1 asks for the full ones
+// the one-product kernels take half tiles (two CTAs per SM) unless COBWEB_B200_FULL_TILE=1 asks for the full ones;
+// tf (leaf-row modes only): the tagged instantiation
 template <int NPROD, int MODE>
-static int h_launch(const cw_h_set *hs, const void *A, int64_t nq, int nt_begin, int nt_count, const HEpi &epi, cudaStream_t st) {
+static int h_launch(const cw_h_set *hs, const void *A, int64_t nq, int nt_begin, int nt_count, const HEpi &epi, cudaStream_t st,
+                    const cw_tag_filter *tf = nullptr) {
     static const bool full_tile = getenv("COBWEB_B200_FULL_TILE") && atoi(getenv("COBWEB_B200_FULL_TILE")) != 0;
-    if (NPROD == 1 && !full_tile) return h_launch_t<NPROD, MODE, true>(hs, A, nq, nt_begin, nt_count, epi, st);
-    return h_launch_t<NPROD, MODE, false>(hs, A, nq, nt_begin, nt_count, epi, st);
+    if constexpr (MODE != EPI_NODE) {
+        if (tf) {
+            if (NPROD == 1 && !full_tile) return h_launch_t<NPROD, MODE, true, true>(hs, A, nq, nt_begin, nt_count, epi, st, tf);
+            return h_launch_t<NPROD, MODE, false, true>(hs, A, nq, nt_begin, nt_count, epi, st, tf);
+        }
+    }
+    if (NPROD == 1 && !full_tile) return h_launch_t<NPROD, MODE, true, false>(hs, A, nq, nt_begin, nt_count, epi, st, nullptr);
+    return h_launch_t<NPROD, MODE, false, false>(hs, A, nq, nt_begin, nt_count, epi, st, nullptr);
 }
 
 int cw_small_predict_impl(const cw_index *ix, const float *Q, int64_t nq, const int32_t *which, const int32_t *n_dev,
                           int32_t which_off, int scatter, int k, float *sm_Q, float *sm_scores, int32_t *sm_scratch, int32_t *sm_sid,
-                          float *sm_val, int32_t *sm_n, int32_t *out_sid, float *out_val, cudaStream_t st);
+                          float *sm_val, int32_t *sm_n, int32_t *out_sid, float *out_val, cudaStream_t st,
+                          const cw_tag_filter *tf);
 
 // one chunk of at most w->cap_q queries, all on the device
 // ev (optional): CW_FUSED_STAGES + 1 events recorded at the stage boundaries (cw_fused_profile)
+// tf (optional): the tagged form, tf->query_tags indexed like this chunk's Q
 static int fused_chunk(const cw_fused_index *fi, const cw_fused_work *w, const float *Q, int64_t nq, int k, int32_t *out_sid,
-                       float *out_val, cudaStream_t st, cudaEvent_t *ev = nullptr) {
+                       float *out_val, cudaStream_t st, cudaEvent_t *ev = nullptr, const cw_tag_filter *tf = nullptr) {
     CwRange range("cw_fused_chunk");
     static const char *const stage_names[CW_FUSED_STAGES] = {"query_operands", "internal_scores", "cumulative_sums", "sample_threshold",
                                                               "leaf_filter", "finish", "fallback_audit"};
@@ -1381,7 +1467,7 @@ static int fused_chunk(const cw_fused_index *fi, const cw_fused_work *w, const f
     const float inv_prior = 1.0f / fi->prior_var;
     if (fi->n_sample_tiles > 0) {
         if ((rc = cw_check_cuda(cudaMemsetAsync(w->slots, 0x80, (size_t)nq * 32 * sizeof(int), st), "cw_fused: memset"))) return rc;
-        if ((rc = h_launch<1, EPI_TAU>(&fi->leaves, w->A_leaf, nq, 0, fi->n_sample_tiles, epi, st))) return rc;
+        if ((rc = h_launch<1, EPI_TAU>(&fi->leaves, w->A_leaf, nq, 0, fi->n_sample_tiles, epi, st, tf))) return rc;
         const int m = k + 2 < 32 ? k + 2 : 32;
         h_tau_kernel<<<(unsigned)((nq + 127) / 128), 128, 0, st>>>(w->slots, qv, nq, m, fi->e1max, inv_prior, fi->hmax, fi->lmax,
                                                                   fi->wfac, fi->eps_scale, fi->ix.max_len, w->tau);
@@ -1389,7 +1475,7 @@ static int fused_chunk(const cw_fused_index *fi, const cw_fused_work *w, const f
         h_fill_kernel<<<(unsigned)((nq + 255) / 256), 256, 0, st>>>(w->tau, nq, -INFINITY);
     }
     mark(4);
-    if ((rc = h_launch<1, EPI_FILTER>(&fi->leaves, w->A_leaf, nq, 0, fi->leaves.n_ntiles, epi, st))) return rc;
+    if ((rc = h_launch<1, EPI_FILTER>(&fi->leaves, w->A_leaf, nq, 0, fi->leaves.n_ntiles, epi, st, tf))) return rc;
     mark(5);
     FinArgs a;
     a.ix = fi->ix;
@@ -1419,6 +1505,8 @@ static int fused_chunk(const cw_fused_index *fi, const cw_fused_work *w, const f
     a.out_val = out_val;
     a.flag = w->flag;
     a.stats = w->stats;
+    a.qtags = tf ? tf->query_tags : nullptr;
+    a.sent_tags = tf ? tf->sent_tags : nullptr;
     fin_carve(a, w->flag + 4 + w->cap_q + CW_SMALL_Q, w->cap_q, w->fin_ml);
     // the candidates of a select warp sit in shared memory: at most FQ_WARPS x 2048 x 12 bytes (fused_args_ok bounds cap)
     const int sel_smem = FQ_WARPS * w->cap * 12;
@@ -1429,15 +1517,15 @@ static int fused_chunk(const cw_fused_index *fi, const cw_fused_work *w, const f
     const unsigned gq = (unsigned)((nq + FQ_WARPS - 1) / FQ_WARPS);
     fn_select_kernel<<<gq, FQ_WARPS * 32, sel_smem, st>>>(a);
     cw_exact_rows_launch(a.ix, a.RM, Q, nq, a.ref_b, a.meta, FM_STRIDE, FM_NSEL, KC1, a.ref_s, 1, st);
-    fn_line_kernel<<<gq, FQ_WARPS * 32, 0, st>>>(a);
+    (tf ? fn_line_kernel<true> : fn_line_kernel<false>)<<<gq, FQ_WARPS * 32, 0, st>>>(a);
     cw_exact_rows_launch(a.ix, a.RM, Q, nq, a.anc_b, a.meta, FM_STRIDE, FM_NANC, a.em, a.anc_s, 1, st);
-    fn_topk_kernel<<<gq, FQ_WARPS * 32, 0, st>>>(a);
+    (tf ? fn_topk_kernel<true> : fn_topk_kernel<false>)<<<gq, FQ_WARPS * 32, 0, st>>>(a);
     if ((rc = cw_check_cuda(cudaGetLastError(), "cw_fused_predict"))) return rc;
     mark(6);
     // flagged queries: exact small-batch path, driven by the device-side count
     for (int r = 0; r < CW_FUSED_FB_ROUNDS; r++) {
         if ((rc = cw_small_predict_impl(&fi->ix, Q, CW_SMALL_Q, w->flag + 4, w->flag, r * CW_SMALL_Q, 1, k, w->sm_Q, w->sm_scores,
-                                        w->sm_scratch, w->sm_sid, w->sm_val, w->sm_n, out_sid, out_val, st)))
+                                        w->sm_scratch, w->sm_sid, w->sm_val, w->sm_n, out_sid, out_val, st, tf)))
             return rc;
     }
     h_unresolved_kernel<<<1, 1, 0, st>>>(w->flag, CW_FUSED_FB_ROUNDS * CW_SMALL_Q, w->stats);
@@ -1452,7 +1540,7 @@ static int fused_chunk(const cw_fused_index *fi, const cw_fused_work *w, const f
         int *which = w->flag + 4 + w->cap_q;
         h_audit_pick_kernel<<<1, CW_SMALL_Q, 0, st>>>(which, (int)n_a, (int)every, (int)((w->audit_phase / CW_FUSED_AUDIT_STRIDE) % every), nq);
         if ((rc = cw_small_predict_impl(&fi->ix, Q, n_a, which, nullptr, 0, 0, k, w->sm_Q, w->sm_scores, w->sm_scratch, w->sm_sid,
-                                        w->sm_val, w->sm_n, out_sid, out_val, st)))
+                                        w->sm_val, w->sm_n, out_sid, out_val, st, tf)))
             return rc;
         h_audit_cmp_kernel<<<1, CW_SMALL_Q, 0, st>>>(which, (int)n_a, k, w->sm_sid, w->sm_val, out_sid, out_val, w->stats);
     }
@@ -1486,6 +1574,24 @@ extern "C" int cw_fused_predict(const cw_fused_index *fi, const cw_fused_work *w
     for (int64_t lo = 0; lo < nq; lo += w->cap_q) {
         const int64_t n = nq - lo < w->cap_q ? nq - lo : w->cap_q;
         int rc = fused_chunk(fi, w, Q + lo * fi->ix.D, n, k, out_sid + lo * k, out_val + lo * k, (cudaStream_t)stream);
+        if (rc) return rc;
+    }
+    return 0;
+}
+
+// Tagged form: the chunks take their slice of the query masks; flagged and audited queries run the tagged small path
+extern "C" int cw_fused_predict_tagged(const cw_fused_index *fi, const cw_fused_work *w, const cw_tag_filter *tf, const float *Q,
+                                       int64_t nq, int k, int32_t *out_sid, float *out_val, void *stream) {
+    if (!fused_args_ok(fi, w, k) || !tf || !tf->query_tags || !tf->pos_tags || !tf->leaf_tags || !tf->sent_tags || !Q || !out_sid ||
+        !out_val || nq < 0) {
+        cw_set_error("cw_fused_predict_tagged: bad argument (k=%d, 1..%d; every tag array is needed)", k, CW_FUSED_MAX_K);
+        return CW_E_ARG;
+    }
+    for (int64_t lo = 0; lo < nq; lo += w->cap_q) {
+        const int64_t n = nq - lo < w->cap_q ? nq - lo : w->cap_q;
+        cw_tag_filter t = *tf;
+        t.query_tags = tf->query_tags + lo;
+        int rc = fused_chunk(fi, w, Q + lo * fi->ix.D, n, k, out_sid + lo * k, out_val + lo * k, (cudaStream_t)stream, nullptr, &t);
         if (rc) return rc;
     }
     return 0;
@@ -1528,7 +1634,8 @@ extern "C" int cw_fused_predict_host(const cw_fused_index *fi, const cw_fused_wo
         if (n_flag > CW_FUSED_FB_ROUNDS * CW_SMALL_Q) {  // more flagged queries than the device-side rounds take: finish them now
             for (int off = CW_FUSED_FB_ROUNDS * CW_SMALL_Q; off < n_flag; off += CW_SMALL_Q)
                 if ((rc = cw_small_predict_impl(&fi->ix, w->Q_dev, CW_SMALL_Q, w->flag + 4, w->flag, off, 1, k, w->sm_Q, w->sm_scores,
-                                                w->sm_scratch, w->sm_sid, w->sm_val, w->sm_n, w->out_sid_dev, w->out_val_dev, st)))
+                                                w->sm_scratch, w->sm_sid, w->sm_val, w->sm_n, w->out_sid_dev, w->out_val_dev, st,
+                                                nullptr)))
                     return rc;
             cudaMemcpyAsync(out_sid_host + lo * k, w->out_sid_dev, (size_t)n * k * sizeof(int32_t), cudaMemcpyDeviceToHost, st);
             cudaMemcpyAsync(out_val_host + lo * k, w->out_val_dev, (size_t)n * k * sizeof(float), cudaMemcpyDeviceToHost, st);

@@ -8,11 +8,13 @@ get_weight_schedule_info :414, force_rebuild_index :422, cobweb_predict_fast :42
 cobweb_predict :435, print_tree :463, dump_json :484, load_json :501, __len__ :557, attributes
 sentences / sentence_to_node / tree / device / max_init_search.  visualize_subtrees (graphviz
 rendering) is out of scope and raises NotImplementedError.
-Additive: predict_fast_batch / predict_batch / rank_scores_batch for query batches.
+Additive: predict_fast_batch / predict_batch / rank_scores_batch for query batches; set_sentence_tags /
+get_sentence_tags and predict_fast_batch(..., query_tags=) for tag-filtered retrieval.
 
 Deliberate differences (DESIGN.md "Tie-breaking"): no 1e-6*randn noise and no in-leaf
 random.shuffle -- exact ties are broken by ascending sentence id.
 """
+import base64
 import ctypes as C
 import json
 import os
@@ -105,6 +107,7 @@ class DenseIndex:
         self.hx = None
         self._rows = None
         self._pos_of_sid = None
+        self._tag_cache = None
         self.mode = "fp32"
         self.eps_scale = self.EPS_SCALE
         self.audit_every = self.AUDIT_EVERY
@@ -213,6 +216,22 @@ class DenseIndex:
             p[self.pos_rec[:, 3].long()] = torch.arange(self.n_pos, dtype=torch.int32, device=p.device)
             self._pos_of_sid = p
         return self._pos_of_sid
+
+    def tag_arrays(self, sent_tags, version):
+        """What the tagged kernels read of the sentences' tag words sent_tags [n sentences] int32, derived once per tag
+        version: "pos" [n_pos] the tag of each position's sentence and, once the fused operands exist, "leaf" [n_leaf] the
+        OR of the tags of each fused leaf row's sentences (cw_leaf_tags)."""
+        c = self._tag_cache
+        if c is None or c["version"] != version:
+            c = self._tag_cache = {"version": version, "sent": sent_tags, "leaf": None,
+                                   "pos": sent_tags[self.pos_rec[:, 3].long()].contiguous()}
+        if c["leaf"] is None and self.hx is not None:
+            hx = self.hx
+            leaf = torch.empty(hx["n_leaf"], dtype=torch.int32, device=sent_tags.device)
+            _lib.check(_lib.load().cw_leaf_tags(hx["sent_off"].data_ptr(), hx["sent_ids"].data_ptr(), hx["n_leaf"],
+                                                sent_tags.data_ptr(), leaf.data_ptr(), _lib.stream_ptr()), "cw_leaf_tags")
+            c["leaf"] = leaf
+        return c
 
     def bytes(self):
         b = (self.R.numel() + self.MB.numel() + self.sumlog.numel()) * 4
@@ -358,9 +377,16 @@ class DenseIndex:
                                                 _lib.stream_ptr()), "cw_small_predict")
         return sids, vals
 
-    def predict(self, Q, k, want_leaf_scores=False, mode=None, small=True):
+    def predict(self, Q, k, want_leaf_scores=False, mode=None, small=True, query_tags=None, sent_tags=None, tag_version=None):
         """Device batch -> (sids [nq,k] int32, scores [nq,k], leaf_scores [nq,L] or None).  mode overrides self.mode for
-        this call; small=False keeps batches of up to SMALL_Q queries off the small-batch path (tests)."""
+        this call; small=False keeps batches of up to SMALL_Q queries off the small-batch path (tests).  query_tags [nq]
+        int32 (with the sentences' tag words sent_tags and their version): only sentences s with
+        sent_tags[s] & query_tags[q] != 0 are ranked, short rows padded with -1 / -inf (predict_tagged)."""
+        if query_tags is not None:
+            if want_leaf_scores:
+                raise ValueError("leaf scores are not filtered by tags")
+            s, v = self.predict_tagged(Q, k, query_tags, sent_tags, tag_version, mode=mode, small=small)
+            return s, v, None
         L = _lib.load()
         if want_leaf_scores and self.sentence_ids is not None:
             raise ValueError("leaf scores are indexed by global sentence id; not available on a sentence shard")
@@ -406,6 +432,65 @@ class DenseIndex:
                                              sids[lo:lo + nq].data_ptr(), vals[lo:lo + nq].data_ptr(),
                                              ws["scratch"].data_ptr(), _lib.stream_ptr()), "cw_dense_paths_topk")
         return sids, vals, leaf
+
+    def predict_tagged(self, Q, k, query_tags, sent_tags, tag_version, mode=None, small=True):
+        """The k (1..MAX_K) best eligible sentences per query, routed like predict: cw_small_predict_tagged for up to
+        SMALL_Q queries, cw_fused_predict_tagged in "fused" mode, else cw_dense_paths_topk_tagged over the FP32 node scores."""
+        if self.sentence_ids is not None:
+            raise ValueError("tag filters are indexed by global sentence id; not available on a sentence shard")
+        L = _lib.load()
+        mode = mode or self.mode
+        if mode not in self.MODES:
+            raise ValueError(f"mode must be one of {self.MODES}")
+        if not 1 <= k <= _lib.MAX_K:
+            raise ValueError(f"k must lie in [1, {_lib.MAX_K}]")
+        nq = Q.shape[0]
+        sids = torch.full((nq, k), -1, dtype=torch.int32, device=Q.device)
+        vals = torch.full((nq, k), float("-inf"), dtype=torch.float32, device=Q.device)
+        if not nq or not self.n_pos:
+            return sids, vals
+        if mode == "fused" and self.hx is None:
+            self._build_fused()
+        t = self.tag_arrays(sent_tags, tag_version)
+        tf = _lib.CwTagFilter()
+        tf.query_tags, tf.pos_tags, tf.sent_tags = query_tags.data_ptr(), t["pos"].data_ptr(), sent_tags.data_ptr()
+        tf.leaf_tags = t["leaf"].data_ptr() if t["leaf"] is not None else None
+        st = _lib.stream_ptr()
+        if small and nq <= _lib.SMALL_Q:
+            sm = self.small_workspace(k)
+            _lib.check(L.cw_small_predict_tagged(C.byref(self.ix), C.byref(tf), Q.data_ptr(), nq, None, None, 0, 0, k,
+                                                 sm["Q"].data_ptr(), sm["scores"].data_ptr(), sm["scratch"].data_ptr(),
+                                                 sm["sid"].data_ptr(), sm["val"].data_ptr(), sm["n"].data_ptr(), sids.data_ptr(),
+                                                 vals.data_ptr(), st), "cw_small_predict_tagged")
+            return sids, vals
+        if mode == "fused" and k <= _lib.FUSED_MAX_K and self.nn >= self.TENSOR_MIN_NODES and self.hx["smem_ok"]:
+            hw = self.fused_workspace(nq, k)
+            fi, w = self._fused_struct(hw)
+            hw["stats"].zero_()
+            _lib.check(L.cw_fused_predict_tagged(C.byref(fi), C.byref(w), C.byref(tf), Q.data_ptr(), nq, k, sids.data_ptr(),
+                                                 vals.data_ptr(), st), "cw_fused_predict_tagged")
+            hw["stats_host"].copy_(hw["stats"], non_blocking=True)
+            torch.cuda.current_stream().synchronize()
+            stats = hw["stats_host"].numpy().copy()
+            self._account(stats)
+            if stats[1]:  # flagged queries past the device-side rounds: the FP32 form answers them
+                idx = torch.nonzero(sids[:, 0] == _lib.SID_UNRESOLVED).view(-1)
+                s2, v2 = self.predict_tagged(Q[idx].contiguous(), k, query_tags[idx].contiguous(), sent_tags, tag_version,
+                                             mode="fp32", small=False)
+                sids[idx], vals[idx] = s2, v2
+            return sids, vals
+        step = self.chunk_queries()
+        for lo in range(0, nq, step):
+            n = min(step, nq - lo)
+            ws = self.workspace(min(step, nq), k)
+            q = Q[lo:lo + n]
+            _lib.check(L.cw_dense_node_scores(C.byref(self.ix), q.data_ptr(), n, ws["xt"].data_ptr(), ws["scores"].data_ptr(),
+                                              ws["ldq"], st), "cw_dense_node_scores")
+            tf.query_tags = query_tags[lo:lo + n].data_ptr()
+            _lib.check(L.cw_dense_paths_topk_tagged(C.byref(self.ix), C.byref(tf), ws["scores"].data_ptr(), ws["ldq"], n, k,
+                                                    sids[lo:lo + n].data_ptr(), vals[lo:lo + n].data_ptr(),
+                                                    ws["scratch"].data_ptr(), st), "cw_dense_paths_topk_tagged")
+        return sids, vals
 
     def predict_one(self, q, k):
         """One query (contiguous float32 numpy row) -> list of k sentence ids: the shortest way through the exact
@@ -729,17 +814,90 @@ class CobwebWrapper:
         emb = input if is_embedding else self.encode_func([input])[0]
         return self.tree._as_device_vec(emb).reshape(1, -1)
 
-    def predict_fast_batch(self, Q, k=5):
-        """Batched cobweb_predict_fast(return_ids=True): device tensors (ids [nq,k], scores [nq,k])."""
+    # ------------------------------------------------------------------ sentence tags
+    @staticmethod
+    def _as_tag_words(v, n, what):
+        """Integers in [-2^31, 2^32) (a scalar, broadcast, or [n]) -> device int32 [n] with the same 32 bits."""
+        t = torch.as_tensor(v, device="cuda")
+        if t.dtype.is_floating_point or t.dtype.is_complex or t.dtype == torch.bool or t.dim() > 1:
+            raise ValueError(f"{what} must be integers: a scalar or a vector")
+        t = t.to(torch.int64)
+        if t.dim() == 0:
+            t = t.expand(n)
+        elif t.numel() != n:
+            raise ValueError(f"{what} has {t.numel()} entries for {n}")
+        if t.numel() and bool(((t < -(1 << 31)) | (t >= (1 << 32))).any()):
+            raise ValueError(f"{what} must be 32-bit words (integers in [-2^31, 2^32))")
+        return torch.where(t >= (1 << 31), t - (1 << 32), t).to(torch.int32).contiguous()
+
+    def _tag_words(self):
+        """Device int32 [len(self)]: the tag word of every sentence; sentences never tagged (added since) have 0."""
+        t, n = getattr(self, "_tags", None), len(self)
+        if t is None or t.numel() != n:
+            new = torch.zeros(n, dtype=torch.int32, device=self.device)
+            if t is not None:
+                new[: min(n, t.numel())] = t[: min(n, t.numel())]
+            self._tags = new
+            self._tag_version = getattr(self, "_tag_version", 0) + 1
+        return self._tags
+
+    def set_sentence_tags(self, ids, tags):
+        """Additive: set the 32-bit tag word of sentences ids [m] to tags ([m] or one value for all; integers in
+        [-2^31, 2^32), read as 32 bits).  Every sentence starts with tag 0.  predict_fast_batch(Q, k, query_tags=...) ranks
+        for query q only the sentences s with tags[s] & query_tags[q] != 0."""
+        cur = self._tag_words()
+        ids = torch.as_tensor(ids, device=self.device)
+        if ids.dtype.is_floating_point or ids.dtype.is_complex or ids.dtype == torch.bool or ids.dim() > 1:
+            raise ValueError("ids must be an integer vector of sentence ids")
+        ids = ids.reshape(-1).to(torch.int64)
+        n = len(self)
+        if ids.numel() and bool(((ids < 0) | (ids >= n)).any()):
+            raise ValueError(f"sentence ids must lie in [0, {n})")
+        if torch.unique(ids).numel() != ids.numel():
+            raise ValueError("ids must not repeat")
+        words = self._as_tag_words(tags, ids.numel(), "tags")
+        new = cur.clone()
+        new[ids] = words
+        self._tags = new
+        self._tag_version += 1
+
+    def get_sentence_tags(self):
+        """Additive: the tag word of every sentence, device int32 [len(self)] (a copy)."""
+        return self._tag_words().clone()
+
+    def predict_fast_batch(self, Q, k=5, query_tags=None):
+        """Batched cobweb_predict_fast(return_ids=True): device tensors (ids [nq,k], scores [nq,k]).  query_tags
+        (additive): a mask per query ([nq]) or one for all; query q then ranks only the sentences s with
+        tags[s] & query_tags[q] != 0 (set_sentence_tags), and rows with fewer than k of them are padded with -1 / -inf.
+        Scores are the same bits as rank_scores_batch(Q)."""
         self.build_prediction_index()
         Q = self.tree._as_device_mat(Q)
         k = min(int(k), self._index.n_pos)
+        if query_tags is not None:
+            return self._predict_fast_tagged(Q, k, query_tags)
         if k > _lib.MAX_K:
             _, _, leaf = self._index.predict(Q, 0, want_leaf_scores=True, mode="fp32")
             vals, ids = torch.sort(leaf, dim=1, descending=True, stable=True)
             return ids[:, :k].to(torch.int32), vals[:, :k]
         sids, vals, _ = self._index.predict(Q, k)
         return sids, vals
+
+    def _predict_fast_tagged(self, Q, k, query_tags):
+        qt = self._as_tag_words(query_tags, Q.shape[0], "query_tags")
+        tags = self._tag_words()
+        if k < 1:
+            return (torch.empty((Q.shape[0], 0), dtype=torch.int32, device=Q.device),
+                    torch.empty((Q.shape[0], 0), dtype=torch.float32, device=Q.device))
+        if k <= _lib.MAX_K:
+            return self._index.predict_tagged(Q, k, qt, tags, self._tag_version)
+        # the leaf matrix with ineligible entries at -inf; eligible entries first, each part in (score desc, id asc)
+        _, _, leaf = self._index.predict(Q, 0, want_leaf_scores=True, mode="fp32")
+        elig = (tags.unsqueeze(0) & qt.unsqueeze(1)) != 0
+        vals, ids = torch.sort(leaf.masked_fill_(~elig, float("-inf")), dim=1, descending=True, stable=True)
+        e = elig.gather(1, ids)
+        _, o = torch.sort((~e).to(torch.uint8), dim=1, stable=True)
+        ids, vals, e = ids.gather(1, o)[:, :k], vals.gather(1, o)[:, :k], e.gather(1, o)[:, :k]
+        return torch.where(e, ids, -1).to(torch.int32), vals
 
     def predict_fast_sharded(self, Q, k=5, world=None, rank=None):
         """Store-sharded dense predict (SURVEY 8e, trees beyond one HBM): this rank indexes and
@@ -951,10 +1109,12 @@ class CobwebWrapper:
     def save_snapshot(self, path):
         """Additive (SURVEY 8f-2): binary snapshot of tree + sentence map + sentences; a 1M-node tree is a few seconds of
         streaming instead of gigabytes of decimal JSON.  load_snapshot restores an equivalent wrapper."""
-        self.tree.save_snapshot(path, self._leaf_of_sentence,
-                                extra={"sentences": self.sentences if any(s is not None for s in self.sentences) else None,
-                                       "n_sentences": len(self.sentences), "max_init_search": self.max_init_search,
-                                       "level_weights": self._level_weights})
+        extra = {"sentences": self.sentences if any(s is not None for s in self.sentences) else None,
+                 "n_sentences": len(self.sentences), "max_init_search": self.max_init_search, "level_weights": self._level_weights}
+        tags = self._tag_words()
+        if bool((tags != 0).any()):  # little-endian int32 words, base64 (a snapshot without them loads as all 0)
+            extra["sentence_tags"] = base64.b64encode(tags.cpu().numpy().astype("<i4").tobytes()).decode()
+        self.tree.save_snapshot(path, self._leaf_of_sentence, extra=extra)
 
     @staticmethod
     def load_snapshot(path, encode_func=lambda x: x):
@@ -969,6 +1129,9 @@ class CobwebWrapper:
         w.max_init_search = extra.get("max_init_search", 100000)
         w._level_weights = extra.get("level_weights")
         w.tree._sent_stale, w.tree._sent_loader = True, w._load_sentence_lists
+        if extra.get("sentence_tags"):
+            t = np.frombuffer(base64.b64decode(extra["sentence_tags"]), "<i4").astype(np.int32)
+            w._tags, w._tag_version = torch.as_tensor(t, device=w.device), 1
         return w
 
     def get_node_path_stats(self, sentence_id):
