@@ -130,8 +130,17 @@ class DenseIndex:
 
     def fused_ready(self, k):
         """True if a top-k request is served by the fused pipeline (else: the FP32 form)."""
-        return (self.mode == "fused" and self.hx is not None and 1 <= k <= _lib.FUSED_MAX_K and
-                self.nn >= self.TENSOR_MIN_NODES and self.hx["smem_ok"])
+        return self._route(1, k, self.mode, small=False) == "fused"
+
+    def _route(self, nq, k, mode, small=True, leaf=False):
+        """The pipeline of a call for the top-k of nq queries: "small" (the exact small-batch path), "fused" or "fp32".
+        Every pipeline returns the same ids and scores; this rule only decides which is fastest."""
+        if small and not leaf and 1 <= k <= _lib.MAX_K and 0 < nq <= _lib.SMALL_Q and self.n_pos:
+            return "small"
+        if (mode == "fused" and not leaf and self.hx is not None and 1 <= k <= _lib.FUSED_MAX_K and
+                self.nn >= self.TENSOR_MIN_NODES and self.hx["smem_ok"] and nq > 0):
+            return "fused"
+        return "fp32"
 
     def _build_fused(self):
         """Operands of the fused mode: fp16 operand sets for the internal rows (hi + lo) and the leaf rows (hi), per-leaf
@@ -265,8 +274,17 @@ class DenseIndex:
             val=torch.empty((nq, k), dtype=torch.float32, device=dev),
             scratch=torch.empty(max(1, nq * L.cw_topk_chunks(max(self.n_pos, 1)) * k * 2), dtype=torch.int32, device=dev),
         )
+        w = ws["w"] = _lib.CwDenseWork()
+        w.Q_dev, w.xt_scratch, w.node_scores, w.ldq = ws["q"].data_ptr(), ws["xt"].data_ptr(), ws["scores"].data_ptr(), ldq
+        w.out_sid_dev, w.out_score_dev, w.scratch = ws["sid"].data_ptr(), ws["val"].data_ptr(), ws["scratch"].data_ptr()
         self._ws = ws
         return ws
+
+    def _fp32_chunks(self, nq, k):
+        """Chunks of up to chunk_queries() queries for the FP32 form: yields (row slice, workspace)."""
+        step = self.chunk_queries()
+        for lo in range(0, nq, step):
+            yield slice(lo, min(nq, lo + step)), self.workspace(min(step, nq), k)
 
     def small_workspace(self, k):
         """Buffers of the exact small-batch path (cw_small_predict)."""
@@ -286,6 +304,8 @@ class DenseIndex:
             sid_host=torch.empty((Q, k), dtype=torch.int32).pin_memory(),
             val_host=torch.empty((Q, k), dtype=torch.float32).pin_memory(),
         )
+        # sm_Q, sm_scores, sm_scratch, sm_sid, sm_val, sm_n of every small-batch entry point and of cw_fused_work
+        sm["ptrs"] = tuple(sm[n].data_ptr() for n in ("Q", "scores", "scratch", "sid", "val", "n"))
         return sm
 
     def fused_chunk_queries(self):
@@ -327,8 +347,7 @@ class DenseIndex:
         w.Q_dev, w.A_int, w.A_leaf, w.qv, w.S = (hw[n].data_ptr() for n in ("Q", "A_int", "A_leaf", "qv", "S"))
         w.slots, w.tau, w.cnt, w.cand_val, w.cand_row = (hw[n].data_ptr() for n in ("slots", "tau", "cnt", "cand_val", "cand_row"))
         w.flag, w.out_sid_dev, w.out_val_dev, w.stats = (hw[n].data_ptr() for n in ("flag", "sid", "val", "stats"))
-        w.sm_Q, w.sm_scores, w.sm_scratch = sm["Q"].data_ptr(), sm["scores"].data_ptr(), sm["scratch"].data_ptr()
-        w.sm_sid, w.sm_val, w.sm_n = sm["sid"].data_ptr(), sm["val"].data_ptr(), sm["n"].data_ptr()
+        w.sm_Q, w.sm_scores, w.sm_scratch, w.sm_sid, w.sm_val, w.sm_n = sm["ptrs"]
         hw["w"] = w
         self._hws = hw
         return hw
@@ -367,140 +386,109 @@ class DenseIndex:
 
     def predict_small(self, Q, k):
         """Exact small-batch path for up to SMALL_Q queries on the device (cw_small_predict)."""
-        nq = Q.shape[0]
-        sm = self.small_workspace(k)
-        sids = torch.empty((nq, k), dtype=torch.int32, device=Q.device)
-        vals = torch.empty((nq, k), dtype=torch.float32, device=Q.device)
-        _lib.check(_lib.load().cw_small_predict(C.byref(self.ix), Q.data_ptr(), nq, None, None, 0, 0, k, sm["Q"].data_ptr(),
-                                                sm["scores"].data_ptr(), sm["scratch"].data_ptr(), sm["sid"].data_ptr(),
-                                                sm["val"].data_ptr(), sm["n"].data_ptr(), sids.data_ptr(), vals.data_ptr(),
-                                                _lib.stream_ptr()), "cw_small_predict")
+        sids = torch.empty((Q.shape[0], k), dtype=torch.int32, device=Q.device)
+        vals = torch.empty((Q.shape[0], k), dtype=torch.float32, device=Q.device)
+        self._run_small(Q, k, sids, vals)
         return sids, vals
 
     def predict(self, Q, k, want_leaf_scores=False, mode=None, small=True, query_tags=None, sent_tags=None, tag_version=None):
         """Device batch -> (sids [nq,k] int32, scores [nq,k], leaf_scores [nq,L] or None).  mode overrides self.mode for
         this call; small=False keeps batches of up to SMALL_Q queries off the small-batch path (tests).  query_tags [nq]
         int32 (with the sentences' tag words sent_tags and their version): only sentences s with
-        sent_tags[s] & query_tags[q] != 0 are ranked, short rows padded with -1 / -inf (predict_tagged)."""
-        if query_tags is not None:
-            if want_leaf_scores:
-                raise ValueError("leaf scores are not filtered by tags")
-            s, v = self.predict_tagged(Q, k, query_tags, sent_tags, tag_version, mode=mode, small=small)
-            return s, v, None
-        L = _lib.load()
-        if want_leaf_scores and self.sentence_ids is not None:
-            raise ValueError("leaf scores are indexed by global sentence id; not available on a sentence shard")
+        sent_tags[s] & query_tags[q] != 0 are ranked (k in 1..MAX_K), short rows padded with -1 / -inf."""
+        if query_tags is not None and want_leaf_scores:
+            raise ValueError("leaf scores are not filtered by tags")
+        if self.sentence_ids is not None and (want_leaf_scores or query_tags is not None):
+            what = "leaf scores" if want_leaf_scores else "tag filters"
+            raise ValueError(f"{what} are indexed by global sentence id; not available on a sentence shard")
         mode = mode or self.mode
         if mode not in self.MODES:
             raise ValueError(f"mode must be one of {self.MODES}")
-        nq_total = Q.shape[0]
+        nq, tf = Q.shape[0], None
+        if query_tags is None:
+            sids = torch.empty((nq, max(k, 1)), dtype=torch.int32, device=Q.device)
+            vals = torch.empty((nq, max(k, 1)), dtype=torch.float32, device=Q.device)
+        else:
+            if not 1 <= k <= _lib.MAX_K:
+                raise ValueError(f"k must lie in [1, {_lib.MAX_K}]")
+            sids = torch.full((nq, k), -1, dtype=torch.int32, device=Q.device)
+            vals = torch.full((nq, k), float("-inf"), dtype=torch.float32, device=Q.device)
+            if not nq or not self.n_pos:
+                return sids, vals, None
         if mode == "fused" and self.hx is None and self.n_pos:
             self._build_fused()
-        if small and not want_leaf_scores and 1 <= k <= _lib.MAX_K and 0 < nq_total <= _lib.SMALL_Q and self.n_pos:
-            s, v = self.predict_small(Q, k)
-            return s, v, None
-        if mode == "fused" and not want_leaf_scores and self.hx is not None and 1 <= k <= _lib.FUSED_MAX_K and \
-                self.nn >= self.TENSOR_MIN_NODES and self.hx["smem_ok"] and nq_total > 0:
-            hw = self.fused_workspace(nq_total, k)
-            fi, w = self._fused_struct(hw)
-            sids = torch.empty((nq_total, k), dtype=torch.int32, device=Q.device)
-            vals = torch.empty((nq_total, k), dtype=torch.float32, device=Q.device)
-            hw["stats"].zero_()
-            _lib.check(L.cw_fused_predict(C.byref(fi), C.byref(w), Q.data_ptr(), nq_total, k, sids.data_ptr(), vals.data_ptr(),
-                                          _lib.stream_ptr()), "cw_fused_predict")
-            hw["stats_host"].copy_(hw["stats"], non_blocking=True)
-            torch.cuda.current_stream().synchronize()  # the one read-back of a call: counters (flagged / audit)
-            st = hw["stats_host"].numpy().copy()
-            self._account(st)
-            if st[1]:  # more flagged queries in a chunk than the device-side rounds take: the FP32 form answers them
-                idx = torch.nonzero(sids[:, 0] == _lib.SID_UNRESOLVED).view(-1)
-                s2, v2, _ = self.predict(Q[idx].contiguous(), k, mode="fp32", small=False)
-                sids[idx], vals[idx] = s2, v2
-            return sids, vals, None
-        step = self.chunk_queries()
-        sids = torch.empty((nq_total, max(k, 1)), dtype=torch.int32, device=Q.device)
-        vals = torch.empty((nq_total, max(k, 1)), dtype=torch.float32, device=Q.device)
-        leaf = torch.empty((nq_total, self.n_pos), dtype=torch.float32, device=Q.device) if want_leaf_scores else None
-        for lo in range(0, nq_total, step):
-            nq = min(step, nq_total - lo)
-            ws = self.workspace(min(step, nq_total), k)
-            q = Q[lo:lo + nq]
-            _lib.check(L.cw_dense_node_scores(C.byref(self.ix), q.data_ptr(), nq, ws["xt"].data_ptr(), ws["scores"].data_ptr(),
-                                              ws["ldq"], _lib.stream_ptr()), "cw_dense_node_scores")
-            _lib.check(L.cw_dense_paths_topk(C.byref(self.ix), ws["scores"].data_ptr(), ws["ldq"], nq, k,
-                                             leaf[lo:lo + nq].data_ptr() if leaf is not None else None,
-                                             sids[lo:lo + nq].data_ptr(), vals[lo:lo + nq].data_ptr(),
-                                             ws["scratch"].data_ptr(), _lib.stream_ptr()), "cw_dense_paths_topk")
+        if query_tags is not None:
+            t = self.tag_arrays(sent_tags, tag_version)
+            tf = _lib.CwTagFilter()
+            tf.query_tags, tf.pos_tags, tf.sent_tags = query_tags.data_ptr(), t["pos"].data_ptr(), sent_tags.data_ptr()
+            tf.leaf_tags = t["leaf"].data_ptr() if t["leaf"] is not None else None
+        leaf = torch.empty((nq, self.n_pos), dtype=torch.float32, device=Q.device) if want_leaf_scores else None
+        route = self._route(nq, k, mode, small, want_leaf_scores)
+        if route == "small":
+            self._run_small(Q, k, sids, vals, tf)
+        elif route == "fused":
+            self._run_fused(Q, k, sids, vals, tf, query_tags)
+        else:
+            self._run_fp32(Q, k, sids, vals, tf, query_tags, leaf)
         return sids, vals, leaf
 
-    def predict_tagged(self, Q, k, query_tags, sent_tags, tag_version, mode=None, small=True):
-        """The k (1..MAX_K) best eligible sentences per query, routed like predict: cw_small_predict_tagged for up to
-        SMALL_Q queries, cw_fused_predict_tagged in "fused" mode, else cw_dense_paths_topk_tagged over the FP32 node scores."""
-        if self.sentence_ids is not None:
-            raise ValueError("tag filters are indexed by global sentence id; not available on a sentence shard")
-        L = _lib.load()
-        mode = mode or self.mode
-        if mode not in self.MODES:
-            raise ValueError(f"mode must be one of {self.MODES}")
-        if not 1 <= k <= _lib.MAX_K:
-            raise ValueError(f"k must lie in [1, {_lib.MAX_K}]")
-        nq = Q.shape[0]
-        sids = torch.full((nq, k), -1, dtype=torch.int32, device=Q.device)
-        vals = torch.full((nq, k), float("-inf"), dtype=torch.float32, device=Q.device)
-        if not nq or not self.n_pos:
-            return sids, vals
-        if mode == "fused" and self.hx is None:
-            self._build_fused()
-        t = self.tag_arrays(sent_tags, tag_version)
-        tf = _lib.CwTagFilter()
-        tf.query_tags, tf.pos_tags, tf.sent_tags = query_tags.data_ptr(), t["pos"].data_ptr(), sent_tags.data_ptr()
-        tf.leaf_tags = t["leaf"].data_ptr() if t["leaf"] is not None else None
-        st = _lib.stream_ptr()
-        if small and nq <= _lib.SMALL_Q:
-            sm = self.small_workspace(k)
-            _lib.check(L.cw_small_predict_tagged(C.byref(self.ix), C.byref(tf), Q.data_ptr(), nq, None, None, 0, 0, k,
-                                                 sm["Q"].data_ptr(), sm["scores"].data_ptr(), sm["scratch"].data_ptr(),
-                                                 sm["sid"].data_ptr(), sm["val"].data_ptr(), sm["n"].data_ptr(), sids.data_ptr(),
-                                                 vals.data_ptr(), st), "cw_small_predict_tagged")
-            return sids, vals
-        if mode == "fused" and k <= _lib.FUSED_MAX_K and self.nn >= self.TENSOR_MIN_NODES and self.hx["smem_ok"]:
-            hw = self.fused_workspace(nq, k)
-            fi, w = self._fused_struct(hw)
-            hw["stats"].zero_()
-            _lib.check(L.cw_fused_predict_tagged(C.byref(fi), C.byref(w), C.byref(tf), Q.data_ptr(), nq, k, sids.data_ptr(),
-                                                 vals.data_ptr(), st), "cw_fused_predict_tagged")
-            hw["stats_host"].copy_(hw["stats"], non_blocking=True)
-            torch.cuda.current_stream().synchronize()
-            stats = hw["stats_host"].numpy().copy()
-            self._account(stats)
-            if stats[1]:  # flagged queries past the device-side rounds: the FP32 form answers them
-                idx = torch.nonzero(sids[:, 0] == _lib.SID_UNRESOLVED).view(-1)
-                s2, v2 = self.predict_tagged(Q[idx].contiguous(), k, query_tags[idx].contiguous(), sent_tags, tag_version,
-                                             mode="fp32", small=False)
-                sids[idx], vals[idx] = s2, v2
-            return sids, vals
-        step = self.chunk_queries()
-        for lo in range(0, nq, step):
-            n = min(step, nq - lo)
-            ws = self.workspace(min(step, nq), k)
-            q = Q[lo:lo + n]
-            _lib.check(L.cw_dense_node_scores(C.byref(self.ix), q.data_ptr(), n, ws["xt"].data_ptr(), ws["scores"].data_ptr(),
-                                              ws["ldq"], st), "cw_dense_node_scores")
-            tf.query_tags = query_tags[lo:lo + n].data_ptr()
-            _lib.check(L.cw_dense_paths_topk_tagged(C.byref(self.ix), C.byref(tf), ws["scores"].data_ptr(), ws["ldq"], n, k,
-                                                    sids[lo:lo + n].data_ptr(), vals[lo:lo + n].data_ptr(),
-                                                    ws["scratch"].data_ptr(), st), "cw_dense_paths_topk_tagged")
-        return sids, vals
+    # Each runner writes the top-k of the queries Q into sids / vals.  Given a tag filter tf (and the query tags qt it
+    # points to), it calls the _tagged form of its entry points, which take the untagged form's arguments plus tf.
+    def _run_small(self, Q, k, sids, vals, tf=None):
+        """The exact small-batch path (cw_small_predict[_tagged]) for up to SMALL_Q queries."""
+        L, sm = _lib.load(), self.small_workspace(k)
+        args = (Q.data_ptr(), Q.shape[0], None, None, 0, 0, k, *sm["ptrs"], sids.data_ptr(), vals.data_ptr(), _lib.stream_ptr())
+        if tf is None:
+            _lib.check(L.cw_small_predict(C.byref(self.ix), *args), "cw_small_predict")
+        else:
+            _lib.check(L.cw_small_predict_tagged(C.byref(self.ix), C.byref(tf), *args), "cw_small_predict_tagged")
+
+    def _run_fused(self, Q, k, sids, vals, tf=None, qt=None):
+        """The fused pipeline (cw_fused_predict[_tagged]); the FP32 form answers the rows it leaves unresolved."""
+        L, nq = _lib.load(), Q.shape[0]
+        hw = self.fused_workspace(nq, k)
+        fi, w = self._fused_struct(hw)
+        hw["stats"].zero_()
+        args = (Q.data_ptr(), nq, k, sids.data_ptr(), vals.data_ptr(), _lib.stream_ptr())
+        if tf is None:
+            _lib.check(L.cw_fused_predict(C.byref(fi), C.byref(w), *args), "cw_fused_predict")
+        else:
+            _lib.check(L.cw_fused_predict_tagged(C.byref(fi), C.byref(w), C.byref(tf), *args), "cw_fused_predict_tagged")
+        hw["stats_host"].copy_(hw["stats"], non_blocking=True)
+        torch.cuda.current_stream().synchronize()  # the one read-back of a call: counters (flagged / audit)
+        st = hw["stats_host"].numpy().copy()
+        self._account(st)
+        if st[1]:  # more flagged queries in a chunk than the device-side rounds take: the FP32 form answers them
+            idx = torch.nonzero(sids[:, 0] == _lib.SID_UNRESOLVED).view(-1)
+            s2, v2 = sids[idx], vals[idx]
+            self._run_fp32(Q[idx].contiguous(), k, s2, v2, tf, qt[idx].contiguous() if tf is not None else None)
+            sids[idx], vals[idx] = s2, v2
+
+    def _run_fp32(self, Q, k, sids, vals, tf=None, qt=None, leaf=None):
+        """The FP32 form chunk by chunk: node scores (cw_dense_node_scores), then path sums and top-k
+        (cw_dense_paths_topk[_tagged]); leaf [nq, n_pos] (untagged only) also receives every sentence's score."""
+        L, st = _lib.load(), _lib.stream_ptr()
+        for r, ws in self._fp32_chunks(Q.shape[0], k):
+            q = Q[r]
+            _lib.check(L.cw_dense_node_scores(C.byref(self.ix), q.data_ptr(), q.shape[0], ws["xt"].data_ptr(),
+                                              ws["scores"].data_ptr(), ws["ldq"], st), "cw_dense_node_scores")
+            if tf is None:
+                _lib.check(L.cw_dense_paths_topk(C.byref(self.ix), ws["scores"].data_ptr(), ws["ldq"], q.shape[0], k,
+                                                 leaf[r].data_ptr() if leaf is not None else None, sids[r].data_ptr(),
+                                                 vals[r].data_ptr(), ws["scratch"].data_ptr(), st), "cw_dense_paths_topk")
+            else:
+                tf.query_tags = qt[r].data_ptr()
+                _lib.check(L.cw_dense_paths_topk_tagged(C.byref(self.ix), C.byref(tf), ws["scores"].data_ptr(), ws["ldq"],
+                                                        q.shape[0], k, sids[r].data_ptr(), vals[r].data_ptr(),
+                                                        ws["scratch"].data_ptr(), st), "cw_dense_paths_topk_tagged")
 
     def predict_one(self, q, k):
         """One query (contiguous float32 numpy row) -> list of k sentence ids: the shortest way through the exact
         small-batch path (one C call: H2D, two kernels + merge, D2H, sync; no torch objects created)."""
         sm = self.small_workspace(k)
         sid, val = sm["sid_host"], sm["val_host"]
-        _lib.check(_lib.load().cw_small_predict_host(C.byref(self.ix), q.ctypes.data, 1, k, sm["Q"].data_ptr(),
-                                                     sm["scores"].data_ptr(), sm["scratch"].data_ptr(), sm["sid"].data_ptr(),
-                                                     sm["val"].data_ptr(), sm["n"].data_ptr(), sid.data_ptr(), val.data_ptr(),
-                                                     _lib.stream_ptr()), "cw_small_predict_host")
+        _lib.check(_lib.load().cw_small_predict_host(C.byref(self.ix), q.ctypes.data, 1, k, *sm["ptrs"], sid.data_ptr(),
+                                                     val.data_ptr(), _lib.stream_ptr()), "cw_small_predict_host")
         return sid.view(-1)[:k].tolist()
 
     # ------------------------------------------------------------------ pair scores
@@ -584,35 +572,28 @@ class DenseIndex:
         (FP32 form); H2D + kernels + D2H + sync inside."""
         L = _lib.load()
         Qh = Q_host if torch.is_tensor(Q_host) else torch.from_numpy(np.ascontiguousarray(Q_host, np.float32))
-        nq_total = Qh.shape[0]
+        nq = Qh.shape[0]
         if out_sid is None:
-            out_sid = torch.empty((nq_total, k), dtype=torch.int32)
-            out_val = torch.empty((nq_total, k), dtype=torch.float32)
-        if 0 < nq_total <= _lib.SMALL_Q and 1 <= k <= _lib.MAX_K and self.n_pos:
+            out_sid = torch.empty((nq, k), dtype=torch.int32)
+            out_val = torch.empty((nq, k), dtype=torch.float32)
+        route = self._route(nq, k, self.mode)
+        if route == "small":
             sm = self.small_workspace(k)
-            _lib.check(L.cw_small_predict_host(C.byref(self.ix), Qh.data_ptr(), nq_total, k, sm["Q"].data_ptr(),
-                                               sm["scores"].data_ptr(), sm["scratch"].data_ptr(), sm["sid"].data_ptr(),
-                                               sm["val"].data_ptr(), sm["n"].data_ptr(), out_sid.data_ptr(), out_val.data_ptr(),
-                                               _lib.stream_ptr()), "cw_small_predict_host")
-            return out_sid, out_val
-        if self.fused_ready(k) and nq_total > 0:
-            hw = self.fused_workspace(nq_total, k)
+            _lib.check(L.cw_small_predict_host(C.byref(self.ix), Qh.data_ptr(), nq, k, *sm["ptrs"], out_sid.data_ptr(),
+                                               out_val.data_ptr(), _lib.stream_ptr()), "cw_small_predict_host")
+        elif route == "fused":
+            hw = self.fused_workspace(nq, k)
             fi, w = self._fused_struct(hw)
             st = (C.c_int32 * _lib.FUSED_STATS)()
-            _lib.check(L.cw_fused_predict_host(C.byref(fi), C.byref(w), Qh.data_ptr(), nq_total, k, out_sid.data_ptr(),
+            _lib.check(L.cw_fused_predict_host(C.byref(fi), C.byref(w), Qh.data_ptr(), nq, k, out_sid.data_ptr(),
                                                out_val.data_ptr(), st, _lib.stream_ptr()), "cw_fused_predict_host")
             self._account(np.asarray(list(st), np.int32))
-            return out_sid, out_val
-        step = self.chunk_queries()
-        for lo in range(0, nq_total, step):
-            nq = min(step, nq_total - lo)
-            ws = self.workspace(min(step, nq_total), k)
-            w = _lib.CwDenseWork()
-            w.Q_dev, w.xt_scratch, w.node_scores, w.ldq = ws["q"].data_ptr(), ws["xt"].data_ptr(), ws["scores"].data_ptr(), ws["ldq"]
-            w.out_sid_dev, w.out_score_dev, w.scratch = ws["sid"].data_ptr(), ws["val"].data_ptr(), ws["scratch"].data_ptr()
-            _lib.check(L.cw_predict_dense_host(C.byref(self.ix), C.byref(w), Qh[lo:lo + nq].data_ptr(), nq, k,
-                                               out_sid[lo:lo + nq].data_ptr(), out_val[lo:lo + nq].data_ptr(),
-                                               _lib.stream_ptr()), "cw_predict_dense_host")
+        else:
+            for r, ws in self._fp32_chunks(nq, k):
+                q = Qh[r]
+                _lib.check(L.cw_predict_dense_host(C.byref(self.ix), C.byref(ws["w"]), q.data_ptr(), q.shape[0], k,
+                                                   out_sid[r].data_ptr(), out_val[r].data_ptr(), _lib.stream_ptr()),
+                           "cw_predict_dense_host")
         return out_sid, out_val
 
 
@@ -889,7 +870,8 @@ class CobwebWrapper:
             return (torch.empty((Q.shape[0], 0), dtype=torch.int32, device=Q.device),
                     torch.empty((Q.shape[0], 0), dtype=torch.float32, device=Q.device))
         if k <= _lib.MAX_K:
-            return self._index.predict_tagged(Q, k, qt, tags, self._tag_version)
+            sids, vals, _ = self._index.predict(Q, k, query_tags=qt, sent_tags=tags, tag_version=self._tag_version)
+            return sids, vals
         # the leaf matrix with ineligible entries at -inf; eligible entries first, each part in (score desc, id asc)
         _, _, leaf = self._index.predict(Q, 0, want_leaf_scores=True, mode="fp32")
         elig = (tags.unsqueeze(0) & qt.unsqueeze(1)) != 0
