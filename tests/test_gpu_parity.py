@@ -220,9 +220,22 @@ def test_ifit_matches_reference_golden(golden_dir, name):
     np.testing.assert_allclose(ns, g["node_scores"], rtol=2e-5, atol=floor)
 
 
-@pytest.mark.parametrize("n,d,kind,k", [(600, 128, "unit", 10), (500, 256, "whitened", 5), (300, 1024, "unit", 10)])
-def test_categorize_bit_exact_vs_oracle(n, d, kind, k):
-    x, tree, ref = build_pair(n, d, kind)
+def _cat_case(n, d, kind, k, **kw):
+    flags = "".join(f"-{key}={val}" for key, val in kw.items())
+    return pytest.param(n, d, kind, k, kw, id=f"{n}-{d}-{kind}-{k}{flags}")
+
+
+# D = 7, 33: scalar loads and a partial last group; D = 7, 30, 33, 64: several teams per warp (Gp = 2, 8, 16, 16);
+# D = 2048: a team of 512 threads (16 warps).  The flags reach the long form of log_prob (use_info=False) and the cached
+# form's variance rows under the other scoring settings.
+@pytest.mark.parametrize("n,d,kind,k,kw", [
+    _cat_case(600, 128, "unit", 10), _cat_case(500, 256, "whitened", 5), _cat_case(300, 1024, "unit", 10),
+    _cat_case(200, 7, "whitened", 10), _cat_case(300, 30, "unit", 10), _cat_case(300, 33, "unit", 10),
+    _cat_case(300, 64, "unit", 10), _cat_case(150, 2048, "unit", 10),
+    _cat_case(300, 96, "whitened", 10, use_info=False), _cat_case(300, 96, "whitened", 10, use_kl=False),
+    _cat_case(300, 96, "whitened", 10, acuity_cutoff=True), _cat_case(300, 96, "whitened", 10, prior_var=0.01)])
+def test_categorize_bit_exact_vs_oracle(n, d, kind, k, kw):
+    x, tree, ref = build_pair(n, d, kind, **kw)
     tree.ifit_batch(x, tag_sentences=True)
     ref.ifit(x)
     pos, rpos = assert_same_tree(tree, ref)
@@ -762,7 +775,7 @@ def test_fused_predict_small_and_odd_shapes():
 def test_ifit_greedy_mode(golden_dir):
     """COBWEB_GREEDY_MODE (src/utils/constants.py; CobwebTorchTree.py:209-213): the kernel takes "new" at every internal
     node.  Equal to the reference's recorded tree, and to the oracle beyond the scoring lists' fan-out limit (the flat
-    tree's root has one child per instance)."""
+    tree's root has one child per instance); best-first retrieval on that flat tree equals the oracle's."""
     from rag_cobweb_b200 import constants
     g = np.load(os.path.join(golden_dir, "greedy_unit_150x24.npz"))
     x = synth.corpus(150, 24, "unit", seed=0)
@@ -782,8 +795,18 @@ def test_ifit_greedy_mode(golden_dir):
     x = synth.corpus(n, d, "whitened", seed=2)
     tree, ref = CobwebTorchTree((d,), greedy_mode=True), OracleTree(d, greedy=True)
     leaves = tree.ifit_batch(x, tag_sentences=True).cpu().numpy()
-    assert_same_tree(tree, ref, leaves, ref.ifit(x))
+    pos, rpos = assert_same_tree(tree, ref, leaves, ref.ifit(x))
     assert tree.bfs()["nchild"][0] == n > 2048
+    # best-first on the flat tree: the root's expansion scores 3000 children in 47 rounds of 64 teams into one frontier
+    q, _ = synth.queries(x, 32, "whitened", seed=1)
+    r = tree.categorize_batch(q, retrieve_k=10)
+    rl, rnf, _, rcalls = ref.categorize(q, k=10)
+    assert np.array_equal(pos[r["leaves"].cpu().numpy()], rpos[rl]) and np.array_equal(r["nfound"].cpu().numpy(), rnf)
+    assert np.array_equal(r["lp_calls"].cpu().numpy(), rcalls)
+    got = tree.categorize_batch(q)
+    _, _, rbest, rcalls = ref.categorize(q, k=0)
+    assert np.array_equal(pos[got["best"].cpu().numpy()], rpos[rbest])
+    assert np.array_equal(got["lp_calls"].cpu().numpy(), rcalls)
 
 
 def test_reference_json_fixture_and_snapshot(golden_dir, tmp_path):
