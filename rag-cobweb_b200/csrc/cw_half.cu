@@ -972,25 +972,62 @@ fn_select_kernel(const FinArgs a) {
     if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(a.stats + 5, (int)a.nq);
 }
 
-__device__ __forceinline__ void cp_async8(void *dst, const void *src) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_u32(dst)), "l"(src) : "memory");
-}
 __device__ __forceinline__ void cp_async4(void *dst, const void *src) {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(smem_u32(dst)), "l"(src) : "memory");
+}
+// adds to the transaction count of the barrier's current phase without arriving
+__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
+    asm volatile("mbarrier.expect_tx.relaxed.cta.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
+}
+
+// The exact chain over 32 attributes of a row segment in shared memory: rv = the segment's {r, mb} pairs, xs = the
+// query's 32 attributes.  The whole piece is read into registers first (16-byte reads; an ODD row starts 8 bytes off
+// that alignment and is read by float2), then the chain runs in ascending d.
+template <bool ODD>
+__device__ __forceinline__ float exact_chain32(const float2 *rv, const float *xs, float acc) {
+    float4 rr[16], xv[8];
+#pragma unroll
+    for (int j = 0; j < 16; j++) {
+        if (ODD) {
+            const float2 u = rv[2 * j], v = rv[2 * j + 1];
+            rr[j] = make_float4(u.x, u.y, v.x, v.y);
+        } else {
+            rr[j] = reinterpret_cast<const float4 *>(rv)[j];  // {r, mb} of 2 attributes
+        }
+    }
+#pragma unroll
+    for (int j = 0; j < 8; j++) xv[j] = reinterpret_cast<const float4 *>(xs)[j];
+#pragma unroll
+    for (int j = 0; j < 16; j++) {
+        const float x0 = (j & 1) ? xv[j >> 1].z : xv[j >> 1].x, x1 = (j & 1) ? xv[j >> 1].w : xv[j >> 1].y;
+        const float t0 = __fmaf_rn(x0, rr[j].x, rr[j].y);
+        acc = __fmaf_rn(t0, t0, acc);
+        const float t1 = __fmaf_rn(x1, rr[j].z, rr[j].w);
+        acc = __fmaf_rn(t1, t1, acc);
+    }
+    return acc;
 }
 
 // Exact node scores with the FP32 path's arithmetic: out[q * stride + i] = -0.5 (sumlog[b] + sum_d (x_qd r_bd + mb_bd)^2)
 // for b = list[q * stride + i], i < n = meta[q * meta_stride + n_word].  One warp per (query, row block): blockIdx.y
 // takes rows [y * per, (y + 1) * per) with per = max(EX_R, ceil(n / gridDim.y)), so a long list is spread over several
-// warps (gridDim.y = 1: one warp takes the whole list); a warp's rows go in rounds of at most EX_R.  For the
-// arithmetic lane = row (every lane runs its row's FMA chain in ascending d from 0, so the result is bit-identical to
-// dense_score_kernel), for the loads lane = attribute: per 32 attributes of a row one coalesced 256-byte cp.async
-// segment into a ring of EX_STAGES segments, EX_STAGES - 1 ahead of the arithmetic.  A row's segment is padded to
-// EX_RS = 34 float2, so the 16-byte reads by row are conflict-free (8 lanes, 8 different 4-bank groups) and a lane takes
-// its whole segment into registers before the chain runs over it.  No registers hold the rows in flight, so a warp needs
-// only its ring and 12 warps fit on an SM.
-constexpr int EX_WARPS = 4, EX_R = 16, EX_STAGES = 4, EX_RS = 34;
-constexpr int EX_WARP_BYTES = EX_STAGES * EX_R * EX_RS * 8 + EX_STAGES * 32 * 4;
+// warps (gridDim.y = 1: one warp takes the whole list); a warp's rows go in rounds of at most EX_R.  Lane = row: every
+// lane runs its row's FMA chain in ascending d from 0, so the result is bit-identical to dense_score_kernel.
+// The rows arrive by bulk copies (cp.async.bulk, completion counted in bytes on an mbarrier), EX_SEG attributes (512
+// bytes) of a row per copy, into a ring of EX_STAGES slots, EX_STAGES - 1 segments ahead of the arithmetic; each lane
+// copies its own row's segment.  One warp per CTA, so a warp slot is handed to the next work item as soon as its list
+// is done rather than when the CTA's longest list is; 12 such CTAs (17 KB each) fit an SM.  This geometry was chosen
+// by timing the cfg3 launches against others (DESIGN §5).  A bulk copy needs 16-byte-aligned ends; a row of the
+// [nn, D, 2] buffer (16-byte aligned: the entry points check it) starts 8 bytes off when b * D is odd, so a copy takes
+// the aligned-down span (at most EX_SEG * 8 + 16 bytes: the slot pitch EX_RS) and the lane reads its segment from that
+// offset.  No copy reads past the buffer's last byte: where that byte ends 8 bytes into a 16-byte unit, the copy stops
+// short and the lane reads the buffer's last {r, mb} pair from global memory.  The pitch of EX_SEG + 2 float2 puts
+// consecutive rows 4 banks apart, so the 16-byte reads by row are conflict-free.  The query's slice of a segment comes
+// with 4-byte cp.async copies, one commit group per segment.
+constexpr int EX_WARPS = 1, EX_R = 16, EX_SEG = 64, EX_STAGES = 2, EX_RS = EX_SEG + 2;
+// per warp: the ring [EX_STAGES][EX_R][EX_RS] float2, the query slices [EX_STAGES][EX_SEG], one mbarrier per slot
+constexpr int EX_WARP_BYTES = (EX_STAGES * EX_R * EX_RS * 8 + EX_STAGES * EX_SEG * 4 + EX_STAGES * 8 + 15) / 16 * 16;
+static_assert(EX_SEG % 32 == 0 && EX_RS * 8 % 16 == 0, "ring geometry");
 __global__ void __launch_bounds__(EX_WARPS * 32)
 fn_exact_kernel(const cw_index ix, const float2 *__restrict__ RM, const float *__restrict__ Q, long long nq,
                 const int *__restrict__ list, const int *__restrict__ meta, int meta_stride, int n_word, int stride,
@@ -998,27 +1035,48 @@ fn_exact_kernel(const cw_index ix, const float2 *__restrict__ RM, const float *_
     extern __shared__ __align__(16) unsigned char ex_smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, D = ix.D;
     float2 *ring = reinterpret_cast<float2 *>(ex_smem + (size_t)warp * EX_WARP_BYTES);  // [EX_STAGES][EX_R][EX_RS]
-    float *xr = reinterpret_cast<float *>(ring + EX_STAGES * EX_R * EX_RS);             // [EX_STAGES][32]
+    float *xr = reinterpret_cast<float *>(ring + EX_STAGES * EX_R * EX_RS);             // [EX_STAGES][EX_SEG]
+    const uint32_t bar0 = smem_u32(xr + EX_STAGES * EX_SEG);                             // [EX_STAGES] mbarriers
     const long long q = (long long)blockIdx.x * EX_WARPS + warp;
     if (q >= nq) return;
     const int n_all = meta[q * meta_stride + n_word];
     const int per = max(EX_R, (n_all + (int)gridDim.y - 1) / (int)gridDim.y), first = (int)blockIdx.y * per;
     if (first >= n_all) return;
     const int n = min(n_all, first + per);  // rows [first, n)
+    if (lane == 0) {
+        for (int s = 0; s < EX_STAGES; s++) mbar_init(bar0 + 8 * s, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    __syncwarp();
     const float *xq = Q + q * D;
-    const int n_seg = (D + 31) / 32;
+    const int n_seg = (D + EX_SEG - 1) / EX_SEG;
+    const long long lim = (long long)ix.nn * D * 8 & ~15ll;  // the buffer's last 16-byte boundary
+    unsigned parity = 0;  // bit s: the phase of slot s's barrier that the next wait on it expects
     const int n_rounds = (n - first + EX_R - 1) / EX_R, rpr = (n - first + n_rounds - 1) / n_rounds;  // rows per round <= EX_R
     for (int lo = first; lo < n; lo += rpr) {
         const int cnt = min(rpr, n - lo);
         const int b = lane < cnt ? list[q * stride + lo + lane] : 0;
+        const long long rb = (long long)b * D * 8;  // byte offset of the lane's row
+        const int odd = (int)(rb & 8);              // 8 when the row starts off 16-byte alignment
         auto issue = [&](int seg) {
             if (seg < n_seg) {
-                const int s = seg & (EX_STAGES - 1), d = seg * 32 + lane;
-                for (int r = 0; r < cnt; r++) {
-                    const int br = __shfl_sync(0xffffffffu, b, r);
-                    if (d < D) cp_async8(ring + (s * EX_R + r) * EX_RS + lane, RM + (size_t)br * D + d);
+                const int s = seg % EX_STAGES, d0 = seg * EX_SEG;
+                const uint32_t bar = bar0 + 8 * s;
+                if (lane < cnt) {
+                    const long long from = rb + d0 * 8 - odd;
+                    long long to = (rb + (long long)min(D, d0 + EX_SEG) * 8 + 15) & ~15ll;
+                    if (to > lim) to -= 16;
+                    if (to > from) {
+                        mbar_expect_tx(bar, (uint32_t)(to - from));
+                        bulk_g2s(smem_u32(ring + (s * EX_R + lane) * EX_RS), reinterpret_cast<const char *>(RM) + from,
+                                 (uint32_t)(to - from), bar);
+                    }
                 }
-                if (d < D) cp_async4(xr + s * 32 + lane, xq + d);
+#pragma unroll
+                for (int i = lane; i < EX_SEG; i += 32)
+                    if (d0 + i < D) cp_async4(xr + s * EX_SEG + i, xq + d0 + i);
+                __syncwarp();  // every lane's expected bytes are on the barrier before it can complete
+                if (lane == 0) mbar_arrive(bar);
             }
             asm volatile("cp.async.commit_group;" ::: "memory");  // one group per segment, empty past the end
         };
@@ -1027,31 +1085,25 @@ fn_exact_kernel(const cw_index ix, const float2 *__restrict__ RM, const float *_
         float acc = 0.0f;
         for (int seg = 0; seg < n_seg; seg++) {
             issue(seg + EX_STAGES - 1);
+            const int s = seg % EX_STAGES, d0 = seg * EX_SEG;
             asm volatile("cp.async.wait_group %0;" ::"n"(EX_STAGES - 1) : "memory");
-            __syncwarp();
-            const int s = seg & (EX_STAGES - 1), dd = seg * 32;
-            const float2 *rv = ring + (s * EX_R + lane) * EX_RS;
-            const float *xs = xr + s * 32;
+            mbar_wait(bar0 + 8 * s, (parity >> s) & 1u);
+            parity ^= 1u << s;
+            __syncwarp();  // the query slice: every lane's copies
+            const float2 *rv = ring + (s * EX_R + lane) * EX_RS + (odd >> 3);
+            const float *xs = xr + s * EX_SEG;
             if (lane < cnt) {
-                if (dd + 32 <= D) {
-                    float4 rr[16], xv[8];
 #pragma unroll
-                    for (int j = 0; j < 16; j++) rr[j] = reinterpret_cast<const float4 *>(rv)[j];  // {r, mb} of 2 attributes
-#pragma unroll
-                    for (int j = 0; j < 8; j++) xv[j] = reinterpret_cast<const float4 *>(xs)[j];
-#pragma unroll
-                    for (int j = 0; j < 16; j++) {
-                        const float x0 = (j & 1) ? xv[j >> 1].z : xv[j >> 1].x, x1 = (j & 1) ? xv[j >> 1].w : xv[j >> 1].y;
-                        const float t0 = __fmaf_rn(x0, rr[j].x, rr[j].y);
-                        acc = __fmaf_rn(t0, t0, acc);
-                        const float t1 = __fmaf_rn(x1, rr[j].z, rr[j].w);
-                        acc = __fmaf_rn(t1, t1, acc);
-                    }
-                } else {
-                    for (int j = 0; j < D - dd; j++) {
-                        const float2 v = rv[j];
-                        const float t = __fmaf_rn(xs[j], v.x, v.y);
-                        acc = __fmaf_rn(t, t, acc);
+                for (int c = 0; c < EX_SEG; c += 32) {
+                    if (d0 + c + 32 <= D) {
+                        acc = odd ? exact_chain32<true>(rv + c, xs + c, acc) : exact_chain32<false>(rv + c, xs + c, acc);
+                    } else {
+                        for (int j = c; j < D - d0; j++) {
+                            const float2 v = rb + (d0 + j + 1) * 8 > lim ? RM[(size_t)b * D + d0 + j] : rv[j];
+                            const float t = __fmaf_rn(xs[j], v.x, v.y);
+                            acc = __fmaf_rn(t, t, acc);
+                        }
+                        break;
                     }
                 }
             }
@@ -1552,6 +1604,7 @@ static bool fused_args_ok(const cw_fused_index *fi, const cw_fused_work *w, int 
     if (!fi || !w || k < 1 || k > CW_FUSED_MAX_K || fi->n_leaf < 1 || fi->ix.n_pos < 1 || !fi->ix.path_idx || !fi->ix.level_w ||
         !fi->ix.sumlog || !fi->rows || !fi->leaf_row_b || !fi->leaf_pos || !fi->sent_off || !fi->sent_ids)
         return false;
+    if (reinterpret_cast<uintptr_t>(fi->rows) % 16) return false;  // fn_exact_kernel's bulk copies
     if (!set_ok(&fi->leaves, fi->ix.D) || fi->leaves.nprod != 1 || fi->leaves.n_rows != fi->n_leaf) return false;
     if (fi->n_int && (!set_ok(&fi->internal, fi->ix.D) || fi->internal.nprod != 3 || fi->internal.layout != CW_H_F2 ||
                       fi->internal.n_rows != fi->n_int))

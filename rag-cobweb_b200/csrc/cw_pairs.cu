@@ -237,6 +237,10 @@ static int pair_check(const char *what, const cw_index *ix, const float *rows, c
         cw_set_error("%s: null pointer", what);
         return CW_E_ARG;
     }
+    if (reinterpret_cast<uintptr_t>(rows) % 16) {  // fn_exact_kernel fetches the rows with bulk copies
+        cw_set_error("%s: rows must be 16-byte aligned", what);
+        return CW_E_ARG;
+    }
     return 0;
 }
 
