@@ -836,6 +836,45 @@ void co_dense_scores(int D, long nq, const float *Q, int nn, const float *means,
     if (leaf_scores) co_leaf_scores(nq, nn, node_scores, nl, maxlen, path_idx, path_w, leaf_scores);
 }
 
+/* Operands of the engine's FP32 form (dense_operands in the CUDA sources): r = 1 / sqrt(var), mb = -(mean * r),
+ * each a single binary32 operation, so that (x - mean)^2 / var = (x * r + mb)^2. */
+void co_fp32_operands(int D, int nn, const float *means, const float *vars, float *r, float *mb) {
+    for (size_t i = 0; i < (size_t)nn * D; i++) {
+        r[i] = 1.0f / sqrtf(vars[i]);
+        mb[i] = -(means[i] * r[i]);
+    }
+}
+
+/* out[i] = fmaf(a[i], b[i], c[i]): the fused multiply-add co_fp32_node_scores uses, exposed so the tests can check it
+ * against exact rational arithmetic. */
+void co_fmaf_array(long n, const float *a, const float *b, const float *c, float *out) {
+    for (long i = 0; i < n; i++) out[i] = fmaf(a[i], b[i], c[i]);
+}
+
+/* Node scores of the engine's FP32 form bit for bit (dense_score_kernel / small_scores_kernel): per (query, node) one
+ * chain over d ascending, u = fma(x, r, mb); acc = fma(u, u, acc) from acc = +0, then -0.5 * (sumlog + acc).  libm
+ * fmaf is correctly rounded, as the device's FFMA is. */
+void co_fp32_node_scores(int D, long nq, const float *Q, int nn, const float *means, const float *vars,
+                         const float *sumlog, float *node_scores) {
+    float *r = (float *)malloc(sizeof(float) * (size_t)nn * D);
+    float *mb = (float *)malloc(sizeof(float) * (size_t)nn * D);
+    co_fp32_operands(D, nn, means, vars, r, mb);
+#pragma omp parallel for collapse(2) schedule(static)
+    for (long q = 0; q < nq; q++) {
+        for (int b = 0; b < nn; b++) {
+            const float *x = Q + (size_t)q * D, *rb = r + (size_t)b * D, *mbb = mb + (size_t)b * D;
+            float acc = 0.0f;
+            for (int d = 0; d < D; d++) {
+                const float u = fmaf(x[d], rb[d], mbb[d]);
+                acc = fmaf(u, u, acc);
+            }
+            node_scores[(size_t)q * nn + b] = -0.5f * (sumlog[b] + acc);
+        }
+    }
+    free(r);
+    free(mb);
+}
+
 /* Throughput-oriented variant of the same scores for the CPU baseline (bench.py): plain
  * binary32 accumulation, vectorisable, one pass per query over the node matrices like the
  * reference's broadcast expression.  Not used for parity. */

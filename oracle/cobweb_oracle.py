@@ -63,6 +63,9 @@ def lib():
         L.co_leaf_scores.argtypes = [C.c_long, C.c_int, fp, C.c_long, C.c_int, ip, fp, fp]
         L.co_dense_scores_fast.argtypes = [C.c_int, C.c_long, fp, C.c_int, fp, fp, fp, fp]
         L.co_topk.argtypes = [fp, C.c_long, C.c_int, ip, fp]
+        L.co_fp32_operands.argtypes = [C.c_int, C.c_int, fp, fp, fp, fp]
+        L.co_fp32_node_scores.argtypes = [C.c_int, C.c_long, fp, C.c_int, fp, fp, fp, fp]
+        L.co_fmaf_array.argtypes = [C.c_long, fp, fp, fp, fp]
         L.co_logf.restype = C.c_float
         L.co_logf.argtypes = [C.c_float]
         L.co_sum_public.restype = C.c_float
@@ -244,6 +247,32 @@ class OracleTree:
         lib().co_dense_scores(self.d, nq, _f(Q), nn, _f(ix["means"]), _f(ix["vars"]), _f(ix["sumlog"]), L,
                               ix["path_idx"].shape[1], _i(ix["path_idx"]), _f(ix["path_w"]), _f(ns), _f(ls))
         return ns, ls
+
+    def fp32_operands(self):
+        """(r, mb) [nn, D] of the engine's FP32 form in BFS order: r = 1 / sqrt(var), mb = -(mean * r)."""
+        ix = self.index
+        r, mb = np.empty_like(ix["vars"]), np.empty_like(ix["vars"])
+        lib().co_fp32_operands(self.d, r.shape[0], _f(ix["means"]), _f(ix["vars"]), _f(r), _f(mb))
+        return r, mb
+
+    def fp32_scores(self, Q):
+        """(node_scores [nq, Nn], leaf_scores [nq, L]) of the engine's FP32 form bit for bit: the node score chain
+        u = fma(x, r, mb), acc = fma(u, u, acc) over d ascending, -0.5 * (sumlog + acc); then the path product."""
+        ix = self.index
+        Q = _f32(np.atleast_2d(Q))
+        nq, nn, L = Q.shape[0], ix["means"].shape[0], ix["path_idx"].shape[0]
+        ns = np.empty((nq, nn), np.float32)
+        lib().co_fp32_node_scores(self.d, nq, _f(Q), nn, _f(ix["means"]), _f(ix["vars"]), _f(ix["sumlog"]), _f(ns))
+        return ns, leaf_scores(ns, ix["path_idx"], ix["path_w"])
+
+
+def fmaf(a, b, c):
+    """Elementwise fmaf(a, b, c) in binary32, the fused multiply-add of fp32_scores."""
+    a, b, c = np.broadcast_arrays(_f32(a), _f32(b), _f32(c))
+    a, b, c = _f32(a), _f32(b), _f32(c)
+    out = np.empty(a.shape, np.float32)
+    lib().co_fmaf_array(a.size, _f(a), _f(b), _f(c), _f(out))
+    return out
 
 
 def leaf_scores(node_scores, path_idx, path_w):

@@ -244,6 +244,8 @@ __device__ __forceinline__ int float_key(float f) {
     return i >= 0 ? i : i ^ 0x7fffffff;
 }
 __device__ __forceinline__ float key_float(int k) { return __int_as_float(k >= 0 ? k : k ^ 0x7fffffff); }
+// the per-query shared thresholds before any chunk published one (cudaMemsetAsync with 0x80: the key of -3.396e38)
+constexpr int THR_UNSET = (int)0x80808080u;
 
 // Rare path of the kernel below (the path length changes a handful of times per chunk); kept out
 // of line so that its binary64 division does not inflate the hot loop's register allocation.
@@ -382,7 +384,10 @@ paths_topk_kernel(const float *__restrict__ ST, unsigned ldq, long long nq, int 
               published = thr_s;
               atomicMax(gslot, float_key(thr_s));
           }
-          gthr = fmaxf(gthr, key_float(__ldcg(gslot)));
+          // the slot starts at the memset pattern THR_UNSET, the key of a finite score: until a chunk publishes a
+          // larger key it bounds nothing, so that a query with fewer than k finite scores still collects its -inf ones
+          const int key = __ldcg(gslot);
+          if (key > THR_UNSET) gthr = fmaxf(gthr, key_float(key));
       }
       const int re = min(n, rb + 32);
       for (int r = rb; r < re; r++) {
@@ -441,8 +446,8 @@ paths_topk_kernel(const float *__restrict__ ST, unsigned ldq, long long nq, int 
                 float es = NEG_INF;
                 int ei = -1;
                 if (lane < k) { es = Ls[base + lane]; ei = Li[base + lane]; }
-                // empty ranks hold -inf, so they never beat a finite candidate
-                const int pos = __popc(__ballot_sync(0xffffffffu, es > cv || (es == cv && ei < sid)));
+                // empty ranks (id -1) never beat a candidate, not even one that scores -inf
+                const int pos = __popc(__ballot_sync(0xffffffffu, ei >= 0 && (es > cv || (es == cv && ei < sid))));
                 const float ps = __shfl_sync(0xffffffffu, es, (k - 2) & 31);
                 const int pi = __shfl_sync(0xffffffffu, ei, (k - 2) & 31);
                 if (lane >= pos && lane + 1 < k) { Ls[base + lane + 1] = es; Li[base + lane + 1] = ei; }
@@ -675,7 +680,7 @@ static int paths_topk_launch(const cw_index *ix, const float *node_scores, int64
     int *cand_i = scratch + (size_t)nq * n_chunks * (k > 0 ? k : 1);
     int *shared_thr = scratch + (size_t)2 * nq * n_chunks * (k > 0 ? k : 1);  // [nq] inside the extra chunk of scratch
     if (k > 0) {
-        // 0x80808080 is the key of a large negative score: below every real one
+        // THR_UNSET: no threshold yet
         int rc = cw_check_cuda(cudaMemsetAsync(shared_thr, 0x80, (size_t)nq * sizeof(int), st), "cw_dense_paths_topk: memset");
         if (rc) return rc;
     }

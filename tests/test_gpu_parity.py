@@ -276,6 +276,8 @@ def test_dense_predict_vs_oracle(n, d, kind):
     # score = -0.5 * (sumlog + quad) can cancel to ~0: absolute floor of a few ulps of |sumlog|
     floor = 8 * EPS32 * float(np.abs(ix["sumlog"]).max())
     np.testing.assert_allclose(ns, rns, rtol=1e-5, atol=floor)
+    # and bit for bit the CPU model of the FP32 form's arithmetic (tests/test_fp32_form.py)
+    assert np.array_equal(np.ascontiguousarray(ns).view(np.int32), ref.fp32_scores(q)[0].view(np.int32))
     ids, vals, leaf = w._index.predict(qd, k, want_leaf_scores=True)
     leaf, ids, vals = leaf.cpu().numpy(), ids.cpu().numpy(), vals.cpu().numpy()
     np.testing.assert_allclose(leaf, rls, rtol=1e-5, atol=floor)
